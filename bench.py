@@ -1,16 +1,18 @@
 #!/usr/bin/env python
 """bench.py - sclens() throughput on synthetic data of the BASELINE.json shapes.
 
-    python bench.py --gpus N --steps K --warmup W [--workload C|B|small|D|E] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload C|B|small|D|E] [--impl reference] [--dump-outputs DIR]
 
 Workloads: C = 68k cells x 20k genes (BASELINE.json configs[2], the shape the metric is quoted on; default),
 B = 10k x 20k (configs[1]), small = 2k x 3k (smoke), D = 500k x 25k (configs[3]: signal stage only - cell-sharded
 Gram + NCCL reduce of the packed triangle + the two eigensolves), E = C with 100 perturbation replicates (configs[4]).
 
-The run budgets itself: the driver gives one N of the scaling series 870 s, so warm-up stops after 3 passes (or
-earlier than requested when the passes already agree within 1 %) and the timed passes are min(--steps, what fits in
-SCLENS_BENCH_BUDGET_S, default 600 s, from process start); the line reports `steps` actually timed next to
-`steps_requested`.
+Exactly --steps passes are timed.  Warm-up runs --warmup passes but stops after the third once two consecutive passes
+agree within 1 %; the line reports the warm-up passes run next to `warmup_requested`.
+
+--dump-outputs DIR writes what the last timed pass computed - the arrays a caller reads back from the handle - as
+DIR/<name>.npy (float32 / float64, at most 64 MB in all).  The synthetic inputs depend on the workload's seed only, so
+two builds run with the same arguments can be compared output for output.
 
 One "step" = one complete sclens() pass (signal detection + robustness test, n_perturb=20) over
 the synthetic count matrix of the workload.  Our arm:
@@ -311,6 +313,52 @@ def make_counts_csc_gpu(N, M, seed, device, gene_block=64):
     return X
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def pass_outputs(h, si, ri):
+    """Everything a caller reads back from the handle after a pass (scl_get_*), by name, as float32 / float64 arrays:
+    the signal stage, and the robustness stage when the pass ran one (ri is None otherwise)."""
+    out = {"L": h.L(), "L_mp": h.L_mp()}
+    for k in ("n_signal", "n_Lmp", "lambda_c", "b_plus", "b_minus", "ks_static", "pass_"):
+        out[k] = np.float64(getattr(si, k))
+    if si.n_signal > 0:
+        out["signal_ev"] = h.signal_ev()
+        out["signal_evec"] = h.signal_evec()
+        out.update({f"rec_{k}": v for k, v in h.rec_vals().items()})
+    if ri is not None:
+        for k in ("n_search", "min_pc", "n_robust", "n_add", "p_sel", "p_th", "n_subspace_fallbacks"):
+            out[k] = np.float64(getattr(ri, k))
+        out["gene_basis"] = h.gene_basis()
+        out["b_"], out["m_scores"], out["sd_scores"] = h.scores()
+        out["sig_id"] = h.sig_id().astype(np.float64)
+        out["search_p"], out["search_d"] = h.search_trace()
+    return out
+
+
+def dump_outputs(outdir, arrays, limit=DUMP_LIMIT_BYTES):
+    """DIR/<name>.npy for every array.  Should the whole exceed `limit`, each array over an equal share of it keeps a
+    fixed, seeded sample of its longest axis; the sampled positions go to DIR/<name>_index.npy."""
+    os.makedirs(outdir, exist_ok=True)
+    share = limit // len(arrays) - 256          # two .npy headers
+    sample = sum(np.asarray(a).nbytes for a in arrays.values()) > limit - 128 * len(arrays)
+    written = 0
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        if sample and a.nbytes > share:
+            ax = int(np.argmax(a.shape))
+            keep = max(1, share // (a.nbytes // a.shape[ax] + 8))          # sampled slices + their float64 positions
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[ax], size=keep, replace=False))
+            a = np.take(a, idx, axis=ax)
+            np.save(os.path.join(outdir, f"{name}_index.npy"), idx.astype(np.float64))
+            written += idx.size * 8
+        np.save(os.path.join(outdir, f"{name}.npy"), a)
+        written += a.nbytes
+    return written
+
+
 _REAL_STDOUT = None
 
 
@@ -332,7 +380,7 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None, help="timed passes requested (default 2; fewer are timed when they do not fit the budget)")
+    ap.add_argument("--steps", type=int, default=2, help="timed passes")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     # default = the configuration BASELINE.json's metric is quoted on (68k x 20k, fits one GPU)
@@ -341,11 +389,13 @@ def main():
     ap.add_argument("--gram-mode", type=int, default=0)
     ap.add_argument("--e2e-steps", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--budget-s", type=float, default=float(os.environ.get("SCLENS_BENCH_BUDGET_S", "600")),
-                    help="wall-clock budget of the whole run, from process start")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed pass to DIR/<name>.npy")
     args = ap.parse_args()
-    if args.steps is None:
-        args.steps = 2
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU pass; the reference arm times stages only")
     if args.n_perturb is None:
         args.n_perturb = 100 if args.workload == "E" else 20
     signal_only = args.workload == "D"
@@ -440,12 +490,7 @@ def main():
         if len(warm_s) >= 3 and abs(warm_s[-1] - warm_s[-2]) <= 0.01 * warm_s[-1]:
             break
     warm_done = len(warm_s)
-    t_pass = warm_s[-1] if warm_s else 70.0
-    # ---- how many timed passes fit: the end-to-end call(s) and (N = 1) the CPU sample still have to run afterwards
-    reserve = args.e2e_steps * (t_pass + 5.0) + (45.0 if (world == 1 and not args.no_cpu_baseline) else 0.0) + 15.0
-    left = args.budget_s - (time.perf_counter() - T_START) - reserve
-    steps = int(max(1, min(args.steps, left // max(t_pass, 1e-3))))
-    steps = int(agree(float(steps), dist.ReduceOp.MIN if world > 1 else None))
+    steps = args.steps
 
     h.reset_profile()
     launches0 = h.profile().kernel_launches
@@ -463,6 +508,9 @@ def main():
     ms = agree(ms, dist.ReduceOp.MAX if world > 1 else None)
     ms_per_step = ms / steps
     value = N / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:      # every rank holds the same results of the shared pass
+        nbytes = dump_outputs(args.dump_outputs, pass_outputs(h, si, ri))
+        log(f"[rank 0] outputs of the last timed pass: {nbytes / 2 ** 20:.1f} MB in {args.dump_outputs}")
 
     # ---- e2e through the public API with host buffers (pinned), results read back
     e2e = None
@@ -602,7 +650,7 @@ def main():
             "data": "synthetic", "config": config, "clocks": clk, "gpu_launches": int(launches),
             "roofline": roofline, "stage_ms_over_timed_region": stage_ms, "phase_ms": phase, "phase_ms_last_step": phase,
             "gemm_tflops": {"other_gemm_2mnk": rate(prof.other_gemm_flops, prof.other_gemm_ms, 1e12)},
-            "result": result, "budget_s": args.budget_s, "wall_s_at_line": None}
+            "result": result, "wall_s_at_line": None}
     if ri is not None and ri.t_perturb_ms > 0:
         line["perturbation_replicates_per_s"] = args.n_perturb / (ri.t_perturb_ms * 1e-3)
     if e2e is not None:

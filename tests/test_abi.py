@@ -45,15 +45,20 @@ def test_struct_layouts_match_header(lib_built, tmp_path):
 
 
 def test_fails_loudly_without_gpu(lib_built):
-    import torch
-    from sclens_b200 import Handle, SclError, sclens
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(SclError) as e:
-        Handle()
-    assert e.value.code == -4 and "no CPU fallback" in str(e.value)
-    with pytest.raises(ValueError):
-        sclens(np.eye(4), device_="cpu")
+    """In a process that sees no device (none there, or hidden by CUDA_VISIBLE_DEVICES)."""
+    import subprocess
+    import sys
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "import numpy as np, pytest\n"
+            "from sclens_b200 import Handle, SclError, sclens\n"
+            "with pytest.raises(SclError) as e:\n"
+            "    Handle()\n"
+            "assert e.value.code == -4 and 'no CPU fallback' in str(e.value)\n"
+            "with pytest.raises(ValueError):\n"
+            "    sclens(np.eye(4), device_='cpu')\n" % ROOT)
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                         text=True)
+    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
 
 
 def test_product_never_imports_oracle():

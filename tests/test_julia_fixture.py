@@ -1,9 +1,9 @@
 """Oracle pin: consumes a fixture written by julia/export_fixture.jl (the unmodified reference run with a seeded RNG:
 draws bundle + result Dict) and checks the oracle - and, with a GPU, the CUDA path - against it.
 
-No Julia exists in the build image, so no such fixture is committed: the Julia-side tests SKIP until someone drops one in
-tests/golden/julia_fixture/ (or points SCLENS_JULIA_FIXTURE at it).  The reader and the comparison are exercised on every
-run by a fixture in the same format written from the oracle itself (which proves the plumbing, not the oracle)."""
+No run of the Julia reference has been recorded yet, so no such fixture is committed: the Julia-side tests SKIP until one
+is committed as tests/golden/julia_fixture/ (they read nothing outside the repository).  The reader and the comparison
+are exercised on every run by a fixture in the same format written from the oracle itself (which proves the plumbing, not the oracle)."""
 import os
 
 import numpy as np
@@ -13,7 +13,7 @@ import scipy.sparse as sp
 from oracle import sclens_oracle as orc
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-FIXTURE = os.environ.get("SCLENS_JULIA_FIXTURE", os.path.join(HERE, "golden", "julia_fixture"))
+FIXTURE = os.path.join(HERE, "golden", "julia_fixture")
 JULIA_TYPES = {"UInt32": np.uint32, "Int64": np.int64, "Float64": np.float64, "Float32": np.float32, "Int32": np.int32}
 
 
