@@ -274,6 +274,49 @@ SCL_API int32_t scl_op_denoise(scl_handle* h, int32_t N, int32_t M, int32_t r, c
                        const double* TGC, const double* mat2_mean, const double* mat2_std, const double* norm_tgc,
                        const double* cent, int32_t out_f32, void* out);
 
+/* ---- apply_umap! (:863-873, UMAP.jl UMAP_) on the device ------------------------------------------------------------ */
+/* Parameters of UMAP_ with its defaults in the host mirrors: n_neighbors 15, n_components 2, n_epochs 300, metric 1
+ * (0 = euclidean, 1 = cosine), init 0 (0 = spectral, 1 = random), neg_sample_rate 5, spectral_maxiter 100, min_dist 0.1,
+ * spread 1, learning_rate 1, repulsion_strength 1, local_connectivity 1, seed 0. */
+typedef struct {
+  int32_t n_neighbors;       /* k: 1 <= k <= 64, k < N */
+  int32_t n_components;      /* nc: 1 <= nc <= 16 */
+  int32_t n_epochs;          /* >= 0; 0 returns the start */
+  int32_t metric;            /* 0 euclidean, 1 cosine (1/2 |x^ - y^|^2 of unit rows; a zero row is at distance 1) */
+  int32_t init;              /* 0 spectral (random start when the iteration does not converge), 1 uniform in [-10, 10] */
+  int32_t neg_sample_rate;   /* negative samples per fired edge */
+  int32_t spectral_maxiter;  /* outer iterations of the spectral block iteration (degree-8 Chebyshev filter each) */
+  int32_t reserved0;
+  double min_dist, spread, learning_rate, repulsion_strength, local_connectivity;
+  uint64_t seed;             /* every draw is a hash of (seed, stream, epoch, vertex, slot) */
+  int32_t reserved[4];
+} scl_umap_params;
+
+typedef struct {
+  double a, b;               /* fitted 1 / (1 + a x^(2b)) */
+  int64_t graph_nnz;         /* stored entries of the symmetric fuzzy graph */
+  int32_t spectral_iters;    /* outer iterations of the spectral start (0 when not run) */
+  int32_t init_fallback;     /* 1: the spectral start did not converge and the random start was taken */
+  double t_knn_ms, t_graph_ms, t_init_ms, t_layout_ms;   /* CUDA events on the handle's stream */
+  int32_t reserved[4];
+} scl_umap_info;
+
+/* Exact k nearest neighbours of the rows of X (N x d column-major), self excluded, ascending in (distance, index):
+ * idx / dist are N x k row-major ([i * k + s], 0-based).  metric as in scl_umap_params. */
+SCL_API int32_t scl_op_knn(scl_handle* h, int32_t N, int32_t d, const float* X, int32_t k, int32_t metric, int32_t* idx,
+                           float* dist);
+/* UMAP_(X', nc) of apply_umap!: kNN, fuzzy graph, start, layout.  init_embedding (N x nc column-major) replaces the
+ * computed start when not NULL (with n_epochs = 0 each stage can be checked on its own).  embedding: N x nc column-major.
+ * The kNN and the graph stay on the handle (scl_get_umap_knn, scl_get_umap_graph).  Same seed, same bits. */
+SCL_API int32_t scl_op_umap(scl_handle* h, int32_t N, int32_t d, const float* X, const scl_umap_params* p,
+                            const float* init_embedding, float* embedding, scl_umap_info* info);
+/* The fuzzy graph of the last scl_op_umap: symmetric N x N CSR, sorted columns, 0-based.  Call with NULL arrays for *nnz. */
+SCL_API int32_t scl_get_umap_graph(scl_handle* h, int64_t* nnz, uint32_t* rowptr /* N+1 */, uint32_t* colidx, float* val);
+/* The kNN of the last scl_op_umap (N x k row-major, as scl_op_knn). */
+SCL_API int32_t scl_get_umap_knn(scl_handle* h, int32_t* idx, float* dist);
+/* The a / b fit of UMAP_ (Levenberg-Marquardt on the host, Float64).  Pure host code. */
+SCL_API int32_t scl_umap_fit_ab(double min_dist, double spread, double* a, double* b);
+
 /* ---- kernel-level timing harness (device-resident synthetic operands; used by bench.py and the ncu captures) ---- */
 /* Gram / GEMM kernel alone: rows x K binary16 operand generated on the device; mode bit0 = split (hi+lo) operands,
  * bit1 = full GEMM instead of the syrk schedule; chunk_kb = k-blocks per accumulation chunk (0 = default).

@@ -38,6 +38,21 @@ mutable struct SclRobustInfo
     n_subspace_fallbacks::Int32; reserved::Int32
     SclRobustInfo() = new()
 end
+struct SclUmapParams
+    n_neighbors::Int32; n_components::Int32; n_epochs::Int32; metric::Int32
+    init::Int32; neg_sample_rate::Int32; spectral_maxiter::Int32; reserved0::Int32
+    min_dist::Float64; spread::Float64; learning_rate::Float64; repulsion_strength::Float64; local_connectivity::Float64
+    seed::UInt64
+    reserved::NTuple{4,Int32}
+end
+mutable struct SclUmapInfo
+    a::Float64; b::Float64
+    graph_nnz::Int64
+    spectral_iters::Int32; init_fallback::Int32
+    t_knn_ms::Float64; t_graph_ms::Float64; t_init_ms::Float64; t_layout_ms::Float64
+    reserved::NTuple{4,Int32}
+    SclUmapInfo() = new()
+end
 
 function check(h, rc)
     rc == 0 && return
@@ -141,6 +156,58 @@ function get_denoised_df(inp_obj; out32::Bool=false)
     odf = DataFrame(out, inp_obj[:gene_id])                                         # :928
     insertcols!(odf, 1, :cell => inp_obj[:cell_id])                                 # :929
     odf
+end
+
+# metric of apply_umap!: :cosine / :euclidean, or a Distances.jl CosineDist() / Euclidean() (matched by type name, so
+# Distances.jl need not be loaded here)
+function umap_metric(metric)
+    name = metric isa Symbol ? String(metric) : lowercase(String(nameof(typeof(metric))))
+    name in ("cosine", "cosinedist") && return Int32(1)
+    name in ("euclidean",) && return Int32(0)
+    error("apply_umap!: unsupported metric $(metric) (cosine or euclidean)")
+end
+
+"""
+    apply_umap!(l_inp; k=15, nc=2, md=0.1, metric=CosineDist(), n_epochs=300, seed=0)
+
+Drop-in for scLENS.apply_umap! (src/scLENS.jl:863-873) on the device: exact kNN, fuzzy graph, spectral start and a
+deterministic synchronous layout (DESIGN.md).  Reads `:pca_n1` when it exists and has at least one signal column,
+otherwise `:pca`.  Stores `:umap` (N x nc) and `:umap_obj` = (graph = SparseMatrixCSC, knns, dists) (k x N, 1-based
+indices, UMAP.jl's layout) and returns `l_inp`.
+"""
+function apply_umap!(l_inp; k=15, nc=2, md=0.1, metric=:cosine, n_epochs=300, seed=0)
+    src = haskey(l_inp, :pca_n1) && size(l_inp[:pca_n1], 2) > 1 ? l_inp[:pca_n1] : l_inp[:pca]
+    X = Matrix{Float32}(src[!, 2:end])                                              # N x r, column-major
+    N, d = size(X)
+    p = Ref(SclUmapParams(k, nc, n_epochs, umap_metric(metric), 0, 5, 100, 0, md, 1.0, 1.0, 1.0, 1.0, UInt64(seed),
+                          ntuple(_ -> Int32(0), 4)))
+    info = Ref(SclUmapInfo())
+    emb = Matrix{Float32}(undef, N, nc)
+    hr = Ref{Ptr{Cvoid}}(C_NULL)
+    cfg = Ref(default_config())
+    rc = ccall((:scl_create, LIB), Int32, (Ptr{Ptr{Cvoid}}, Ptr{SclConfig}), hr, cfg)
+    rc == 0 || check(C_NULL, rc)
+    h = hr[]
+    try
+        check(h, ccall((:scl_op_umap, LIB), Int32,
+                       (Ptr{Cvoid}, Int32, Int32, Ptr{Float32}, Ptr{SclUmapParams}, Ptr{Float32}, Ptr{Float32}, Ptr{SclUmapInfo}),
+                       h, N, d, X, p, C_NULL, emb, info))
+        nnz = Ref{Int64}(0)
+        check(h, ccall((:scl_get_umap_graph, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{UInt32}, Ptr{UInt32}, Ptr{Float32}),
+                       h, nnz, C_NULL, C_NULL, C_NULL))
+        rowptr = Vector{UInt32}(undef, N + 1); colidx = Vector{UInt32}(undef, nnz[]); val = Vector{Float32}(undef, nnz[])
+        check(h, ccall((:scl_get_umap_graph, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{UInt32}, Ptr{UInt32}, Ptr{Float32}),
+                       h, nnz, rowptr, colidx, val))
+        knns = Matrix{Int32}(undef, k, N); dists = Matrix{Float32}(undef, k, N)   # row-major N x k == column-major k x N
+        check(h, ccall((:scl_get_umap_knn, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}, Ptr{Float32}), h, knns, dists))
+        # the graph is symmetric: its CSR arrays are the CSC arrays of the same matrix
+        graph = SparseMatrixCSC(N, N, Int.(rowptr) .+ 1, Int.(colidx) .+ 1, val)
+        l_inp[:umap] = emb
+        l_inp[:umap_obj] = (graph = graph, knns = knns .+ Int32(1), dists = dists)
+    finally
+        ccall((:scl_destroy, LIB), Int32, (Ptr{Cvoid},), h)
+    end
+    l_inp
 end
 
 end # module

@@ -61,6 +61,20 @@ class Profile(C.Structure):
                 ("comm_bytes", C.c_double)]
 
 
+class UmapParams(C.Structure):
+    _fields_ = [("n_neighbors", C.c_int32), ("n_components", C.c_int32), ("n_epochs", C.c_int32), ("metric", C.c_int32),
+                ("init", C.c_int32), ("neg_sample_rate", C.c_int32), ("spectral_maxiter", C.c_int32),
+                ("reserved0", C.c_int32), ("min_dist", C.c_double), ("spread", C.c_double), ("learning_rate", C.c_double),
+                ("repulsion_strength", C.c_double), ("local_connectivity", C.c_double), ("seed", C.c_uint64),
+                ("reserved", C.c_int32 * 4)]
+
+
+class UmapInfo(C.Structure):
+    _fields_ = [("a", C.c_double), ("b", C.c_double), ("graph_nnz", C.c_int64), ("spectral_iters", C.c_int32),
+                ("init_fallback", C.c_int32), ("t_knn_ms", C.c_double), ("t_graph_ms", C.c_double),
+                ("t_init_ms", C.c_double), ("t_layout_ms", C.c_double), ("reserved", C.c_int32 * 4)]
+
+
 _u32p = C.POINTER(C.c_uint32)
 _f32p = C.POINTER(C.c_float)
 _f64p = C.POINTER(C.c_double)
@@ -132,6 +146,11 @@ SIGNATURES = {
     "scl_op_scores_from_pairs": [_f32p, C.c_int32, C.c_int32, C.c_double, _f64p, _f64p, _i32p, _i32p],
     "scl_op_denoise": [_hp, C.c_int32, C.c_int32, C.c_int32, _f32p, _f32p, _f64p, _f64p, _f64p, _f64p, _f64p, C.c_int32,
                        C.c_void_p],
+    "scl_op_knn": [_hp, C.c_int32, C.c_int32, _f32p, C.c_int32, C.c_int32, _i32p, _f32p],
+    "scl_op_umap": [_hp, C.c_int32, C.c_int32, _f32p, C.POINTER(UmapParams), _f32p, _f32p, C.POINTER(UmapInfo)],
+    "scl_get_umap_graph": [_hp, _i64p, _u32p, _u32p, _f32p],
+    "scl_get_umap_knn": [_hp, _i32p, _f32p],
+    "scl_umap_fit_ab": [C.c_double, C.c_double, _f64p, _f64p],
     "scl_bench_gram": [_hp, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _f64p, _f64p],
     "scl_bench_syevd": [_hp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _f64p],
     "scl_bench_syevd_concurrent": [_hp, C.c_int32, C.c_int32, C.c_int32, _f64p],

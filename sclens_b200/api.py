@@ -23,7 +23,7 @@ except ImportError:  # pragma: no cover
     pd = None
 
 from . import _lib
-from ._lib import Config, Profile, RobustInfo, SclError, SignalInfo, as_f32, as_u32, ptr
+from ._lib import Config, Profile, RobustInfo, SclError, SignalInfo, UmapInfo, UmapParams, as_f32, as_u32, ptr
 
 
 def df2sparr(inp_df):
@@ -259,6 +259,101 @@ class Handle:
         self._ck(self.lib.scl_get_perturbed_evec(self.h, r, ptr(V, C.c_float), ptr(L, C.c_float)))
         return V.T, L
 
+    # ---- apply_umap stages (scl_op_knn / scl_op_umap)
+    def knn(self, X, k=15, metric="cosine"):
+        """Exact kNN of the rows of X (N x d): (idx, dist), both N x k, self excluded, ascending (distance, index)."""
+        Xc = _umap_matrix(X)
+        N, d = Xc.shape[1], Xc.shape[0]
+        k, m = _umap_k(k, N), _umap_metric(metric)
+        idx, dist = np.empty((N, k), np.int32), np.empty((N, k), np.float32)
+        self._ck(self.lib.scl_op_knn(self.h, N, d, ptr(Xc, C.c_float), k, m, ptr(idx, C.c_int32), ptr(dist, C.c_float)))
+        return idx, dist
+
+    def umap(self, X, k=15, nc=2, md=0.1, metric="cosine", *, n_epochs=300, seed=0, init="spectral", init_embedding=None,
+             spread=1.0, learning_rate=1.0, repulsion_strength=1.0, neg_sample_rate=5, local_connectivity=1.0,
+             spectral_maxiter=100):
+        """UMAP_ of apply_umap! on the rows of X (N x d): returns (embedding N x nc, UmapInfo).  ``init_embedding``
+        (N x nc) replaces the computed start.  The kNN and the fuzzy graph stay on the handle (umap_graph, umap_knn)."""
+        Xc = _umap_matrix(X)
+        N, d = Xc.shape[1], Xc.shape[0]
+        p = _umap_params(N, k, nc, md, metric, n_epochs, seed, init, spread, learning_rate, repulsion_strength,
+                         neg_sample_rate, local_connectivity, spectral_maxiter)
+        ie = None
+        if init_embedding is not None:
+            ie = np.ascontiguousarray(np.asarray(init_embedding, dtype=np.float32).T)    # N x nc column-major
+            if ie.shape != (p.n_components, N) or not np.isfinite(ie).all():
+                raise ValueError("init_embedding must be a finite N x nc array")
+        out = np.empty((p.n_components, N), np.float32)
+        info = UmapInfo()
+        self._ck(self.lib.scl_op_umap(self.h, N, d, ptr(Xc, C.c_float), C.byref(p), ptr(ie, C.c_float), ptr(out, C.c_float),
+                                      C.byref(info)))
+        self.umap_N, self.umap_k = N, p.n_neighbors
+        return out.T.copy(), info
+
+    def umap_graph(self) -> sp.csr_matrix:
+        nnz = C.c_int64()
+        self._ck(self.lib.scl_get_umap_graph(self.h, C.byref(nnz), None, None, None))
+        N = self.umap_N
+        rp, ci, v = np.empty(N + 1, np.uint32), np.empty(max(1, nnz.value), np.uint32), np.empty(max(1, nnz.value), np.float32)
+        self._ck(self.lib.scl_get_umap_graph(self.h, C.byref(nnz), ptr(rp, C.c_uint32), ptr(ci, C.c_uint32), ptr(v, C.c_float)))
+        n = nnz.value
+        return sp.csr_matrix((v[:n], ci[:n].astype(np.int64), rp.astype(np.int64)), shape=(N, N))
+
+    def umap_knn(self):
+        N, k = self.umap_N, self.umap_k
+        idx, dist = np.empty((N, k), np.int32), np.empty((N, k), np.float32)
+        self._ck(self.lib.scl_get_umap_knn(self.h, ptr(idx, C.c_int32), ptr(dist, C.c_float)))
+        return idx, dist
+
+
+_UMAP_METRICS = {"euclidean": 0, "cosine": 1}
+_UMAP_INITS = {"spectral": 0, "random": 1}
+
+
+def _umap_matrix(X):
+    """N x d host matrix -> C-order d x N Float32 (== N x d column-major), checked finite."""
+    if pd is not None and isinstance(X, pd.DataFrame):
+        X = X.iloc[:, 1:].to_numpy() if X.shape[1] and X.columns[0] == "cell" else X.to_numpy()
+    X = np.asarray(X, dtype=np.float32)
+    if X.ndim != 2 or X.shape[0] < 2 or X.shape[1] < 1 or X.shape[1] > 1024:
+        raise ValueError("need an N x d matrix with N >= 2 and 1 <= d <= 1024")
+    if not np.isfinite(X).all():
+        raise ValueError("the input has non-finite entries")
+    return np.ascontiguousarray(X.T)
+
+
+def _umap_k(k, N):
+    k = int(k)
+    if not (1 <= k <= 64) or k >= N:
+        raise ValueError(f"n_neighbors must satisfy 1 <= k <= 64 and k < N (k = {k}, N = {N})")
+    return k
+
+
+def _umap_metric(metric):
+    m = getattr(metric, "lower", lambda: None)()
+    if m not in _UMAP_METRICS:
+        raise ValueError(f"metric must be one of {sorted(_UMAP_METRICS)}, got {metric!r}")
+    return _UMAP_METRICS[m]
+
+
+def _umap_params(N, k, nc, md, metric, n_epochs, seed, init, spread, learning_rate, repulsion_strength, neg_sample_rate,
+                 local_connectivity, spectral_maxiter):
+    k = _umap_k(k, N)
+    if not (1 <= int(nc) <= 16):
+        raise ValueError("nc must be in [1, 16]")
+    if init not in _UMAP_INITS:
+        raise ValueError(f"init must be one of {sorted(_UMAP_INITS)}, got {init!r}")
+    if int(n_epochs) < 0 or int(neg_sample_rate) < 0 or int(spectral_maxiter) < 0:
+        raise ValueError("n_epochs, neg_sample_rate and spectral_maxiter must be >= 0")
+    vals = dict(min_dist=float(md), spread=float(spread), learning_rate=float(learning_rate),
+                repulsion_strength=float(repulsion_strength), local_connectivity=float(local_connectivity))
+    if not all(math.isfinite(v) for v in vals.values()) or vals["min_dist"] < 0 or vals["spread"] <= 0 \
+            or vals["learning_rate"] <= 0 or vals["repulsion_strength"] < 0 or not (0 <= vals["local_connectivity"] <= k):
+        raise ValueError(f"bad UMAP parameters {vals}")
+    return UmapParams(n_neighbors=k, n_components=int(nc), n_epochs=int(n_epochs), metric=_umap_metric(metric),
+                      init=_UMAP_INITS[init], neg_sample_rate=int(neg_sample_rate), spectral_maxiter=int(spectral_maxiter),
+                      seed=int(seed) & (2 ** 64 - 1), **vals)
+
 
 def sclens(inp_df, device_="gpu", th=60, p_step=0.001, n_perturb=20, centering="mean", *, draws=None, seed=0,
            gram_mode=_lib.SCL_GRAM_FP16, exact_perturb=False, verbose=True, device=0, return_handle=False, comm=None, handle=None):
@@ -484,3 +579,47 @@ def get_denoised_df(inp_obj, device_="gpu", *, device=0, handle=None, dtype=np.f
     odf = pd.DataFrame(out.T, columns=[str(g) for g in inp_obj["gene_id"]])
     odf.insert(0, "cell", np.asarray(inp_obj["cell_id"]))
     return odf
+
+
+def apply_umap(res, k=15, nc=2, md=0.1, metric="cosine", *, n_epochs=300, seed=0, init="spectral", device=0, handle=None,
+               spread=1.0, learning_rate=1.0, repulsion_strength=1.0, neg_sample_rate=5, local_connectivity=1.0,
+               spectral_maxiter=100):
+    """Drop-in for scLENS.apply_umap! (:863-873): UMAP of the robust signals on the device.  Reads ``res["pca_n1"]``
+    when it exists and has at least one column, otherwise ``res["pca"]`` (N x r, DataFrame with a leading "cell" column
+    or array).  Stores ``res["umap"]`` (N x nc, rows in ``cell_id`` order) and ``res["umap_obj"]`` = {"graph": the
+    symmetric fuzzy graph as scipy CSR, "knns", "dists": N x k (0-based), "a", "b", "info"} and returns ``res``.
+    Exact kNN (no NN-descent) and a synchronous, deterministic epoch: the same seed gives the same embedding."""
+    def signals(key):
+        m = res.get(key)
+        if pd is not None and isinstance(m, pd.DataFrame) and "cell" in m.columns:
+            m = m.drop(columns="cell")
+        return m if m is not None and np.ndim(m) == 2 and np.shape(m)[1] >= 1 else None
+
+    src = signals("pca_n1")
+    if src is None:
+        src = signals("pca")
+    if src is None:
+        raise ValueError("the result has neither a non-empty 'pca_n1' nor a 'pca' entry")
+    X = _umap_matrix(src)
+    N = X.shape[1]
+    _umap_params(N, k, nc, md, metric, n_epochs, seed, init, spread, learning_rate, repulsion_strength, neg_sample_rate,
+                 local_connectivity, spectral_maxiter)    # every argument checked before a device is touched
+    own = handle is None
+    h = Handle(device=device) if own else handle
+    try:
+        emb, info = h.umap(X.T, k, nc, md, metric, n_epochs=n_epochs, seed=seed, init=init, spread=spread,
+                           learning_rate=learning_rate, repulsion_strength=repulsion_strength,
+                           neg_sample_rate=neg_sample_rate, local_connectivity=local_connectivity,
+                           spectral_maxiter=spectral_maxiter)
+        graph = h.umap_graph()
+        knns, dists = h.umap_knn()
+    finally:
+        if own:
+            h.close()
+    res["umap"] = emb
+    res["umap_obj"] = {"graph": graph, "knns": knns, "dists": dists, "a": info.a, "b": info.b,
+                       "info": {"graph_nnz": info.graph_nnz, "spectral_iters": info.spectral_iters,
+                                "init_fallback": info.init_fallback,
+                                "timings_ms": {"knn": info.t_knn_ms, "graph": info.t_graph_ms, "init": info.t_init_ms,
+                                               "layout": info.t_layout_ms}}}
+    return res

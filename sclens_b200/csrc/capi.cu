@@ -1,6 +1,7 @@
 // extern "C" surface of libsclens_b200.so (see include/sclens_b200.h).
 #include "nccl_dyn.h"
 #include <chrono>
+#include <cmath>
 #include <cstring>
 #include <thread>
 #include "handle.h"
@@ -982,6 +983,93 @@ int32_t scl_op_denoise(scl_handle* h, int32_t N, int32_t M, int32_t r, const flo
     SCL_CUDA(cudaMemcpyAsync(out, dout.p, bytes, cudaMemcpyDeviceToHost, h->st));
     SCL_CUDA(cudaStreamSynchronize(h->st));
   });
+}
+
+// ---- apply_umap! -----------------------------------------------------------------------------------------------------
+namespace {
+void check_umap_input(int32_t N, int32_t d, const float* X, int32_t k, int32_t metric) {
+  SCL_REQUIRE(X != nullptr, "X is NULL");
+  SCL_REQUIRE(N >= 2 && d >= 1 && d <= 1024, "bad shape");
+  SCL_REQUIRE(k >= 1 && k <= 64 && k < N, "need 1 <= n_neighbors <= 64 and n_neighbors < N");
+  SCL_REQUIRE(metric == 0 || metric == 1, "metric must be 0 (euclidean) or 1 (cosine)");
+  const size_t n = (size_t)N * d;
+  for (size_t i = 0; i < n; ++i) SCL_REQUIRE(std::isfinite(X[i]), "X has a non-finite entry");
+}
+}  // namespace
+
+int32_t scl_op_knn(scl_handle* h, int32_t N, int32_t d, const float* X, int32_t k, int32_t metric, int32_t* idx, float* dist) {
+  if (!h || !idx || !dist) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    check_umap_input(N, d, X, k, metric);
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    Tmp<float> dX((size_t)N * d, h->st);
+    Tmp<int32_t> di((size_t)N * k, h->st);
+    Tmp<float> dd((size_t)N * k, h->st);
+    SCL_CUDA(cudaMemcpyAsync(dX.p, X, (size_t)N * d * sizeof(float), cudaMemcpyHostToDevice, h->st));
+    knn_device(dX.p, N, d, k, metric, di.p, dd.p, h->st);
+    SCL_CUDA(cudaMemcpyAsync(idx, di.p, (size_t)N * k * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaMemcpyAsync(dist, dd.p, (size_t)N * k * sizeof(float), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaStreamSynchronize(h->st));
+  });
+}
+
+int32_t scl_op_umap(scl_handle* h, int32_t N, int32_t d, const float* X, const scl_umap_params* p, const float* init_embedding,
+                    float* embedding, scl_umap_info* info) {
+  if (!h || !p || !embedding || !info) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    const scl_umap_params& q = *p;
+    check_umap_input(N, d, X, q.n_neighbors, q.metric);
+    SCL_REQUIRE(q.n_components >= 1 && q.n_components <= 16, "n_components must be in [1, 16]");
+    SCL_REQUIRE(q.n_epochs >= 0 && q.init >= 0 && q.init <= 1 && q.neg_sample_rate >= 0 && q.spectral_maxiter >= 0,
+                "bad n_epochs / init / neg_sample_rate / spectral_maxiter");
+    SCL_REQUIRE(std::isfinite(q.min_dist) && q.min_dist >= 0 && std::isfinite(q.spread) && q.spread > 0,
+                "need min_dist >= 0 and spread > 0");
+    SCL_REQUIRE(std::isfinite(q.learning_rate) && q.learning_rate > 0 && std::isfinite(q.repulsion_strength) &&
+                q.repulsion_strength >= 0, "need learning_rate > 0 and repulsion_strength >= 0");
+    SCL_REQUIRE(std::isfinite(q.local_connectivity) && q.local_connectivity >= 0 && q.local_connectivity <= q.n_neighbors,
+                "need 0 <= local_connectivity <= n_neighbors");
+    const size_t ne = (size_t)N * q.n_components;
+    if (init_embedding)
+      for (size_t i = 0; i < ne; ++i) SCL_REQUIRE(std::isfinite(init_embedding[i]), "init_embedding has a non-finite entry");
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    h->have_umap_graph = false;
+    Tmp<float> dX((size_t)N * d, h->st), dI(init_embedding ? ne : 1, h->st), dE(ne, h->st);
+    SCL_CUDA(cudaMemcpyAsync(dX.p, X, (size_t)N * d * sizeof(float), cudaMemcpyHostToDevice, h->st));
+    if (init_embedding) SCL_CUDA(cudaMemcpyAsync(dI.p, init_embedding, ne * sizeof(float), cudaMemcpyHostToDevice, h->st));
+    umap_run(h, dX.p, N, d, q, init_embedding ? dI.p : nullptr, dE.p, info);
+    SCL_CUDA(cudaMemcpyAsync(embedding, dE.p, ne * sizeof(float), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaStreamSynchronize(h->st));
+  });
+}
+
+int32_t scl_get_umap_graph(scl_handle* h, int64_t* nnz, uint32_t* rowptr, uint32_t* colidx, float* val) {
+  if (!h || !nnz) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    SCL_REQUIRE(h->have_umap_graph, "scl_op_umap has not completed");
+    *nnz = (int64_t)h->ug_nnz;
+    if (rowptr && colidx && val) {
+      SCL_CUDA(cudaMemcpyAsync(rowptr, h->ug_rowptr.p, (h->ug_N + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->st));
+      SCL_CUDA(cudaMemcpyAsync(colidx, h->ug_col.p, h->ug_nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->st));
+      SCL_CUDA(cudaMemcpyAsync(val, h->ug_val.p, h->ug_nnz * sizeof(float), cudaMemcpyDeviceToHost, h->st));
+      SCL_CUDA(cudaStreamSynchronize(h->st));
+    }
+  });
+}
+
+int32_t scl_get_umap_knn(scl_handle* h, int32_t* idx, float* dist) {
+  if (!h || !idx || !dist) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    SCL_REQUIRE(h->have_umap_graph, "scl_op_umap has not completed");
+    const size_t n = (size_t)h->uk_N * h->uk_k;
+    SCL_CUDA(cudaMemcpyAsync(idx, h->uk_idx.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaMemcpyAsync(dist, h->uk_dist.p, n * sizeof(float), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaStreamSynchronize(h->st));
+  });
+}
+
+int32_t scl_umap_fit_ab(double min_dist, double spread, double* a, double* b) {
+  if (!a || !b || !std::isfinite(min_dist) || !(min_dist >= 0) || !std::isfinite(spread) || !(spread > 0)) return SCL_ERR_INVALID;
+  return guard(nullptr, [&] { umap_fit_ab(min_dist, spread, a, b); });
 }
 
 }  // extern "C"

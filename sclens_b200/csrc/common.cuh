@@ -114,6 +114,8 @@ struct NormStats {
 struct Workspace;  // sparse scratch, defined in sparse.cu
 
 // ---- sparse.cu ----
+// out[0..n] = exclusive scan of in[0..n-1], out[n] = total (one CTA)
+void exclusive_scan(const uint32_t* in, uint32_t* out, int n, cudaStream_t st);
 void build_csr_mirror(SpMat& A, cudaStream_t st);
 void upload_csc(SpMat& A, int N, int M, size_t nnz, const uint32_t* colptr, const uint32_t* rowval,
                 const float* val, int index_base, cudaStream_t st);

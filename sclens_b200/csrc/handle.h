@@ -59,6 +59,17 @@ struct scl_handle {
   std::vector<double> m_scores, sd_scores;
   std::vector<int32_t> sig_id;
   std::vector<float> gene_basis;  // [M][n_signal] (== column-major n_signal x M)
+
+  // apply_umap: kNN ([N][k], ascending (distance, index)) and fuzzy graph (symmetric CSR, sorted columns) of the last call
+  int uk_N = 0, uk_k = 0;
+  scl::DBuf<int32_t> uk_idx;
+  scl::DBuf<float> uk_dist;
+  bool have_umap_graph = false;
+  int ug_N = 0;
+  size_t ug_nnz = 0;
+  scl::DBuf<uint32_t> ug_rowptr, ug_col, ug_rev;   // ug_rev[e]: position of the reverse edge of e
+  scl::DBuf<float> ug_val;
+  scl::DBuf<double> ug_deg;
 };
 
 namespace scl {
@@ -73,6 +84,14 @@ int pass_task_step(int task, int refine_task);
 void score_from_pairs(const std::vector<float>& b_, int k, int n_pairs, double th, std::vector<double>& m,
                       std::vector<double>& sd, std::vector<int32_t>& sig);
 void plan_gram_shard(int64_t K, int64_t ld, int world, int rank, int64_t* k0, int64_t* k1);
+// umap.cu
+// exact kNN of the N x d column-major device matrix dX: d_idx / d_dist [N][k], self excluded, ascending (distance, index)
+void knn_device(const float* dX, int N, int d, int k, int metric, int32_t* d_idx, float* d_dist, cudaStream_t st);
+void umap_fit_ab(double min_dist, double spread, double* a, double* b);
+uint64_t umap_stream_key(uint64_t seed, uint32_t stream, uint32_t epoch);
+// d_init: N x nc column-major start (null: computed start); d_emb: N x nc column-major result
+void umap_run(scl_handle* h, const float* dX, int N, int d, const scl_umap_params& p, const float* d_init, float* d_emb,
+              scl_umap_info* info);
 // preprocess.cu
 bool preprocess_device(const SpMat& X, const uint8_t* d_gene_flags, const scl_qc_params& p, std::vector<int32_t>& fc_idx,
                        std::vector<int32_t>& gene_idx, SpMat& out, cudaStream_t st);

@@ -140,7 +140,7 @@ static inline int grid_for(size_t n, int threads, int cap = 148 * 16) {
   return (int)g;
 }
 
-static void exclusive_scan(const uint32_t* in, uint32_t* out, int n, cudaStream_t st) {
+void exclusive_scan(const uint32_t* in, uint32_t* out, int n, cudaStream_t st) {
   k_exclusive_scan<<<1, 1024, 0, st>>>(in, out, n);
   SCL_CUDA(cudaGetLastError());
 }

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <cmath>
 #include "handle.h"
+#include "subspace.h"
 #include "tmp.cuh"
 
 namespace scl {
@@ -27,13 +28,6 @@ constexpr double kAmpLimit = 2.0e3;
 constexpr float kGScale = 64.f;
 
 inline size_t round8(size_t x) { return (x + 7) / 8 * 8; }
-
-__host__ __device__ inline uint64_t mix64s(uint64_t x) {
-  x ^= x >> 30; x *= 0xbf58476d1ce4e5b9ull;
-  x ^= x >> 27; x *= 0x94d049bb133111ebull;
-  x ^= x >> 31;
-  return x;
-}
 
 __global__ void k_random_rows(float* __restrict__ q, int rows, int n, uint64_t seed) {
   size_t total = (size_t)rows * n;
@@ -50,7 +44,7 @@ __global__ void k_random_rows(float* __restrict__ q, int rows, int n, uint64_t s
 // S[ra][rb] += A[ra][n] * B[rb][n]^T over one slab of kSlab positions per CTA (Float64).
 // smem: sA[kSlab][pa], sB[kSlab][pb] (position-major so the 4x4 register tiles read float4).
 __global__ void __launch_bounds__(256) k_gram_ts(const float* __restrict__ A, int ra, const float* __restrict__ B, int rb,
-                                                 int n, double* __restrict__ S) {
+                                                 int n, double* __restrict__ S, double* __restrict__ part) {
   extern __shared__ float sm[];
   const int pa = ((ra + 3) / 4) * 4 + 4, pb = ((rb + 3) / 4) * 4 + 4;
   float* sA = sm;
@@ -91,8 +85,20 @@ __global__ void __launch_bounds__(256) k_gram_ts(const float* __restrict__ A, in
       for (int u = 0; u < 4; ++u)
 #pragma unroll
         for (int v = 0; v < 4; ++v)
-          if (i + u < ra && j + v < rb) atomicAdd(&S[(size_t)(i + u) * rb + j + v], acc[u][v]);
+          if (i + u < ra && j + v < rb) {
+            if (part) part[(size_t)blockIdx.x * ra * rb + (size_t)(i + u) * rb + j + v] = acc[u][v];
+            else atomicAdd(&S[(size_t)(i + u) * rb + j + v], acc[u][v]);
+          }
     }
+}
+
+// S[e] = sum over CTAs of part[cta][e], CTAs in ascending order
+__global__ void k_sum_parts(const double* __restrict__ part, int nparts, size_t ne, double* __restrict__ S) {
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < ne; e += (size_t)gridDim.x * blockDim.x) {
+    double s = 0;
+    for (int p = 0; p < nparts; ++p) s += part[(size_t)p * ne + e];
+    S[e] = s;
+  }
 }
 
 // out[c][t] = beta * base[c][t] + alpha * sum_r Tt[c][r] * In[r][t]   (Float64 accumulation)
@@ -160,26 +166,31 @@ __global__ void __launch_bounds__(256) k_residuals(const float* __restrict__ Z, 
   }
 }
 
-struct Ctx {
-  scl_handle* h;
-  cudaStream_t st;
-  int n;
-  size_t ldn;
-  const __half *g_hi, *g_lo;
-};
+}  // namespace
+
+using Ctx = BlockCtx;
 
 void gram_ts(const Ctx& c, const float* A, int ra, const float* B, int rb, double* dS) {
-  SCL_CUDA(cudaMemsetAsync(dS, 0, (size_t)ra * rb * sizeof(double), c.st));
   const int pa = ((ra + 3) / 4) * 4 + 4, pb = ((rb + 3) / 4) * 4 + 4;
   size_t smem = (size_t)kSlab * (A == B ? pa : pa + pb) * sizeof(float);
   SCL_CUDA(cudaFuncSetAttribute(k_gram_ts, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  k_gram_ts<<<(c.n + kSlab - 1) / kSlab, 256, smem, c.st>>>(A, ra, B, rb, c.n, dS);
-  count_launches(1);
+  const int grid = (c.n + kSlab - 1) / kSlab;
+  if (c.fixed_order) {
+    const size_t ne = (size_t)ra * rb;
+    Tmp<double> part((size_t)grid * ne, c.st);
+    k_gram_ts<<<grid, 256, smem, c.st>>>(A, ra, B, rb, c.n, dS, part.p);
+    k_sum_parts<<<(int)std::min<size_t>((ne + 255) / 256, 148 * 4), 256, 0, c.st>>>(part.p, grid, ne, dS);
+    count_launches(2);
+  } else {
+    SCL_CUDA(cudaMemsetAsync(dS, 0, (size_t)ra * rb * sizeof(double), c.st));
+    k_gram_ts<<<grid, 256, smem, c.st>>>(A, ra, B, rb, c.n, dS, nullptr);
+    count_launches(1);
+  }
   SCL_CUDA(cudaGetLastError());
 }
 
 void combine_rows(const Ctx& c, const float* In, int rin, const double* dTt, int rout, double alpha, const float* base,
-                  double beta, float* out, const double* wgt = nullptr) {
+                  double beta, float* out, const double* wgt) {
   size_t smem = (size_t)rin * kSlab * sizeof(float);
   SCL_CUDA(cudaFuncSetAttribute(k_combine_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   k_combine_rows<<<(c.n + kSlab - 1) / kSlab, 256, smem, c.st>>>(In, rin, dTt, rout, c.n, alpha, base, beta, out, wgt);
@@ -187,8 +198,14 @@ void combine_rows(const Ctx& c, const float* In, int rin, const double* dTt, int
   SCL_CUDA(cudaGetLastError());
 }
 
+void residual_norms(const Ctx& c, const float* Z, const float* Q, const double* dTheta, int rows, double* dRes) {
+  k_residuals<<<std::min(rows, 148 * 4), 256, 0, c.st>>>(Z, Q, dTheta, rows, c.n, dRes);
+  count_launches(1);
+  SCL_CUDA(cudaGetLastError());
+}
+
 // Z[rows][n] = (G * Q^T)^T through the tensor-core GEMM (split operands)
-void apply_G(const Ctx& c, const float* Q, int rows, float* Z) {
+static void apply_G(const Ctx& c, const float* Q, int rows, float* Z) {
   Tmp<__half> q_hi((size_t)rows * c.ldn, c.st), q_lo((size_t)rows * c.ldn, c.st);
   strided_split_f32_to_f16(Q, rows, c.n, c.n, (int64_t)c.ldn, q_hi.p, q_lo.p, c.st);
   const int cg = c.h->cfg.cta_group == 1 ? 1 : 2;
@@ -223,7 +240,6 @@ void apply_G(const Ctx& c, const float* Q, int rows, float* Z) {
   }
 }
 
-// host Cholesky S = R^T R (upper), returns Tt[c][r] = (R^-1)[r][c]; false when not positive definite
 bool chol_inverse_t(std::vector<double>& S, int b, std::vector<double>& Tt) {
   std::vector<double> R((size_t)b * b, 0.0);
   for (int j = 0; j < b; ++j) {
@@ -254,7 +270,6 @@ bool chol_inverse_t(std::vector<double>& S, int b, std::vector<double>& Tt) {
   return true;
 }
 
-// Q[rows][n] <- orthonormal basis of its row space (Cholesky QR, Float64 Gram); tmp is scratch [rows][n]
 void chol_qr(const Ctx& c, float* Q, int rows, float* tmp, int passes) {
   Tmp<double> dS((size_t)rows * rows, c.st), dT((size_t)rows * rows, c.st);
   std::vector<double> S((size_t)rows * rows), Tt;
@@ -275,8 +290,6 @@ void chol_qr(const Ctx& c, float* Q, int rows, float* tmp, int passes) {
     SCL_CUDA(cudaStreamSynchronize(c.st));
   }
 }
-
-}  // namespace
 
 void topk_subspace(scl_handle* h, const float* dG, int n, int k, float* dL, float* dV, int* iters_out) {
   cudaStream_t st = h->st;
@@ -381,9 +394,7 @@ void topk_subspace(scl_handle* h, const float* dG, int n, int k, float* dL, floa
     SCL_CUDA(cudaMemcpyAsync(dTheta.p, theta.data(), ba * sizeof(double), cudaMemcpyHostToDevice, st));
     combine_rows(c, Qa, ba, dTt.p, ba, 1.0, nullptr, 0.0, Y0.p);    // Q <- Ritz vectors
     combine_rows(c, Z.p, ba, dTt.p, ba, 1.0, nullptr, 0.0, Y1.p);   // Z <- G * Ritz vectors
-    k_residuals<<<std::min(ba, 148 * 4), 256, 0, st>>>(Y1.p, Y0.p, dTheta.p, ba, n, dRes.p);
-    count_launches(1);
-    SCL_CUDA(cudaGetLastError());
+    residual_norms(c, Y1.p, Y0.p, dTheta.p, ba, dRes.p);
     SCL_CUDA(cudaMemcpyAsync(res.data(), dRes.p, ba * sizeof(double), cudaMemcpyDeviceToHost, st));
     SCL_CUDA(cudaMemcpyAsync(Qa, Y0.p, (size_t)ba * n * sizeof(float), cudaMemcpyDeviceToDevice, st));
     SCL_CUDA(cudaStreamSynchronize(st));
