@@ -219,11 +219,12 @@ SCL_API int32_t scl_op_gram(scl_handle* h, int32_t rows, int64_t K, int64_t ld, 
 SCL_API int32_t scl_op_gemm_tn(scl_handle* h, int32_t m, int32_t n, int64_t K, int64_t lda, int64_t ldb,
                        const uint16_t* a_hi, const uint16_t* a_lo, const uint16_t* b_hi, const uint16_t* b_lo,
                        float alpha, int32_t c_colmajor, float* C);
-/* _get_eigen (:375-382): cuSOLVER syevd('V','U'), ascending. V may be NULL (values only). */
+/* _get_eigen (:375-382) on this library's own eigensolver (scl_op_syevd_tri with all vectors or none), ascending.  V may be
+ * NULL (values only); ms (may be NULL): milliseconds of the solve. */
 SCL_API int32_t scl_op_syevd(scl_handle* h, int32_t n, const float* A, float* L, float* V, double* ms);
-/* The same solve on this library's own eigensolver, the path scl_run_* use (default: the two-stage solver - dense -> band ->
- * tridiagonal, Float64 Sturm multisection + twisted factorisation, back-transformations Q2 and Q1, no library call; orders below
- * 256 or a panel that cannot be factored: own one-stage tridiagonalisation + cusolverDnSormtr; SCL_EIG_API selects).  L: all n
+/* The own eigensolver, the path scl_run_* use: the two-stage solver (dense -> band -> tridiagonal, Float64 Sturm multisection +
+ * twisted factorisation, back-transformations Q2 and Q1, no library call); orders below 256 or a panel that cannot be factored:
+ * own one-stage tridiagonalisation (cusolverDnSsytrd where it declines) + cusolverDnSormtr.  L: all n
  * eigenvalues ascending; V: the eigenvectors with ascending 0-based indices [v0, v1) as the columns of an n x (v1 - v0) column-major
  * array (vector v at V + (v - v0) n; v0 == v1: values only, V may be NULL).  out (may be NULL): out[0..2] = milliseconds of [reduction to tridiagonal form, tridiagonal eigenproblem, back-transformation + copy], out[3..5] =
  * [eigenvalue clusters re-solved by inverse iteration, eigenvalues in such clusters, 1 if the solve fell back to Ssyevd]. */
@@ -331,21 +332,14 @@ SCL_API int32_t scl_bench_gram(scl_handle* h, int32_t rows, int64_t K, int32_t m
  * own tridiagonal stage with all vectors / the vectors il..iu / values only.  mode + 16: solve the data Gram matrix of the
  * last scl_run_signal (needs n == nm) instead of the synthetic one. */
 SCL_API int32_t scl_bench_syevd(scl_handle* h, int32_t n, int32_t mode, int32_t il, int32_t iu, double* ms);
-/* `nsolves` independent Ssyevd solves (mode 0: with vectors, 1: values only) of n x n Wishart matrices issued at the same
- * time from `nsolves` host threads, each with its own stream and cuSOLVER handle; ms_wall = host wall time until all
- * are done (after one untimed round).  Answers whether independent eigensolves (sparsity-search steps) overlap on ONE GPU. */
+/* `nsolves` independent solves on the own eigensolver (as scl_op_syevd; mode 0: with vectors, 1: values only) of n x n
+ * Wishart matrices issued at the same time from `nsolves` host threads, each with its own stream and solver; ms_wall = host
+ * wall time until all are done (after one untimed round).  Answers whether independent eigensolves (sparsity-search steps)
+ * overlap on ONE GPU. */
 SCL_API int32_t scl_bench_syevd_concurrent(scl_handle* h, int32_t n, int32_t nsolves, int32_t mode, double* ms_wall);
-/* Tuning studies only (process-wide).  stat_variant: launch shape of the statistics passes (0-7: line passes,
- * 8: strip passes; < 0 keeps the current one).  stat_heavy: line length above which a whole CTA takes a line
- * (<= 0 keeps).  writer: dense writer, -1 automatic, 0 register/overlay writer, 1 TMA bulk-store writer, 2 / 3
- * TMA bulk-store writer with one / two cp.async-staged entries per thread and line (<= -2 keeps).  Results are
- * identical for every setting. */
-/* Which eigensolver path runs (process-wide; the environment variable SCL_EIG_API sets the same bits): 0 = plain
- * cusolverDnSsyevd; bit 0 Xsyevd; bit 1 Ssyevdx in the search steps; bit 2 own tridiagonal stage (tridiag.cu) between Ssytrd
- * and Sormtr; bit 3 (with 2) index-range vectors in the search steps; bit 4 (with 2) own tridiagonalisation (sytrd.cu).
- * bit 5 (with 2) two-stage reduction (dense -> band -> tridiagonal, sy2sb.cu / sb2st.cu / backtrans.cu) for orders >= 256.
- * v < 0: back to the environment / default. */
-SCL_API int32_t scl_debug_set_eig_api(int32_t v);
+/* Test hook (process-wide): on != 0 makes the own eigensolver take the one-stage path at every order, 0 restores the
+ * choice by order. */
+SCL_API int32_t scl_debug_force_one_stage(int32_t on);
 /* Stage times of the handle's last own-path eigensolve, milliseconds: out[0..4] = dense->band, band->tridiagonal, tridiagonal
  * eigenproblem, stage-2 back-transformation, stage-1 back-transformation (all 0 unless the two-stage path ran); out[5] = 1 when
  * the two-stage path produced the result; out[6] = number of two-stage solves of this handle that fell back to one stage;
@@ -354,17 +348,17 @@ SCL_API int32_t scl_debug_last_solve(scl_handle* h, double out[8]);
 /* Totals over the handle's two-stage solves since scl_reset_profile, milliseconds: out[0..4] = the five stages as above; out[5] =
  * number of two-stage solves; out[6] = eigenvector columns back-transformed; out[7] = solves that fell back to one stage. */
 SCL_API int32_t scl_debug_eig_stage_totals(scl_handle* h, double out[8]);
-/* Kernel variants of the two-stage solver, for the parity tests (process-wide; a negative value restores the environment /
- * default): q2_variant 0 shared-memory window, 1 register-stationary three-term TF32, 2 register-stationary split binary16
- * (SCL_Q2_VARIANT); stage1_engine 0 FP32 FMA, 1 three-term TF32 mma.sync (SCL_TILE_ENGINE); q1_engine 0 FP32 FMA, 1 TF32 mma.sync,
- * 2 split-binary16 mma.sync, 3 eight-panel block reflectors on the tcgen05 GEMM (SCL_TILE_ENGINE_Q1). */
-SCL_API int32_t scl_debug_set_two_stage(int32_t q2_variant, int32_t stage1_engine, int32_t q1_engine);
 /* The stages of the two-stage reduction one by one on a host matrix A (n x n, symmetric, n a multiple of 4), for the stage-wise
  * parity tests: AB (n x 128, band storage AB[j*128 + (i-j)]) after dense -> band; d (n), e (n-1) after band -> tridiagonal;
  * Q2 (n x n, column v at Q2 + v*n) = the stage-2 transformation applied to the identity; Q (same layout) = Q1 Q2.  Any output
  * pointer may be NULL.  flags[0] = panel failure flag, flags[1] = number of panels. */
 SCL_API int32_t scl_debug_two_stage(scl_handle* h, int32_t n, const float* A, float* AB, float* d, float* e, float* Q2, float* Q,
                                     int32_t flags[2]);
+/* Tuning studies only (process-wide).  stat_variant: launch shape of the statistics passes (0-7: line passes,
+ * 8: strip passes; < 0 keeps the current one).  stat_heavy: line length above which a whole CTA takes a line
+ * (<= 0 keeps).  writer: dense writer, -1 automatic, 0 register/overlay writer, 1 TMA bulk-store writer, 2 / 3
+ * TMA bulk-store writer with one / two cp.async-staged entries per thread and line (<= -2 keeps).  Results are
+ * identical for every setting. */
 SCL_API int32_t scl_debug_set_tuning(int32_t stat_variant, int32_t stat_heavy, int32_t writer);
 SCL_API int32_t scl_bench_normalize(scl_handle* h, int32_t layout, int32_t with_lo, int32_t reps, double* ms_stats,
                             double* ms_densify, double* alg_bytes_densify);

@@ -154,10 +154,9 @@ SIGNATURES = {
     "scl_bench_gram": [_hp, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _f64p, _f64p],
     "scl_bench_syevd": [_hp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _f64p],
     "scl_bench_syevd_concurrent": [_hp, C.c_int32, C.c_int32, C.c_int32, _f64p],
-    "scl_debug_set_eig_api": [C.c_int32],
+    "scl_debug_force_one_stage": [C.c_int32],
     "scl_debug_last_solve": [_hp, _f64p],
     "scl_debug_eig_stage_totals": [_hp, _f64p],
-    "scl_debug_set_two_stage": [C.c_int32, C.c_int32, C.c_int32],
     "scl_debug_two_stage": [_hp, C.c_int32, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.POINTER(C.c_int32)],
     "scl_debug_set_tuning": [C.c_int32, C.c_int32, C.c_int32],
     "scl_bench_normalize": [_hp, C.c_int32, C.c_int32, C.c_int32, _f64p, _f64p, _f64p],

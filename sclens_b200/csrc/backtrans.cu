@@ -5,13 +5,13 @@
 // one block I - V T V'.  Generation order is sweep-major; reflectors (s, k) and (s', k') with s < s', k < k' act on disjoint
 // rows, so inside a group of sweeps the product may be taken level by level, and the eigenvectors see: groups descending,
 // levels ascending inside a group (oracle/two_stage_ref.py: apply_q2 == apply_q2_plain).  Every eigenvector is independent:
-// a CTA owns a slab of vectors, keeps the 127-row window of its slab in shared memory (consecutive levels overlap in 63
-// rows, which never leave the SM), and walks all blocks.
-// Q1 (stage-1 panels): Z[r0:] -= (V T) (V' Z[r0:]) panel by panel, last panel first, on the FP32 tile engine (V T was stored by
-// stage 1 in the upper triangle of A).
+// a warp owns 16 vectors, keeps their 128-row window in registers and walks all blocks (k_q2_apply_h, split binary16 on
+// mma.sync).
+// Q1 (stage-1 panels, V T stored by stage 1 in the upper triangle of A): for 64 vectors or more, eight panels at a time as one
+// block reflector on the tcgen05 GEMM of gemm_umma.cu (apply_q1_umma); for fewer, Z[r0:] -= (V T) (V' Z[r0:]) panel by panel,
+// last panel first, on the split-binary16 tile engine of sgemm_tile.cuh.
 #include <cuda_fp16.h>
 #include <algorithm>
-#include <cstdlib>
 #include "common.cuh"
 #include "sgemm_tile.cuh"
 #include "tmp.cuh"
@@ -19,298 +19,10 @@
 
 namespace scl {
 
-std::atomic<int> g_two_stage_override[3] = {{-1}, {-1}, {-1}};
-
 namespace {
 
 constexpr int B = kBand;
-constexpr int VS = 68;   // shared-memory stride of the reflector block and of T
 
-// T factor (row-major, upper triangular) of every (group, level) block of stage-2 reflectors
-__global__ void __launch_bounds__(256) k_q2_tfactor(const float* __restrict__ V2, long long ldv2, const float* __restrict__ tau2,
-                                                    long long ldt2, int n, int nlev, float* __restrict__ Tq) {
-  const int k = (int)blockIdx.x, G = (int)blockIdx.y, s0 = G * B;
-  if (s0 + 1 + B * k > n - 2) return;
-  __shared__ float Vc[B][B + 1], T[B][B + 1];   // T: upper triangle = T, strictly lower triangle = the Gram matrix W (W[a][b] at T[b][a])
-  __shared__ float tau[B];
-  const int tid = (int)threadIdx.x;
-  for (int e = tid; e < B * B; e += 256) {
-    const int j = e / B, i = e % B, s = s0 + j;
-    Vc[j][i] = s < n - 2 ? V2[(size_t)s * ldv2 + (size_t)k * B + i] : 0.f;
-    if (j <= i) T[j][i] = 0.f;
-  }
-  if (tid < B) tau[tid] = s0 + tid < n - 2 ? tau2[(size_t)(s0 + tid) * ldt2 + k] : 0.f;
-  __syncthreads();
-  // W[a][b] = v_a . v_b for a < b: reflector b sits b - a rows below reflector a
-  for (int e = tid; e < B * B; e += 256) {
-    const int a = e / B, b = e % B;
-    if (a < b) {
-      const int sh = b - a;
-      float s = 0.f;
-      for (int i = 0; i + sh < B; ++i) s = fmaf(Vc[a][i + sh], Vc[b][i], s);
-      T[b][a] = s;
-    }
-  }
-  __syncthreads();
-  // forward columnwise larft: T[0:j, j] = -tau_j T[0:j, 0:j] W[0:j, j]
-  for (int j = 0; j < B; ++j) {
-    if (tid < j) {
-      float s = 0.f;
-      for (int q = tid; q < j; ++q) s = fmaf(T[tid][q], T[j][q], s);
-      T[tid][j] = -tau[j] * s;
-    } else if (tid == j) {
-      T[j][j] = tau[j];
-    }
-    __syncthreads();
-  }
-  float* out = Tq + ((size_t)G * nlev + k) * B * B;
-  for (int e = tid; e < B * B; e += 256) out[e] = (e / B) <= (e % B) ? T[e / B][e % B] : 0.f;   // out[c][c'] = T[c][c'], upper triangular
-}
-
-struct Q2Args {
-  const float* V2;
-  long long ldv2;
-  const float* Tq;
-  int n, nlev, ngroups;
-  float* Z;
-  long long ldz;
-  int mvec, nv, nvp;
-};
-
-__device__ __forceinline__ void cp_async4(float* dst, const float* src, bool valid) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
-  const int sz = valid ? 4 : 0;   // src-size 0: the destination is zero-filled, the source is not read
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(d), "l"(src), "r"(sz) : "memory");
-}
-__device__ __forceinline__ void cp_async16(float* dst, const float* src) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-
-// Tensor-core products in error-compensated TF32 (mma.sync m16n8k8): x = hi + lo with hi = tf32(x), lo = tf32(x - hi), and
-// a b ~ a_lo b_hi + a_hi b_lo + a_hi b_hi accumulated in FP32 - FP32-level accuracy (relative 2^-21) with FP32 range, so the
-// reflectors and eigenvectors need no scaling.  The three products of a block have ~230 000 scalar FMAs per CTA; as MMAs
-// they are ~2 700 instructions.
-// (split_tf32 / mma_tf32 / mma_tf32_zero: sgemm_tile.cuh; the rounding is two integer operations per value instead of the
-// dozen instructions cvt.rna.tf32.f32 expands to - the conversions were 60 % of this kernel's instructions)
-using tile::mma_tf32;
-using tile::mma_tf32_zero;
-using tile::split_tf32;
-// d (16 x 8 tiles j < NJ) += A (16 x 8, fragment from a0..a3) * B_j (8 x 8): pb = &B[k = t][n = g] of tile 0, tiles 8 columns apart,
-// rows k and k + 4 at pb and pb4
-constexpr int kMaxNJ = 6;
-__device__ __forceinline__ void mma_row(float (&acc)[kMaxNJ][4], int nj, float a0, float a1, float a2, float a3, const float* pb,
-                                        const float* pb4) {
-  uint32_t ahi[4], alo[4];
-  split_tf32(a0, ahi[0], alo[0]);
-  split_tf32(a1, ahi[1], alo[1]);
-  split_tf32(a2, ahi[2], alo[2]);
-  split_tf32(a3, ahi[3], alo[3]);
-#pragma unroll
-  for (int j = 0; j < kMaxNJ; ++j) {
-    if (j < nj) {
-      uint32_t bhi[2], blo[2];
-      split_tf32(pb[8 * j], bhi[0], blo[0]);
-      split_tf32(pb4[8 * j], bhi[1], blo[1]);
-      float d[4];
-      mma_tf32_zero(d, alo, bhi);
-      mma_tf32(d, ahi, blo);
-      mma_tf32(d, ahi, bhi);
-      acc[j][0] += d[0]; acc[j][1] += d[1]; acc[j][2] += d[2]; acc[j][3] += d[3];
-    }
-  }
-}
-
-// 256 threads.  Warp w works on reflector rows / window rows given by (w & 3) and on the half (w >> 2) of the CTA's vectors
-// (8-vector tiles; nvp = 8 (mod 16), which also keeps the B fragments - 4 rows x 8 vectors per load - on 32 different banks).
-// Everything a block needs from global memory - its reflectors (scattered into the parallelogram), its T factor and the 64
-// window rows that enter - is fetched with cp.async while the previous block is being multiplied (double-buffered V / T, a
-// staging area for the rows); only the first block of a group of sweeps waits for its loads.
-__global__ void __launch_bounds__(256, 1) k_q2_apply(Q2Args a) {
-  extern __shared__ __align__(16) float sm[];
-  const int nvp = a.nvp;
-  float* Zs = sm;                        // [128][nvp]  window rows (slot = window row & 127, see below) x vectors
-  float* Xs = Zs + 128 * nvp;            // [64][nvp]
-  float* X2s = Xs + B * nvp;             // [64][nvp]
-  float* Zst = X2s + B * nvp;            // [64][nvp]   rows entering the window at the next level
-  float* Vs0 = Zst + B * nvp;            // [2][128][VS] parallelogram: Vs[j + i][j] = v_j[i]
-  float* Tt0 = Vs0 + 2 * 128 * VS;       // [2][64][VS]
-  const int tid = (int)threadIdx.x, nthr = (int)blockDim.x;
-  const int lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
-  const int ntile = nvp / 8, nhalf = (ntile + 1) / 2;
-  const int nbase = (warp >> 2) * nhalf, nj = (warp >> 2) ? ntile - nhalf : nhalf;   // this warp's vector tiles
-  const int vb = 8 * nbase;
-  const int vec0 = (int)blockIdx.x * a.nv, nvv = min(a.nv, a.mvec - vec0);
-  const int n = a.n;
-  for (int e = tid; e < 2 * 128 * VS; e += nthr) Vs0[e] = 0.f;
-  for (int e = tid; e < 128 * nvp; e += nthr) Zs[e] = 0.f;
-  __syncthreads();
-  // reflectors and T of block (G, k) into buffer `buf`
-  auto fetch_vt = [&](int G, int k, int buf) {
-    float* Vs = Vs0 + buf * 128 * VS;
-    float* Tt = Tt0 + buf * B * VS;
-    const int s0 = G * B;
-    for (int j = warp; j < B; j += 8) {
-      const int s = s0 + j;
-      const bool ok = s < n - 2;
-      const float* src = ok ? a.V2 + (size_t)s * a.ldv2 + (size_t)k * B : a.V2;
-      cp_async4(&Vs[(j + lane) * VS + j], ok ? src + lane : src, ok);
-      cp_async4(&Vs[(j + lane + 32) * VS + j], ok ? src + lane + 32 : src, ok);
-    }
-    const float* tq = a.Tq + ((size_t)G * a.nlev + k) * B * B;
-    for (int e = tid; e < B * B / 4; e += nthr) cp_async16(&Tt[(e / (B / 4)) * VS + (e % (B / 4)) * 4], tq + (size_t)e * 4);   // Tt[c][c']
-  };
-  // window rows [w0, w0 + nrow) of the window starting at global row rlo: staging area dst[(w - w0)][v], or the window's own slots
-  auto fetch_rows = [&](int rlo, int w0, int nrow, float* dst, int slot0, bool to_slots) {
-    for (int v = warp; v < nvp; v += 8) {
-      const float* src = a.Z + (size_t)(vec0 + min(v, nvv - 1)) * a.ldz + rlo + w0;
-      for (int w = lane; w < nrow; w += 32) {
-        const bool ok = v < nvv && rlo + w0 + w < n;
-        float* d = to_slots ? &Zs[((slot0 + w0 + w) & 127) * nvp + v] : &dst[w * nvp + v];
-        cp_async4(d, ok ? src + w : a.Z, ok);
-      }
-    }
-  };
-  int blk = 0;
-  for (int G = a.ngroups - 1; G >= 0; --G) {
-    const int s0 = G * B, base = s0 + 1;   // window row w of level k is global row base + 64 k + w, kept in slot (64 k + w) & 127
-    if (base > n - 2) continue;
-    // the group's first block: nothing to overlap with
-    fetch_vt(G, 0, blk & 1);
-    fetch_rows(base, 0, 127, nullptr, 0, true);
-    cp_async_commit();
-    for (int k = 0;; ++k, ++blk) {
-      const int rlo = base + B * k;
-      const bool last = rlo + B > n - 2;
-      const float* Vs = Vs0 + (blk & 1) * 128 * VS;
-      const float* Tt = Tt0 + (blk & 1) * B * VS;
-      cp_async_wait_all();
-      __syncthreads();
-      if (!last) {
-        fetch_vt(G, k + 1, (blk + 1) & 1);
-        fetch_rows(rlo + B, B - 1, B, Zst, 0, false);
-        cp_async_commit();
-      }
-      // ---- X[c][vec] = sum_w V[w][c] Z[w][vec]: 16 reflectors c0.. per warp, window rows c0 .. c0 + 79 (w in [c, c + 63])
-      {
-        float acc[kMaxNJ][4];
-#pragma unroll
-        for (int j = 0; j < kMaxNJ; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
-        const int c0 = 16 * (warp & 3);
-#pragma unroll 2
-        for (int ks = 0; ks < 10; ++ks) {
-          const int w0 = c0 + 8 * ks;
-          const float* va = &Vs[(w0 + t) * VS + c0 + g];   // A[m = c][k = w] = V[w][c]
-          const float* zb = &Zs[((B * k + w0 + t) & 127) * nvp + vb + g];
-          const float* zb4 = &Zs[((B * k + w0 + t + 4) & 127) * nvp + vb + g];
-          mma_row(acc, nj, va[0], va[8], va[4 * VS], va[4 * VS + 8], zb, zb4);
-        }
-#pragma unroll
-        for (int j = 0; j < kMaxNJ; ++j)
-          if (j < nj) {
-            *reinterpret_cast<float2*>(&Xs[(c0 + g) * nvp + vb + 8 * j + 2 * t]) = make_float2(acc[j][0], acc[j][1]);
-            *reinterpret_cast<float2*>(&Xs[(c0 + g + 8) * nvp + vb + 8 * j + 2 * t]) = make_float2(acc[j][2], acc[j][3]);
-          }
-      }
-      __syncthreads();
-      // ---- X2[c][vec] = sum_{c' >= c} T[c][c'] X[c'][vec]
-      {
-        float acc[kMaxNJ][4];
-#pragma unroll
-        for (int j = 0; j < kMaxNJ; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
-        const int c0 = 16 * (warp & 3);
-        for (int k0 = c0; k0 < B; k0 += 8) {
-          const float* ta = &Tt[(c0 + g) * VS + k0 + t];   // A[m = c][k = c'] = T[c][c']
-          const float* xb = &Xs[(k0 + t) * nvp + vb + g];
-          mma_row(acc, nj, ta[0], ta[8 * VS], ta[4], ta[8 * VS + 4], xb, xb + 4 * nvp);
-        }
-#pragma unroll
-        for (int j = 0; j < kMaxNJ; ++j)
-          if (j < nj) {
-            *reinterpret_cast<float2*>(&X2s[(c0 + g) * nvp + vb + 8 * j + 2 * t]) = make_float2(acc[j][0], acc[j][1]);
-            *reinterpret_cast<float2*>(&X2s[(c0 + g + 8) * nvp + vb + 8 * j + 2 * t]) = make_float2(acc[j][2], acc[j][3]);
-          }
-      }
-      __syncthreads();
-      // ---- Z[w][vec] -= sum_c V[w][c] X2[c][vec]: window rows 16 mt .. 16 mt + 15 need c in [16 mt - 63, 16 mt + 15]; a warp takes the
-      // row tiles p and p + 4 (2 + 8, 4 + 6, ... = 10 steps of 8 reflectors each way)
-#pragma unroll 1
-      for (int half = 0; half < 2; ++half) {
-        const int mt = (warp & 3) + 4 * half, w0 = 16 * mt;
-        float acc[kMaxNJ][4];
-#pragma unroll
-        for (int j = 0; j < kMaxNJ; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
-        const int clo = max(0, w0 - (B - 1)) & ~7, chi = min(B - 1, w0 + 15);
-        for (int c = clo; c <= chi; c += 8) {
-          const float* va = &Vs[(w0 + g) * VS + c + t];   // A[m = w][k = c] = V[w][c]
-          const float* xb = &X2s[(c + t) * nvp + vb + g];
-          mma_row(acc, nj, va[0], va[8 * VS], va[4], va[8 * VS + 4], xb, xb + 4 * nvp);
-        }
-#pragma unroll
-        for (int j = 0; j < kMaxNJ; ++j)
-          if (j < nj) {
-            float2* z0 = reinterpret_cast<float2*>(&Zs[((B * k + w0 + g) & 127) * nvp + vb + 8 * j + 2 * t]);
-            float2* z1 = reinterpret_cast<float2*>(&Zs[((B * k + w0 + g + 8) & 127) * nvp + vb + 8 * j + 2 * t]);
-            float2 u = *z0, v2 = *z1;
-            u.x -= acc[j][0]; u.y -= acc[j][1];
-            v2.x -= acc[j][2]; v2.y -= acc[j][3];
-            *z0 = u;
-            *z1 = v2;
-          }
-      }
-      __syncthreads();
-      // ---- rows leaving the window go back to global memory (everything at the group's last level)
-      {
-        const int nrow = last ? 127 : B;
-        for (int v = warp; v < nvv; v += 8) {
-          float* dst = a.Z + (size_t)(vec0 + v) * a.ldz + rlo;
-          for (int w = lane; w < nrow; w += 32)
-            if (rlo + w < n) dst[w] = Zs[((B * k + w) & 127) * nvp + v];
-        }
-      }
-      if (last) {
-        ++blk;
-        __syncthreads();
-        break;
-      }
-      // ---- the prefetched rows take the slots of the rows that just left: window rows 63..126 of level k + 1
-      cp_async_wait_all();
-      __syncthreads();
-      for (int w = warp; w < B; w += 8) {
-        float* d = &Zs[((B * (k + 1) + B - 1 + w) & 127) * nvp];
-        const float* sr = &Zst[w * nvp];
-        for (int v = lane; v < nvp; v += 32) d[v] = sr[v];
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------- Q2, register-stationary variant
-// The window of a slab never leaves the register file.  A warp owns 16 eigenvectors and keeps their 128-row window as the
-// accumulator fragments of sixteen m16n8 tiles (vectors = the M dimension, window rows = N).  With vectors on M, the C/D
-// fragment of a tile (thread (g, t): rows g and g + 8, columns 2t and 2t + 1) IS an A fragment of the next product once the
-// contraction index is read as k = t <-> column 2t, k = t + 4 <-> column 2t + 1, and the same permutation is applied to the
-// rows of the B operand when it is fetched.  So  X' = Z' V  ->  X2' = X' T'  ->  Z' -= X2' V'  chain through registers:
-// no shared-memory window, no CTA-wide barrier, and the only operands that come from shared memory are the reflector block
-// and its T factor.  Those are the same for every warp and every vector, so a pre-pass (k_q2_images) writes them once, already
-// split into TF32 (hi, lo) pairs and already in the shared-memory layout, and one elected thread streams one 72 KB image per
-// block through a three-stage cp.async.bulk ring (mbarrier full / empty pairs); warps never wait for each other except
-// through that ring.  Layout of an image: four planes of 64 rows x 72 floats - hi and lo parts of P[c][u] = V[w = u + 8 (c / 8)][c]
-// (72 entries per reflector c: the nine 8-row steps that meet the 8-reflector tile of c), hi and lo parts of T[c][c'].  The
-// B operand of an MMA is a pair of consecutive registers, so a fragment fetched as one 8-byte load from a plane (two
-// consecutive rows of one reflector: the first product and the T product) needs no register moves; the last product reads
-// one row of two consecutive reflectors with 4-byte loads.  Bit 3 of u is flipped by bit 2 of c, which keeps both patterns
-// free of bank conflicts (the last eight entries of a row are not swizzled: a 2-way conflict in one step of nine).
-// Accumulation: the tensor core adds with truncation, so the leading term a_hi b_hi of every step starts from a zero
-// accumulator and is added to the running sum with a rounded FP32 add; the two cross terms, 2^-11 of it, are chained in
-// tensor-core accumulators of their own (their truncation is 2^-35 of the result), which also keeps the dependent chains short.
-constexpr int kImgRow = 72;                     // floats per plane row
-constexpr int kPlane = B * kImgRow;             // 4608 floats per plane
-constexpr int kBlkFloats = 4 * kPlane;          // P hi, P lo, T hi, T lo: 73 728 bytes
-constexpr int kBlkBytes = kBlkFloats * 4;
-constexpr int kStages = 3;
 static_assert(B == 64, "the register-stationary kernel is written for a half bandwidth of 64");
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -340,90 +52,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                : "memory");
 }
 
-__device__ __host__ __forceinline__ int q2_swz(int c) { return ((c >> 2) & 1) << 3; }
-
-// Pre-pass: T factor of block (G, k) as in k_q2_tfactor, then the block's two images at its place in processing order
-// (groups descending, levels ascending: block index (q - G)(q - G + 1) / 2 + k with q = the last group).
-__global__ void __launch_bounds__(256) k_q2_images(const float* __restrict__ V2, long long ldv2, const float* __restrict__ tau2,
-                                                   long long ldt2, int n, int q, float* __restrict__ Img) {
-  const int k = (int)blockIdx.x, G = (int)blockIdx.y, s0 = G * B;
-  if (s0 + 1 + B * k > n - 2) return;
-  __shared__ float Vc[B][B + 1], T[B][B + 1];
-  __shared__ float tau[B];
-  const int tid = (int)threadIdx.x;
-  for (int e = tid; e < B * B; e += 256) {
-    const int j = e / B, i = e % B, s = s0 + j;
-    Vc[j][i] = s < n - 2 ? V2[(size_t)s * ldv2 + (size_t)k * B + i] : 0.f;
-    if (j <= i) T[j][i] = 0.f;
-  }
-  if (tid < B) tau[tid] = s0 + tid < n - 2 ? tau2[(size_t)(s0 + tid) * ldt2 + k] : 0.f;
-  __syncthreads();
-  for (int e = tid; e < B * B; e += 256) {
-    const int a = e / B, b = e % B;
-    if (a < b) {
-      const int sh = b - a;
-      float s = 0.f;
-      for (int i = 0; i + sh < B; ++i) s = fmaf(Vc[a][i + sh], Vc[b][i], s);
-      T[b][a] = s;
-    }
-  }
-  __syncthreads();
-  for (int j = 0; j < B; ++j) {
-    if (tid < j) {
-      float s = 0.f;
-      for (int qq = tid; qq < j; ++qq) s = fmaf(T[tid][qq], T[j][qq], s);
-      T[tid][j] = -tau[j] * s;
-    } else if (tid == j) {
-      T[j][j] = tau[j];
-    }
-    __syncthreads();
-  }
-  float* img = Img + ((size_t)(q - G) * (q - G + 1) / 2 + k) * kBlkFloats;
-  for (int e = tid; e < B * kImgRow; e += 256) {
-    const int c = e / kImgRow, u = e % kImgRow;
-    const int i = u + 8 * (c >> 3) - c - 1;   // window row w = u + 8 (c / 8) is entry w - c - 1 of reflector c
-    const float x = (i >= 0 && i < B) ? Vc[c][i] : 0.f;
-    const int up = u < 64 ? (u ^ q2_swz(c)) : u;
-    uint32_t hi, lo;
-    split_tf32(x, hi, lo);
-    img[c * kImgRow + up] = __uint_as_float(hi);
-    img[kPlane + c * kImgRow + up] = __uint_as_float(lo);
-    const float tv = (u < B && c <= u) ? T[c][u] : 0.f;
-    split_tf32(tv, hi, lo);
-    img[2 * kPlane + c * kImgRow + u] = __uint_as_float(hi);
-    img[3 * kPlane + c * kImgRow + u] = __uint_as_float(lo);
-  }
-}
-
-struct Q2RsArgs {
-  const float* Img;
-  float* Z;
-  long long ldz;
-  int n, mvec, q, tiles, base, extra;   // CTA b owns base + (b < extra) 16-vector tiles
-};
-
-__device__ __forceinline__ void split_frag(const float (&r)[4], uint32_t (&ah)[4], uint32_t (&al)[4]) {
-  split_tf32(r[0], ah[0], al[0]);   // (g, k = t)      <- column 2t
-  split_tf32(r[2], ah[1], al[1]);   // (g + 8, k = t)
-  split_tf32(r[1], ah[2], al[2]);   // (g, k = t + 4)  <- column 2t + 1
-  split_tf32(r[3], ah[3], al[3]);
-}
-__device__ __forceinline__ void ld_b2(uint32_t (&b)[2], const float* p) {
-  const float2 v = *reinterpret_cast<const float2*>(p);
-  b[0] = __float_as_uint(v.x);
-  b[1] = __float_as_uint(v.y);
-}
-// acc += a_hi b_hi from a zero accumulator; cross (+)= a_lo b_hi + a_hi b_lo
-template <bool kFirst>
-__device__ __forceinline__ void mma_step(float (&acc)[4], float (&cross)[4], const uint32_t (&ah)[4], const uint32_t (&al)[4],
-                                         const uint32_t (&bh)[2], const uint32_t (&bl)[2], float sign) {
-  float d[4];
-  mma_tf32_zero(d, ah, bh);
-  if (kFirst) mma_tf32_zero(cross, al, bh);
-  else mma_tf32(cross, al, bh);
-  mma_tf32(cross, ah, bl);
-  acc[0] = fmaf(sign, d[0], acc[0]); acc[1] = fmaf(sign, d[1], acc[1]); acc[2] = fmaf(sign, d[2], acc[2]); acc[3] = fmaf(sign, d[3], acc[3]);
-}
 __device__ __forceinline__ void ld_rows(float (&r)[4], const float* za, const float* zb, bool oka, bool okb, int row, int n) {
   float2 u = make_float2(0.f, 0.f), v = u;
   if (row + 1 < n) {
@@ -445,175 +73,30 @@ __device__ __forceinline__ void st_rows(const float (&r)[4], float* za, float* z
   }
 }
 
-template <int MAXW>
-__global__ void __launch_bounds__(MAXW * 32, 1) k_q2_apply_rs(Q2RsArgs a) {
-  extern __shared__ __align__(16) float sm[];
-  uint64_t* full = reinterpret_cast<uint64_t*>(sm + kStages * kBlkFloats);
-  uint64_t* empty = full + kStages;
-  const int tid = (int)threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
-  const int cta = (int)blockIdx.x;
-  const int ntile = a.base + (cta < a.extra ? 1 : 0);
-  const int tile0 = cta * a.base + min(cta, a.extra);
-  if (tid == 0) {
-    for (int s = 0; s < kStages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], (uint32_t)ntile);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  if (warp >= ntile) return;
-  const int q = a.q, n = a.n;
-  const int nblk = (q + 1) * (q + 2) / 2;
-  if (tid == 0) {
-    for (int b = 0; b < 2 && b < nblk; ++b) {
-      mbar_arrive_expect_tx(&full[b], kBlkBytes);
-      bulk_g2s(sm + b * kBlkFloats, a.Img + (size_t)b * kBlkFloats, kBlkBytes, &full[b]);
-    }
-  }
-  const int va = (tile0 + warp) * 16 + g, vb = va + 8;
-  const bool oka = va < a.mvec, okb = vb < a.mvec;
-  float* za = a.Z + (size_t)(oka ? va : 0) * a.ldz;
-  float* zb = a.Z + (size_t)(okb ? vb : 0) * a.ldz;
-  // thread-constant offsets (floats) into a plane, see the layout above: even / odd 8-row steps, the unswizzled last step
-  const int gb = (g >> 2) & 1, tb = (t >> 1) & 1;
-  const int offA = g * kImgRow + 2 * t, offAe = offA + 8 * gb, offAo = offA - 8 * gb;
-  const int offB = 2 * t * kImgRow + g, offBe = offB + 8 * tb, offBo = offB - 8 * tb;
-  float z[16][4];
-  int b = 0;
-  for (int G = q; G >= 0; --G) {
-    const int nl = q - G + 1;
-    int R0 = B * G;   // the window of level k holds rows R0 .. R0 + 127 (reflector c of the block acts on window rows c + 1 .. c + 64)
-#pragma unroll
-    for (int i = 0; i < 16; ++i) ld_rows(z[i], za, zb, oka, okb, R0 + 8 * i + 2 * t, n);
-    for (int k = 0; k < nl; ++k, ++b, R0 += B) {
-      const int s = b % kStages;
-      if (tid == 0 && b + 2 < nblk) {   // refill the stage block b - 1 used, once every warp has released it
-        const int s2 = (b + 2) % kStages;
-        if (b >= 1) mbar_wait(&empty[s2], (uint32_t)(((b - 1) / kStages) & 1));
-        mbar_arrive_expect_tx(&full[s2], kBlkBytes);
-        bulk_g2s(sm + s2 * kBlkFloats, a.Img + (size_t)(b + 2) * kBlkFloats, kBlkBytes, &full[s2]);
-      }
-      __syncwarp();
-      const bool more = k + 1 < nl;
-      if (more) {   // the 64 rows that enter the window after this block: into L2 now, into registers when their slots are free
-        const int v = (tile0 + warp) * 16 + (lane >> 1);
-        const int r = R0 + 128 + ((lane & 1) ? 63 : 0);
-        if (v < a.mvec && r < n) {
-          const float* pz = a.Z + (size_t)v * a.ldz + r;
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(pz));
-          if (!(lane & 1) && r + 32 < n) asm volatile("prefetch.global.L2 [%0];" ::"l"(pz + 32));
-        }
-      }
-      mbar_wait(&full[s], (uint32_t)((b / kStages) & 1));
-      const float* Ph = sm + s * kBlkFloats;   // planes: Ph, Ph + kPlane (lo), Th = Ph + 2 kPlane, Th + kPlane (lo)
-      const float* Th = Ph + 2 * kPlane;
-      // ---- X'[vec][c] = sum_w Z'[vec][w] V[w][c]: tile j of X' (reflectors 8j ..) meets the row tiles j .. j + 8
-      float x[8][4], xc[8][4];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) x[j][0] = x[j][1] = x[j][2] = x[j][3] = 0.f;
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        uint32_t ah[4], al[4];
-        split_frag(z[i], ah, al);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int d = i - j;
-          if (d >= 0 && d <= 8) {
-            const float* p = Ph + 8 * j * kImgRow + 8 * d + (d == 8 ? offA : ((d & 1) ? offAo : offAe));
-            uint32_t bh[2], bl[2];
-            ld_b2(bh, p);
-            ld_b2(bl, p + kPlane);
-            if (d == 0) mma_step<true>(x[j], xc[j], ah, al, bh, bl, 1.f);
-            else mma_step<false>(x[j], xc[j], ah, al, bh, bl, 1.f);
-          }
-        }
-      }
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        x[j][0] += xc[j][0]; x[j][1] += xc[j][1]; x[j][2] += xc[j][2]; x[j][3] += xc[j][3];
-      }
-      // ---- X2'[vec][c] = sum_{c' >= c} X'[vec][c'] T[c][c']   (a fifth of the work: plain three-term chains from zero)
-      float x2[8][4];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) x2[j][0] = x2[j][1] = x2[j][2] = x2[j][3] = 0.f;
-#pragma unroll
-      for (int jk = 0; jk < 8; ++jk) {
-        uint32_t ah[4], al[4];
-        split_frag(x[jk], ah, al);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          if (j <= jk) {
-            const float* p = Th + (8 * j + g) * kImgRow + 8 * jk + 2 * t;
-            uint32_t bh[2], bl[2];
-            ld_b2(bh, p);
-            ld_b2(bl, p + kPlane);
-            float dd[4];
-            mma_tf32_zero(dd, al, bh);
-            mma_tf32(dd, ah, bl);
-            mma_tf32(dd, ah, bh);
-            x2[j][0] += dd[0]; x2[j][1] += dd[1]; x2[j][2] += dd[2]; x2[j][3] += dd[3];
-          }
-        }
-      }
-      // ---- Z'[vec][w] -= sum_c X2'[vec][c] V[w][c]: row tile i meets the reflector tiles i - 8 .. i
-      {
-        uint32_t x2h[8][4], x2l[8][4];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) split_frag(x2[j], x2h[j], x2l[j]);
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          float zc[4];
-#pragma unroll
-          for (int jc = 0; jc < 8; ++jc) {
-            const int d = i - jc;
-            if (d >= 0 && d <= 8) {
-              const float* p = Ph + 8 * jc * kImgRow + 8 * d + (d == 8 ? offB : ((d & 1) ? offBo : offBe));
-              uint32_t bh[2], bl[2];
-              bh[0] = __float_as_uint(p[0]);
-              bh[1] = __float_as_uint(p[kImgRow]);
-              bl[0] = __float_as_uint(p[kPlane]);
-              bl[1] = __float_as_uint(p[kPlane + kImgRow]);
-              if (jc == (i > 8 ? i - 8 : 0)) mma_step<true>(z[i], zc, x2h[jc], x2l[jc], bh, bl, -1.f);
-              else mma_step<false>(z[i], zc, x2h[jc], x2l[jc], bh, bl, -1.f);
-            }
-          }
-          z[i][0] -= zc[0]; z[i][1] -= zc[1]; z[i][2] -= zc[2]; z[i][3] -= zc[3];
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&empty[s]);
-      // ---- the first 64 rows leave the window (all 128 at the group's last level); the prefetched rows enter
-#pragma unroll
-      for (int i = 0; i < 8; ++i) st_rows(z[i], za, zb, oka, okb, R0 + 8 * i + 2 * t, n);
-      if (more) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-#pragma unroll
-          for (int e = 0; e < 4; ++e) z[i][e] = z[i + 8][e];
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) ld_rows(z[i + 8], za, zb, oka, okb, R0 + 128 + 8 * i + 2 * t, n);   // first used a quarter block later
-      } else {
-#pragma unroll
-        for (int i = 8; i < 16; ++i) st_rows(z[i], za, zb, oka, okb, R0 + 8 * i + 2 * t, n);
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------- Q2, register-stationary variant in split binary16
-// Measured on B200 (scripts/mma_rate.cu): the warp-level tensor path issues one mma.sync per 8 cycles and sub-partition for
-// m16n8k8 TF32 and for m16n8k16 FP16 alike, so a binary16 step contracts twice as many terms in the same time.  Same kernel as
-// above with x = hi + lo / 2048, hi = half(x), lo = half((x - hi) 2048): 22 significant bits like the TF32 pair; the factor keeps
-// lo out of the subnormal range, and values below 6e-5 (eigenvector entries never need more) keep an absolute error of 1.5e-11.
+// ---------------------------------------------------------------------------------------------------------------- Q2
+// The window of a slab never leaves the register file.  A warp owns 16 eigenvectors and keeps their 128-row window as the
+// accumulator fragments of sixteen m16n8 tiles (vectors = the M dimension, window rows = N).  A 16-row step of the window is
+// two accumulator tiles, and their registers (tile i | tile i + 1), converted to binary16, are the A fragment of the next
+// product as they stand (natural k order).  So  X' = Z' V  ->  X2' = X' T'  ->  Z' -= X2' V'  chain through registers: no
+// shared-memory window, no CTA-wide barrier, and the only operands that come from shared memory are the reflector block and
+// its T factor.  Those are the same for every warp and every vector, so a pre-pass (k_q2_images_h) writes them once, already
+// split and already in the shared-memory layout, and one elected thread streams one 40 KB image per block through a
+// four-stage cp.async.bulk ring (mbarrier full / empty pairs); warps never wait for each other except through that ring.
+// Split binary16: x = hi + lo / 2048, hi = half(x), lo = half((x - hi) 2048), 22 significant bits; the factor keeps lo out of
+// the subnormal range, and values below 6e-5 (eigenvector entries never need more) keep an absolute error of 1.5e-11.
 // Everything that is multiplied is O(1) or smaller: eigenvector entries, reflectors (|v| <= 1), T (|tau| <= 2), X, X2.
-// A 16-row step of the window is two accumulator tiles: registers (tile i | tile i + 1) are the A fragment as they stand
-// (natural k order).  B fragments come from the image by ldmatrix: plain for the first product and for T (pairs along the
-// window rows of one reflector), transposed for the last product (pairs along the reflectors of one window row); one
-// ldmatrix.x4 fetches the hi and lo fragments of a step.  Image of a block: binary16 planes P hi, P lo (64 rows of 88: 8
-// zeros, the 72 entries of the nine steps, 8 zeros - the zeros serve the half steps that stick out of the band), T hi, T lo
-// (64 rows of 72); row pitches of 176 and 144 bytes spread the eight 16-byte rows of an ldmatrix over all banks.
+// Measured on B200 (scripts/mma_rate.cu), the warp-level tensor path issues one mma.sync per 8 cycles and sub-partition for
+// m16n8k8 TF32 and for m16n8k16 FP16 alike, so a binary16 step contracts twice as many terms in the same time as the
+// three-term TF32 split of the same 22 bits (254 / 440 ms against 380 / 558 ms for the smallest half / all vectors at
+// n = 20 000).
+// B fragments come from the image by ldmatrix: plain for the first product and for T (pairs along the window rows of one
+// reflector), transposed for the last product (pairs along the reflectors of one window row); one ldmatrix.x4 fetches the hi
+// and lo fragments of a step.  Image of a block: binary16 planes P hi, P lo (64 rows of 88: 8 zeros, the 72 entries of the
+// nine steps, 8 zeros - the zeros serve the half steps that stick out of the band), T hi, T lo (64 rows of 72); row pitches of
+// 176 and 144 bytes spread the eight 16-byte rows of an ldmatrix over all banks.
+// Accumulation: the tensor core adds with truncation, so the leading term a_hi b_hi of every step starts from a zero
+// accumulator and is added to the running sum with a rounded FP32 add; the two cross terms, 2^-11 of it, are chained in
+// tensor-core accumulators of their own (their truncation is 2^-35 of the result), which also keeps the dependent chains short.
 constexpr int kPRowH = 88, kTRowH = 72;
 constexpr int kPPlaneH = B * kPRowH, kTPlaneH = B * kTRowH;        // halves per plane
 constexpr int kBlkHalves = 2 * kPPlaneH + 2 * kTPlaneH;            // 20 480 halves = 40 960 bytes
@@ -621,6 +104,9 @@ constexpr int kBlkBytesH = kBlkHalves * 2;
 constexpr int kStagesH = 4;
 constexpr float kLoScale = 2048.f, kLoInv = 1.f / 2048.f;
 
+// Pre-pass: T factor of block (G, k) (forward columnwise larft on the Gram matrix of its reflectors), then the block's image at
+// its place in processing order (groups descending, levels ascending: block index (q - G)(q - G + 1) / 2 + k with q = the last
+// group).
 __global__ void __launch_bounds__(256) k_q2_images_h(const float* __restrict__ V2, long long ldv2, const float* __restrict__ tau2,
                                                      long long ldt2, int n, int q, __half* __restrict__ Img) {
   const int k = (int)blockIdx.x, G = (int)blockIdx.y, s0 = G * B;
@@ -904,74 +390,16 @@ __global__ void __launch_bounds__(256) k_unit_vectors(float* __restrict__ Z, lon
 }
 
 // ---------------------------------------------------------------------------------------------------------------- Q1
-// Xpart[s][c][vec] = sum over rows i of chunk s of V[c][i] * Z[vec][r0 + i]
-__global__ void __launch_bounds__(256, 2) k_q1_x(const float* __restrict__ Vp, long long lda, int m, const float* __restrict__ Zr,
-                                                 long long ldz, int mvec, float* __restrict__ Xpart, long long ldx, int chunk) {
-  __shared__ __align__(16) float smem[tile::Smem<64>::floats];
-  const int vec0 = (int)blockIdx.x * tile::TM;
-  const int ka = (int)blockIdx.y * chunk, kl = min(m, ka + chunk) - ka;
-  tile::Acc<64> acc;
-  acc.clear();
-  tile::mac<64>(acc, tile::opnd(Zr + (long long)vec0 * ldz + ka, ldz, 1, mvec - vec0, kl), tile::opnd(Vp + ka, lda, 1, B, kl), kl, smem);
-  float* out = Xpart + (size_t)blockIdx.y * B * ldx;
-#pragma unroll
-  for (int b = 0; b < 4; ++b) {
-    const int c = tile::Acc<64>::col(b);
-#pragma unroll
-    for (int a = 0; a < 8; ++a) {
-      const int v = vec0 + tile::Acc<64>::row(a);
-      if (v < mvec) out[(long long)c * ldx + v] = acc.v[a][b];
-    }
-  }
-}
-
-__global__ void k_sum_parts32(const float* __restrict__ part, int nparts, size_t stride, size_t n, float* __restrict__ out) {
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  float s = 0.f;
-  for (int p = 0; p < nparts; ++p) s += part[(size_t)p * stride + i];
-  out[i] = s;
-}
-
-// Z[vec][r0 + i] -= sum_c (V T)[i][c] X[c][vec]   (VTt: the panel's V T as sy2sb left it, element (i, c) at VTt[c + i * lda])
-__global__ void __launch_bounds__(256, 2) k_q1_z(const float* __restrict__ VTt, long long lda, int m, const float* __restrict__ Xp,
-                                                 long long ldx, int mvec, float* Zr, long long ldz) {
-  __shared__ __align__(16) float smem[tile::Smem<128>::floats];
-  const int i0 = (int)blockIdx.x * tile::TM, vec0 = (int)blockIdx.y * tile::TM;
-  tile::Acc<128> acc;
-  acc.clear();
-  tile::mac<128>(acc, tile::opnd(VTt + (long long)i0 * lda, lda, 1, m - i0, B), tile::opnd(Xp + vec0, ldx, 0, mvec - vec0, B), B, smem);
-#pragma unroll
-  for (int b = 0; b < 8; ++b) {
-    const int v = vec0 + tile::Acc<128>::col(b);
-    if (v >= mvec) continue;
-    float* zc = Zr + (long long)v * ldz;
-#pragma unroll
-    for (int a4 = 0; a4 < 2; ++a4) {
-      const int i = i0 + tile::Acc<128>::row(a4 * 4);
-      if (i + 3 < m && ((((uintptr_t)(zc + i)) & 15) == 0)) {
-        float4 z = *reinterpret_cast<float4*>(zc + i);
-        z.x -= acc.v[a4 * 4 + 0][b]; z.y -= acc.v[a4 * 4 + 1][b]; z.z -= acc.v[a4 * 4 + 2][b]; z.w -= acc.v[a4 * 4 + 3][b];
-        *reinterpret_cast<float4*>(zc + i) = z;
-      } else {
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          if (i + q < m) zc[i + q] -= acc.v[a4 * 4 + q][b];
-      }
-    }
-  }
-}
-
-// ---- the same two products on the tensor-core tile engine (error-compensated TF32, sgemm_tile.cuh)
-template <int ENG>
+// Panel by panel on the split-binary16 tile engine of sgemm_tile.cuh: eigenvector slabs, reflector panels and their products
+// are O(1).  Xpart[s][c][vec] = sum over rows i of chunk s of V[c][i] * Z[vec][r0 + i]
 __global__ void __launch_bounds__(256, 2) k_q1_x_tc(const float* __restrict__ Vp, long long lda, int m, const float* __restrict__ Zr,
                                                     long long ldz, int mvec, float* __restrict__ Xpart, long long ldx, int chunk) {
-  __shared__ __align__(16) unsigned char smem[tile::SmemE<ENG, 64>::bytes];
+  __shared__ __align__(16) unsigned char smem[tile::SmemE<2, 64>::bytes];
   const int vec0 = (int)blockIdx.x * tile::TM;
   const int ka = (int)blockIdx.y * chunk, kl = min(m, ka + chunk) - ka;
   tile::AccT<64> acc;
   acc.clear();
-  tile::mac_e<ENG, 64, 1, 1>(acc, tile::opnd(Zr + (long long)vec0 * ldz + ka, ldz, 1, mvec - vec0, kl), tile::opnd(Vp + ka, lda, 1, B, kl), kl, smem);
+  tile::mac_e<2, 64, 1, 1>(acc, tile::opnd(Zr + (long long)vec0 * ldz + ka, ldz, 1, mvec - vec0, kl), tile::opnd(Vp + ka, lda, 1, B, kl), kl, smem);
   float* out = Xpart + (size_t)blockIdx.y * B * ldx;
 #pragma unroll
   for (int nt = 0; nt < tile::AccT<64>::NTL; ++nt)
@@ -984,16 +412,23 @@ __global__ void __launch_bounds__(256, 2) k_q1_x_tc(const float* __restrict__ Vp
       }
 }
 
-// Z[vec][r0 + i] -= sum_c X[c][vec] (V T)[i][c]: vectors on the rows of the tile, matrix rows on its columns, so that a thread's
-// two adjacent outputs are adjacent in memory
-template <int ENG>
+__global__ void k_sum_parts32(const float* __restrict__ part, int nparts, size_t stride, size_t n, float* __restrict__ out) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float s = 0.f;
+  for (int p = 0; p < nparts; ++p) s += part[(size_t)p * stride + i];
+  out[i] = s;
+}
+
+// Z[vec][r0 + i] -= sum_c X[c][vec] (V T)[i][c] (VTt: the panel's V T as sy2sb left it, element (i, c) at VTt[c + i * lda]):
+// vectors on the rows of the tile, matrix rows on its columns, so that a thread's two adjacent outputs are adjacent in memory
 __global__ void __launch_bounds__(256, 2) k_q1_z_tc(const float* __restrict__ VTt, long long lda, int m, const float* __restrict__ Xp,
                                                     long long ldx, int mvec, float* Zr, long long ldz) {
-  __shared__ __align__(16) unsigned char smem[tile::SmemE<ENG, 128>::bytes];
+  __shared__ __align__(16) unsigned char smem[tile::SmemE<2, 128>::bytes];
   const int i0 = (int)blockIdx.x * tile::TM, vec0 = (int)blockIdx.y * tile::TM;
   tile::AccT<128> acc;
   acc.clear();
-  tile::mac_e<ENG, 128, 0, 1>(acc, tile::opnd(Xp + vec0, ldx, 0, mvec - vec0, B), tile::opnd(VTt + (long long)i0 * lda, lda, 1, m - i0, B), B, smem);
+  tile::mac_e<2, 128, 0, 1>(acc, tile::opnd(Xp + vec0, ldx, 0, mvec - vec0, B), tile::opnd(VTt + (long long)i0 * lda, lda, 1, m - i0, B), B, smem);
 #pragma unroll
   for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
@@ -1024,6 +459,8 @@ __global__ void __launch_bounds__(256, 2) k_q1_z_tc(const float* __restrict__ VT
 // converted once per block; powers of two keep their low-order parts in binary16's normal range.
 constexpr int kQ1Panels = 8;
 constexpr float kScV = 1024.f, kScVT = 64.f, kScZ = 1024.f, kScX = 256.f;
+// k-blocks per accumulation chunk of the two large products (profiles/r2_two_stage_stage_times_20000.txt compares 2, 4 and 8)
+constexpr int kQ1ChunkKb = 4;
 
 // V of the block's panels as (hi, lo) binary16, reflector-major [ncols][ldk] over the rows r0 .. n; zero above a panel's first row
 __global__ void __launch_bounds__(256) k_q1_conv_v(const float* __restrict__ A, long long lda, int n, int c0, int r0, long long ldk,
@@ -1155,81 +592,27 @@ void apply_q2(const float* V2, long long ldv2, const float* tau2, long long ldt2
   const int nsweeps = n - 2;
   const int ngroups = (nsweeps + B - 1) / B;
   const int nlev = sb2st_levels(n);
-  // SCL_Q2_VARIANT=0: the shared-memory window kernel (k_q2_apply); 1: the register-stationary kernel in three-term TF32;
-  // default 2: the register-stationary kernel in split binary16 (253 / 440 ms for the smallest half / all vectors at n = 20 000
-  // against 380 / 558 ms for 1 and 818 / 1627 ms for 0)
-  const int variant = q2_variant();
-  if (variant == 2 && n >= 3) {
-    const int q = (n - 3) / B;
-    const size_t nblk = (size_t)(q + 1) * (q + 2) / 2;
-    Tmp<__half> Img(nblk * kBlkHalves, st);
-    k_q2_images_h<<<dim3(nlev, ngroups), 256, 0, st>>>(V2, ldv2, tau2, ldt2, n, q, Img.p);
-    SCL_CUDA(cudaGetLastError());
-    const int tiles = (mvec + 15) / 16, sms = sm_count();
-    const int waves = (tiles + sms * 12 - 1) / (sms * 12);
-    const int grid = std::min(tiles, sms * waves);
-    const int base = tiles / grid, extra = tiles % grid;
-    const int warps = base + (extra ? 1 : 0);
-    const size_t smem = (size_t)kStagesH * kBlkBytesH + 2 * kStagesH * sizeof(uint64_t);
-    Q2HArgs a{Img.p, Z, ldz, n, mvec, q, tiles, base, extra};
-    if (warps <= 8) {
-      SCL_CUDA(cudaFuncSetAttribute(k_q2_apply_h<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_q2_apply_h<8><<<grid, warps * 32, smem, st>>>(a);
-    } else {
-      SCL_CUDA(cudaFuncSetAttribute(k_q2_apply_h<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_q2_apply_h<12><<<grid, warps * 32, smem, st>>>(a);
-    }
-    SCL_CUDA(cudaGetLastError());
-    count_launches(2);
-    return;
-  }
-  if (variant != 0 && n >= 3) {
-    const int q = (n - 3) / B;   // last group; group G has q - G + 1 levels
-    const size_t nblk = (size_t)(q + 1) * (q + 2) / 2;
-    Tmp<float> Img(nblk * kBlkFloats, st);
-    k_q2_images<<<dim3(nlev, ngroups), 256, 0, st>>>(V2, ldv2, tau2, ldt2, n, q, Img.p);
-    SCL_CUDA(cudaGetLastError());
-    // 16-vector tiles, one warp each; at most 12 warps per CTA (registers are granted to a CTA in units of four warps: 255 per
-    // thread up to 8 warps, 168 up to 12), as few waves as that allows
-    const int tiles = (mvec + 15) / 16, sms = sm_count();
-    const int waves = (tiles + sms * 12 - 1) / (sms * 12);
-    const int grid = std::min(tiles, sms * waves);
-    const int base = tiles / grid, extra = tiles % grid;
-    const int warps = base + (extra ? 1 : 0);
-    const size_t smem = (size_t)kStages * kBlkBytes + 2 * kStages * sizeof(uint64_t);
-    Q2RsArgs a{Img.p, Z, ldz, n, mvec, q, tiles, base, extra};
-    if (warps <= 8) {
-      SCL_CUDA(cudaFuncSetAttribute(k_q2_apply_rs<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_q2_apply_rs<8><<<grid, warps * 32, smem, st>>>(a);
-    } else {
-      SCL_CUDA(cudaFuncSetAttribute(k_q2_apply_rs<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_q2_apply_rs<12><<<grid, warps * 32, smem, st>>>(a);
-    }
-    SCL_CUDA(cudaGetLastError());
-    count_launches(2);
-    return;
-  }
-  Tmp<float> Tq((size_t)ngroups * nlev * B * B, st);
-  k_q2_tfactor<<<dim3(nlev, ngroups), 256, 0, st>>>(V2, ldv2, tau2, ldt2, n, nlev, Tq.p);
+  const int q = (n - 3) / B;   // last group; group G has q - G + 1 levels
+  const size_t nblk = (size_t)(q + 1) * (q + 2) / 2;
+  Tmp<__half> Img(nblk * kBlkHalves, st);
+  k_q2_images_h<<<dim3(nlev, ngroups), 256, 0, st>>>(V2, ldv2, tau2, ldt2, n, q, Img.p);
   SCL_CUDA(cudaGetLastError());
-  // vectors per CTA: one CTA per SM and as few rounds as the 88-vector limit allows, balanced; padded to nvp = 8 (mod 16)
-  const int sms = sm_count();
-  const int rounds = (mvec + sms * 88 - 1) / (sms * 88);
-  int nv = (mvec + sms * rounds - 1) / (sms * rounds);
-  nv = std::max(8, (nv + 7) & ~7);
-  int nvp = nv;
-  if ((nvp & 15) == 0) nvp += 8;
-  if (nvp > 88) {   // 96 vectors would not fit: split once more
-    nv = 88;
-    nvp = 88;
+  // 16-vector tiles, one warp each; at most 12 warps per CTA (registers are granted to a CTA in units of four warps: 255 per
+  // thread up to 8 warps, 168 up to 12), as few waves as that allows
+  const int tiles = (mvec + 15) / 16, sms = sm_count();
+  const int waves = (tiles + sms * 12 - 1) / (sms * 12);
+  const int grid = std::min(tiles, sms * waves);
+  const int base = tiles / grid, extra = tiles % grid;
+  const int warps = base + (extra ? 1 : 0);
+  const size_t smem = (size_t)kStagesH * kBlkBytesH + 2 * kStagesH * sizeof(uint64_t);
+  Q2HArgs a{Img.p, Z, ldz, n, mvec, q, tiles, base, extra};
+  if (warps <= 8) {
+    SCL_CUDA(cudaFuncSetAttribute(k_q2_apply_h<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_q2_apply_h<8><<<grid, warps * 32, smem, st>>>(a);
+  } else {
+    SCL_CUDA(cudaFuncSetAttribute(k_q2_apply_h<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_q2_apply_h<12><<<grid, warps * 32, smem, st>>>(a);
   }
-  const int nslab = (mvec + nv - 1) / nv;
-  const int threads = 256;
-  const size_t smem = ((size_t)128 * nvp + 3 * (size_t)B * nvp + 2 * 128 * VS + 2 * (size_t)B * VS) * sizeof(float);
-  SCL_REQUIRE(nvp / 8 <= 2 * kMaxNJ && smem <= 227 * 1024, "apply_q2: slab does not fit");
-  SCL_CUDA(cudaFuncSetAttribute(k_q2_apply, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  Q2Args a{V2, ldv2, Tq.p, n, nlev, ngroups, Z, ldz, mvec, nv, nvp};
-  k_q2_apply<<<nslab, threads, smem, st>>>(a);
   SCL_CUDA(cudaGetLastError());
   count_launches(2);
 }
@@ -1252,7 +635,6 @@ static void apply_q1_umma(const float* A, int n, long long lda, const float* T1,
   const size_t rec_smem = (size_t)(kQ1Panels - 1) * B * B * sizeof(float);
   SCL_CUDA(cudaFuncSetAttribute(k_q1_recursion, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rec_smem));
   long launches = 0;
-  static const int q1_chunk = [] { const char* e = getenv("SCL_Q1_CHUNK_KB"); return e ? atoi(e) : 4; }();
   for (int b = nblocks - 1; b >= 0; --b) {
     const int a = b * kQ1Panels, np = std::min(kQ1Panels, npanels - a);
     const int c0 = a * B, r0 = c0 + B, m = n - r0, ncols = np * B;
@@ -1266,7 +648,7 @@ static void apply_q1_umma(const float* A, int n, long long lda, const float* T1,
     g.A.hi = vh.p; g.A.lo = vl.p; g.A.rows = ncols; g.A.K = m; g.A.ld = ldk;
     g.B.hi = zh.p; g.B.lo = zl.p; g.B.rows = mvec; g.B.K = m; g.B.ld = ldk;
     g.alpha = 1.f / (kScV * kScZ);
-    g.chunk_kb = q1_chunk;   // short tensor-core chains: the accumulator truncates, 3e-8 per MMA of a chain, one-sided
+    g.chunk_kb = kQ1ChunkKb;   // short tensor-core chains: the accumulator truncates, 3e-8 per MMA of a chain, one-sided
     g.epi = Epilogue::Store;
     g.C = Y.p; g.ldc = ldy;
     gemm_umma(g, st);
@@ -1288,7 +670,7 @@ static void apply_q1_umma(const float* A, int n, long long lda, const float* T1,
     u.A.hi = xh.p; u.A.lo = xl.p; u.A.rows = mvec; u.A.K = ncols; u.A.ld = ldo;
     u.B.hi = th.p; u.B.lo = tl.p; u.B.rows = m; u.B.K = ncols; u.B.ld = ldo;
     u.alpha = -1.f / (kScX * kScVT);
-    u.chunk_kb = q1_chunk;
+    u.chunk_kb = kQ1ChunkKb;
     u.C = U.p; u.ldc = ldk;
     gemm_umma(u, st);
     k_q1_add<<<dim3((unsigned)std::min((m + 1023) / 1024, 64), (unsigned)std::min(mvec, 65535)), 256, 0, st>>>(Z, ldz, r0, U.p, ldk, m, mvec);
@@ -1301,7 +683,7 @@ static void apply_q1_umma(const float* A, int n, long long lda, const float* T1,
 void apply_q1(const float* A, int n, long long lda, const float* T1, int npanels, float* Z, long long ldz, int mvec,
               cudaStream_t st) {
   if (mvec <= 0 || npanels <= 0) return;
-  if (tile_engine_q1() == 3 && mvec >= 64) {   // a handful of vectors is not worth the block machinery: panel by panel below
+  if (mvec >= 64) {   // a handful of vectors is not worth the block machinery: panel by panel below
     apply_q1_umma(A, n, lda, T1, npanels, Z, ldz, mvec, st);
     return;
   }
@@ -1310,7 +692,6 @@ void apply_q1(const float* A, int n, long long lda, const float* T1, int npanels
   Tmp<float> Xpart((size_t)max_split * B * ldx, st), Xp((size_t)B * ldx, st);
   const int vt = (mvec + tile::TM - 1) / tile::TM;
   const int slots = 2 * sm_count();
-  const int eng = std::min(2, tile_engine_q1());
   for (int k = npanels - 1; k >= 0; --k) {
     const int c0 = k * B, r0 = c0 + B, m = n - r0;
     if (m < 1) continue;
@@ -1320,19 +701,9 @@ void apply_q1(const float* A, int n, long long lda, const float* T1, int npanels
     chunk = std::max(chunk, 4 * tile::KT);
     split = (m + chunk - 1) / chunk;
     const size_t nx = (size_t)B * ldx;
-    if (eng == 2) {   // eigenvector slabs, reflector panels and their products are O(1): split binary16
-      k_q1_x_tc<2><<<dim3(vt, split), 256, 0, st>>>(Vp, lda, m, Z + r0, ldz, mvec, Xpart.p, ldx, chunk);
-      k_sum_parts32<<<(unsigned)((nx + 255) / 256), 256, 0, st>>>(Xpart.p, split, nx, nx, Xp.p);
-      k_q1_z_tc<2><<<dim3((m + tile::TM - 1) / tile::TM, vt), 256, 0, st>>>(A + c0 + (long long)r0 * lda, lda, m, Xp.p, ldx, mvec, Z + r0, ldz);
-    } else if (eng == 1) {
-      k_q1_x_tc<1><<<dim3(vt, split), 256, 0, st>>>(Vp, lda, m, Z + r0, ldz, mvec, Xpart.p, ldx, chunk);
-      k_sum_parts32<<<(unsigned)((nx + 255) / 256), 256, 0, st>>>(Xpart.p, split, nx, nx, Xp.p);
-      k_q1_z_tc<1><<<dim3((m + tile::TM - 1) / tile::TM, vt), 256, 0, st>>>(A + c0 + (long long)r0 * lda, lda, m, Xp.p, ldx, mvec, Z + r0, ldz);
-    } else {
-      k_q1_x<<<dim3(vt, split), 256, 0, st>>>(Vp, lda, m, Z + r0, ldz, mvec, Xpart.p, ldx, chunk);
-      k_sum_parts32<<<(unsigned)((nx + 255) / 256), 256, 0, st>>>(Xpart.p, split, nx, nx, Xp.p);
-      k_q1_z<<<dim3((m + tile::TM - 1) / tile::TM, vt), 256, 0, st>>>(A + c0 + (long long)r0 * lda, lda, m, Xp.p, ldx, mvec, Z + r0, ldz);
-    }
+    k_q1_x_tc<<<dim3(vt, split), 256, 0, st>>>(Vp, lda, m, Z + r0, ldz, mvec, Xpart.p, ldx, chunk);
+    k_sum_parts32<<<(unsigned)((nx + 255) / 256), 256, 0, st>>>(Xpart.p, split, nx, nx, Xp.p);
+    k_q1_z_tc<<<dim3((m + tile::TM - 1) / tile::TM, vt), 256, 0, st>>>(A + c0 + (long long)r0 * lda, lda, m, Xp.p, ldx, mvec, Z + r0, ldz);
   }
   SCL_CUDA(cudaGetLastError());
   count_launches(3 * npanels);

@@ -675,8 +675,8 @@ int32_t scl_bench_syevd_concurrent(scl_handle* h, int32_t n, int32_t nsolves, in
   });
 }
 
-int32_t scl_debug_set_eig_api(int32_t v) {
-  scl::set_eig_api(v);
+int32_t scl_debug_force_one_stage(int32_t on) {
+  scl::force_one_stage(on != 0);
   return SCL_OK;
 }
 
@@ -686,13 +686,6 @@ int32_t scl_debug_last_solve(scl_handle* h, double* out) {
   out[5] = h->solver->tri_two_stage ? 1.0 : 0.0;
   out[6] = (double)h->solver->ts_fallbacks;
   out[7] = (double)h->solver->tri_fallbacks;
-  return SCL_OK;
-}
-
-int32_t scl_debug_set_two_stage(int32_t q2_variant, int32_t stage1_engine, int32_t q1_engine) {
-  scl::g_two_stage_override[0].store(q2_variant, std::memory_order_relaxed);
-  scl::g_two_stage_override[1].store(stage1_engine, std::memory_order_relaxed);
-  scl::g_two_stage_override[2].store(q1_engine, std::memory_order_relaxed);
   return SCL_OK;
 }
 

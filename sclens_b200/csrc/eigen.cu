@@ -1,10 +1,11 @@
-// Full-spectrum symmetric eigensolve (the one declared library dependency: cuSOLVER syevd,
-// as src/scLENS.jl:377) and the scalar Marchenko-Pastur / Tracy-Widom fit (:390-487).
+// Symmetric eigensolves (_get_eigen, src/scLENS.jl:375-382) on the own solver: the two-stage reduction (twostage.h) or the
+// one-stage path (sytrd.cu), the Float64 tridiagonal stage (tridiag.cu) and the back-transformations.  cuSOLVER serves the
+// one-stage path where the own kernels decline (Ssytrd, Sormtr), the last resort (Ssyevd) and the timing study of the
+// library solvers.  Also the scalar Marchenko-Pastur / Tracy-Widom fit (:390-487).
 #include <cusolverDn.h>
 #include <algorithm>
 #include <cmath>
 #include <atomic>
-#include <cstdlib>
 #include "common.cuh"
 #include "eigen.h"
 #include "tmp.cuh"
@@ -21,7 +22,6 @@ namespace scl {
 
 struct Solver::Impl {
   cusolverDnHandle_t h = nullptr;
-  cusolverDnParams_t params = nullptr;   // 64-bit API (SCL_EIG_API=1)
   DBuf<float> work;
   DBuf<float> tri_d, tri_e, tri_tau, tri_z, tri_keep, tri_pad;   // own tridiagonal stage: T, reflector scalars, vectors, matrix copy, padded copy
   DBuf<double> tri_w;
@@ -31,28 +31,10 @@ struct Solver::Impl {
   Sy2sbAux ts_aux;
   DBuf<double> dwork;
   DBuf<int> info;
-  std::vector<unsigned char> host_work;
 };
 
-// Which library entry point runs the full eigensolves.  0 (default): cusolverDnSsyevd, the call the reference makes
-// through CUDA.jl (:377).  1: cusolverDnXsyevd, the 64-bit generic API - 495 ms against 550 ms at n = 10^4 in a first
-// look (profiles/r1_syevd_study_10000.json); NOT yet parity-tested inside the path, hence opt-in (SCL_EIG_API bit 0).
-// Bit 1: the sparsity-search steps, which use only the n/2+1 smallest eigenvectors (:742), call cusolverDnSsyevdx with
-// an index range instead of a full solve (474 ms in the same first look); also opt-in until parity-tested.
-static std::atomic<int> g_eig_api_override{-1};
-int eig_api() {
-  // default 60: the own tridiagonal stage for every solve (bit 2) with index-range vectors in the search steps (bit 3) behind
-  // the two-stage reduction (bit 5: dense -> band -> tridiagonal, twostage.h); bit 4 = the own one-stage tridiagonalisation,
-  // which a solve falls back to when a panel of the two-stage reduction cannot be factored and which serves orders below
-  // 4 kBand.  Measured at n = 20 000 (all vectors / smallest half / values only): two-stage 1.71 / 1.29 / 0.62 s; one-stage own
-  // sytrd + own stage + Sormtr 2.42 / 2.25 / 2.03 s; Ssytrd + own stage + Sormtr 2.85 s; Ssyevd 3.65 s on the 68k x 20k data
-  // Gram matrix (2.69 s on a synthetic Wishart matrix).  SCL_EIG_API=28 is the one-stage path, 0 the plain library solve (the
-  // call the reference makes).
-  static const int v = [] { const char* e = getenv("SCL_EIG_API"); return e ? atoi(e) : 60; }();
-  const int o = g_eig_api_override.load(std::memory_order_relaxed);
-  return o >= 0 ? o : v;
-}
-void set_eig_api(int v) { g_eig_api_override.store(v, std::memory_order_relaxed); }
+static std::atomic<bool> g_force_one_stage{false};
+void force_one_stage(bool on) { g_force_one_stage.store(on, std::memory_order_relaxed); }
 
 Solver::Solver(cudaStream_t st) : impl(new Impl) {
   SCL_SOLVER(cusolverDnCreate(&impl->h));
@@ -65,12 +47,11 @@ Solver::~Solver() {
     cudaEventDestroy(impl->ts_aux.ready);
     cudaEventDestroy(impl->ts_aux.done);
   }
-  if (impl->params) cusolverDnDestroyParams(impl->params);
   if (impl->h) cusolverDnDestroy(impl->h);
   delete impl;
 }
 
-// Two-stage solve (SCL_EIG_API bit 5): dense -> band -> tridiagonal, Float64 tridiagonal stage, Z = Q1 Q2 E.  Same contract as
+// Two-stage solve: dense -> band -> tridiagonal, Float64 tridiagonal stage, Z = Q1 Q2 E.  Same contract as
 // syevd_tri; a panel that cannot be factored (rank-deficient panel) or a failed tridiagonal stage falls back, loudly and
 // counted, to the one-stage path on a kept copy.
 bool Solver::syevd_2stage(float* dA, int n, float* dW, int v0, int v1, cudaStream_t st) {
@@ -111,9 +92,8 @@ bool Solver::syevd_2stage(float* dA, int n, float* dW, int v0, int v1, cudaStrea
     SCL_CUDA(cudaEventCreateWithFlags(&impl->ts_aux.ready, cudaEventDisableTiming));
     SCL_CUDA(cudaEventCreateWithFlags(&impl->ts_aux.done, cudaEventDisableTiming));
   }
-  static const bool no_ahead = getenv("SCL_NO_LOOKAHEAD") != nullptr;
-  const bool half_ok = tile_engine_s1() == 2 && half_range_ok(Aq, n, lda, st);
-  const int npanels = sy2sb_lower(Aq, n, lda, impl->ts_AB.p, impl->ts_T1.p, impl->ts_fail.p, st, no_ahead ? nullptr : &impl->ts_aux, half_ok);
+  const bool half_ok = half_range_ok(Aq, n, lda, st);
+  const int npanels = sy2sb_lower(Aq, n, lda, impl->ts_AB.p, impl->ts_T1.p, impl->ts_fail.p, st, &impl->ts_aux, half_ok);
   SCL_CUDA(cudaEventRecord(ev[1], st));
   sb2st(impl->ts_AB.p, n, impl->tri_d.p, impl->tri_e.p, m > 0, impl->ts_V2.p, ldv2, impl->ts_tau2.p, ldt2, st);
   SCL_CUDA(cudaEventRecord(ev[2], st));
@@ -163,10 +143,12 @@ bool Solver::syevd_2stage(float* dA, int n, float* dW, int v0, int v1, cudaStrea
   return true;
 }
 
+// Measured at n = 20 000 (all vectors / smallest half / values only): two-stage 1.71 / 1.29 / 0.62 s; one-stage (own
+// tridiagonalisation + own tridiagonal stage + Sormtr) 2.42 / 2.25 / 2.03 s; Ssyevd 3.65 s on the 68k x 20k data Gram matrix.
 bool Solver::syevd_tri(float* dA, int n, float* dW, int v0, int v1, cudaStream_t st) {
   SCL_REQUIRE(n >= 2 && 0 <= v0 && v0 <= v1 && v1 <= n, "bad eigenvector index range");
   tri_two_stage = false;
-  if ((eig_api() & 32) && n >= 4 * kBand) return syevd_2stage(dA, n, dW, v0, v1, st);
+  if (n >= 4 * kBand && !g_force_one_stage.load(std::memory_order_relaxed)) return syevd_2stage(dA, n, dW, v0, v1, st);
   return syevd_tri_one_stage(dA, n, dW, v0, v1, st);
 }
 
@@ -181,10 +163,9 @@ bool Solver::syevd_tri_one_stage(float* dA, int n, float* dW, int v0, int v1, cu
   SCL_CUDA(cudaMemcpyAsync(impl->tri_keep.p, dA, nn * sizeof(float), cudaMemcpyDeviceToDevice, st));
   // the own tridiagonalisation reads 16-byte groups of rows: a matrix whose order is not a multiple of 4 is reduced in a copy
   // with a padded leading dimension (the reflectors stay there for Sormtr)
-  const bool want_own = (eig_api() & 16) != 0;
   float* Aq = dA;
   int lda = n;
-  if (want_own && (n & 3)) {
+  if (n & 3) {
     lda = (n + 3) & ~3;
     impl->tri_pad.ensure((size_t)lda * n);
     SCL_CUDA(cudaMemsetAsync(impl->tri_pad.p, 0, (size_t)lda * n * sizeof(float), st));
@@ -199,7 +180,7 @@ bool Solver::syevd_tri_one_stage(float* dA, int n, float* dW, int v0, int v1, cu
                                            impl->tri_tau.p, impl->tri_z.p, n, &lw2));
   impl->work.ensure((size_t)std::max(lw1, lw2) + 1);
   SCL_CUDA(cudaEventRecord(ev[0], st));
-  tri_own_sytrd = want_own && sytrd_lower(Aq, n, lda, impl->tri_d.p, impl->tri_e.p, impl->tri_tau.p, st);
+  tri_own_sytrd = sytrd_lower(Aq, n, lda, impl->tri_d.p, impl->tri_e.p, impl->tri_tau.p, st);
   if (!tri_own_sytrd)
     SCL_SOLVER(cusolverDnSsytrd(impl->h, CUBLAS_FILL_MODE_LOWER, n, Aq, lda, impl->tri_d.p, impl->tri_e.p, impl->tri_tau.p,
                                 impl->work.p, lw1, impl->info.p));
@@ -245,51 +226,7 @@ bool Solver::syevd_tri_one_stage(float* dA, int n, float* dW, int v0, int v1, cu
 }
 
 // A (n x n, symmetric, full) is overwritten by the eigenvectors when vectors=true.
-void Solver::syevd(float* dA, int n, float* dW, bool vectors, cudaStream_t st) {
-  if (eig_api() & 4) {
-    syevd_tri(dA, n, dW, 0, vectors ? n : 0, st);
-    return;
-  }
-  int lwork = 0;
-  cusolverEigMode_t jobz = vectors ? CUSOLVER_EIG_MODE_VECTOR : CUSOLVER_EIG_MODE_NOVECTOR;
-  if (eig_api() & 1) {
-    if (!impl->params) SCL_SOLVER(cusolverDnCreateParams(&impl->params));
-    size_t wd = 0, wh = 0;
-    SCL_SOLVER(cusolverDnXsyevd_bufferSize(impl->h, impl->params, jobz, CUBLAS_FILL_MODE_UPPER, (int64_t)n, CUDA_R_32F, dA,
-                                           (int64_t)n, CUDA_R_32F, dW, CUDA_R_32F, &wd, &wh));
-    impl->work.ensure(wd / sizeof(float) + 1);
-    if (impl->host_work.size() < wh + 1) impl->host_work.resize(wh + 1);
-    SCL_SOLVER(cusolverDnXsyevd(impl->h, impl->params, jobz, CUBLAS_FILL_MODE_UPPER, (int64_t)n, CUDA_R_32F, dA, (int64_t)n,
-                                CUDA_R_32F, dW, CUDA_R_32F, impl->work.p, wd, impl->host_work.data(), wh, impl->info.p));
-    int info = 0;
-    SCL_CUDA(cudaMemcpyAsync(&info, impl->info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    SCL_CUDA(cudaStreamSynchronize(st));
-    if (info != 0) throw Error(-3, "cusolverDnXsyevd did not converge, info=" + std::to_string(info));
-    return;
-  }
-  SCL_SOLVER(cusolverDnSsyevd_bufferSize(impl->h, jobz, CUBLAS_FILL_MODE_UPPER, n, dA, n, dW, &lwork));
-  impl->work.ensure((size_t)lwork);
-  SCL_SOLVER(cusolverDnSsyevd(impl->h, jobz, CUBLAS_FILL_MODE_UPPER, n, dA, n, dW, impl->work.p, lwork, impl->info.p));
-  int info = 0;
-  SCL_CUDA(cudaMemcpyAsync(&info, impl->info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-  SCL_CUDA(cudaStreamSynchronize(st));
-  if (info != 0) throw Error(-3, "cusolverDnSsyevd did not converge, info=" + std::to_string(info));
-}
-
-// eigenpairs 1..iu (ascending) of A: dW[0..iu), eigenvector i in row i of dA's memory.  Returns the number found.
-int Solver::syevdx_smallest(float* dA, int n, float* dW, int iu, cudaStream_t st) {
-  int lwork = 0, meig = 0;
-  SCL_SOLVER(cusolverDnSsyevdx_bufferSize(impl->h, CUSOLVER_EIG_MODE_VECTOR, CUSOLVER_EIG_RANGE_I, CUBLAS_FILL_MODE_UPPER, n,
-                                          dA, n, 0.f, 0.f, 1, iu, &meig, dW, &lwork));
-  impl->work.ensure((size_t)lwork);
-  SCL_SOLVER(cusolverDnSsyevdx(impl->h, CUSOLVER_EIG_MODE_VECTOR, CUSOLVER_EIG_RANGE_I, CUBLAS_FILL_MODE_UPPER, n, dA, n, 0.f,
-                               0.f, 1, iu, &meig, dW, impl->work.p, lwork, impl->info.p));
-  int info = 0;
-  SCL_CUDA(cudaMemcpyAsync(&info, impl->info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-  SCL_CUDA(cudaStreamSynchronize(st));
-  if (info != 0) throw Error(-3, "cusolverDnSsyevdx did not converge, info=" + std::to_string(info));
-  return meig;
-}
+void Solver::syevd(float* dA, int n, float* dW, bool vectors, cudaStream_t st) { syevd_tri(dA, n, dW, 0, vectors ? n : 0, st); }
 
 void Solver::dsyevd_small(double* dA, int n, double* dW, cudaStream_t st) {
   int lwork = 0;

@@ -11,24 +11,27 @@ struct Solver {
   ~Solver();
   Solver(const Solver&) = delete;
   Solver& operator=(const Solver&) = delete;
-  // cusolverDnSsyevd('V'|'N','U'): eigenvalues ascending in dW, eigenvectors overwrite dA (col-major)
+  // syevd_tri with all vectors (vectors = true) or none: eigenvalues ascending in dW, eigenvectors overwrite dA (col-major)
   void syevd(float* dA, int n, float* dW, bool vectors, cudaStream_t st);
   void dsyevd_small(double* dA, int n, double* dW, cudaStream_t st);
-  int syevdx_smallest(float* dA, int n, float* dW, int iu, cudaStream_t st);
-  // Own middle stage (tridiag.cu): cusolverDnSsytrd -> Float64 multisection + twisted factorisation -> cusolverDnSormtr.
-  // All n eigenvalues ascending in dW; the eigenvectors with ascending indices [v0, v1) in rows [v0, v1) of dA's memory
-  // (v0 == v1: values only); the other rows of dA are overwritten with scratch.  Falls back to Ssyevd on a kept copy of
-  // the matrix (all vectors) when the twisted factorisation fails; returns true when it did not have to.
+  // The own eigensolver: reduction to tridiagonal form -> Float64 multisection + twisted factorisation (tridiag.cu) ->
+  // back-transformation.  All n eigenvalues ascending in dW; the eigenvectors with ascending indices [v0, v1) in rows
+  // [v0, v1) of dA's memory (v0 == v1: values only); the other rows of dA are overwritten with scratch.  Orders >= 4 kBand take
+  // the two-stage reduction, smaller ones the one-stage path.  Falls back to Ssyevd on a kept copy of the matrix (all
+  // vectors) when the tridiagonal stage fails; returns true when it did not have to.
   bool syevd_tri(float* dA, int n, float* dW, int v0, int v1, cudaStream_t st);
+  // one stage: own tridiagonalisation (sytrd.cu; cusolverDnSsytrd where it declines), tridiag.cu, cusolverDnSormtr
   bool syevd_tri_one_stage(float* dA, int n, float* dW, int v0, int v1, cudaStream_t st);
-  // two-stage reduction (sy2sb.cu, sb2st.cu, backtrans.cu) with the same contract; SCL_EIG_API bit 5 routes syevd_tri here
+  // two-stage reduction (sy2sb.cu, sb2st.cu, backtrans.cu) with the same contract; a panel that cannot be factored or a failed
+  // tridiagonal stage falls back to syevd_tri_one_stage
   bool syevd_2stage(float* dA, int n, float* dW, int v0, int v1, cudaStream_t st);
   double ts_ms[5] = {0, 0, 0, 0, 0};   // last two-stage solve: dense->band, band->tridiagonal, tridiagonal eigenproblem, Q2, Q1 + copy
   bool tri_two_stage = false;
   // totals over the two-stage solves since the last reset: the five stages above, [5] solves, [6] eigenvector columns back-transformed
   double ts_total[7] = {0, 0, 0, 0, 0, 0, 0};
   int ts_fallbacks = 0;
-  // milliseconds of the last syevd_tri call: [0] Ssytrd, [1] eigenvalues + eigenvectors of T, [2] Sormtr + copy
+  // milliseconds of the last syevd_tri call: [0] reduction to tridiagonal form, [1] eigenvalues + eigenvectors of T,
+  // [2] back-transformation + copy
   double tri_ms[3] = {0, 0, 0};
   int tri_clusters = 0, tri_clustered = 0, tri_fallbacks = 0;
   bool tri_own_sytrd = false;   // the last syevd_tri call tridiagonalised with sytrd.cu
@@ -45,13 +48,10 @@ struct TridiagStats {
 bool tridiag_eigen(const float* d32, const float* e32, int n, double* w64, float* w32, int v0, int v1, float* Z,
                    long long ldz, cudaStream_t st, TridiagStats* stats);
 
-// SCL_EIG_API: bit 0 = Xsyevd for the full solves, bit 1 = Ssyevdx (index range) in the search steps, bit 2 = own tridiagonal
-// stage (Ssytrd + tridiag.cu + Sormtr) for every solve, bit 3 = with bit 2: vectors of the index range the search step uses only, bit 4 = with bit 2: own tridiagonalisation
-// (sytrd.cu) instead of cusolverDnSsytrd, bit 5 = with bit 2: two-stage reduction (twostage.h) for matrices of order >= 256
 // sytrd.cu: own Householder tridiagonalisation (persistent cooperative kernel), output as ssytrd('L'); false = not handled
 bool sytrd_lower(float* dA, int n, int lda, float* d_d, float* d_e, float* d_tau, cudaStream_t st);
-int eig_api();
-void set_eig_api(int v);   // process-wide override of SCL_EIG_API (tests, timing studies); < 0: back to the environment / default
+// test hook (process-wide): syevd_tri takes the one-stage path at every order, so that path is tested at orders >= 4 kBand
+void force_one_stage(bool on);
 
 struct MpFit {
   std::vector<float> L_mp;

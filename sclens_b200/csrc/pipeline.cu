@@ -784,7 +784,7 @@ struct SearchState {
 
 // device state shared by the search steps of one pass
 struct SearchCtx {
-  float bin_scale = 0, lmax_ref = 0;
+  float bin_scale = 0;
   int n_2 = 0, nw = 0;
   GemmOperand Vr;
   std::vector<float> Lh;
@@ -868,38 +868,17 @@ int search_step_solve(scl_handle* h, SearchCtx& c, SearchState& ss, int s_, scl_
   gram_of(h, Xp, Sp, h->ws_op_hi, h->ws_op_lo, G.p, nm, c.bin_scale, split);
   t_gram += tm.stop();
   int i0 = -1;
-  if ((eig_api() & 12) == 12) {
-    // own tridiagonal stage, vectors of the index range this step reads only (the nw smallest positive eigenpairs plus a
-    // margin for non-positive eigenvalues); all eigenvalues come back, so the "positive" threshold is exact
-    const int iu = std::min(nm, nw + 64);
-    { ProfScope ps(&h->prof, st, PK_SYEVD); h->solver->syevd_tri(G.p, nm, W.p, 0, iu, st); }
-    SCL_CUDA(cudaMemcpyAsync(c.Lh.data(), W.p, nm * sizeof(float), cudaMemcpyDeviceToHost, st));
-    SCL_CUDA(cudaStreamSynchronize(st));
-    const int j = first_positive(c.Lh);
-    if (j + nw <= iu) {
-      i0 = j;
-    } else {   // more than 64 non-positive eigenvalues: rebuild the Gram matrix and take the full solve below
-      gram_of(h, Xp, Sp, h->ws_op_hi, h->ws_op_lo, G.p, nm, c.bin_scale, split);
-    }
-  } else if (eig_api() & 2) {
-    // opt-in: only the nw smallest positive eigenpairs are used below, so ask the library for an index range.  The
-    // "positive" threshold needs the largest eigenvalue, which a range solve does not return: the reference basis'
-    // one (same matrix without the additions) stands in.  Falls back to the full solve when the range does not
-    // reach nw positive eigenvalues.
-    const int iu = std::min(nm, nw + 64);
-    Tmp<float> Gx((size_t)nm * nm, st);
-    SCL_CUDA(cudaMemcpyAsync(Gx.p, G.p, (size_t)nm * nm * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    int meig = 0;
-    { ProfScope ps(&h->prof, st, PK_SYEVD); meig = h->solver->syevdx_smallest(Gx.p, nm, W.p, iu, st); }
-    std::vector<float> Lx(meig);
-    SCL_CUDA(cudaMemcpyAsync(Lx.data(), W.p, meig * sizeof(float), cudaMemcpyDeviceToHost, st));
-    SCL_CUDA(cudaStreamSynchronize(st));
-    int j = 0;
-    while (j < meig && !(Lx[j] > 1e-5f * c.lmax_ref)) ++j;
-    if (j + nw <= meig) {
-      i0 = j;
-      SCL_CUDA(cudaMemcpyAsync(G.p, Gx.p, (size_t)(i0 + nw) * nm * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    }
+  // vectors of the index range this step reads only (the nw smallest positive eigenpairs plus a margin for non-positive
+  // eigenvalues); all eigenvalues come back, so the "positive" threshold is exact
+  const int iu = std::min(nm, nw + 64);
+  { ProfScope ps(&h->prof, st, PK_SYEVD); h->solver->syevd_tri(G.p, nm, W.p, 0, iu, st); }
+  SCL_CUDA(cudaMemcpyAsync(c.Lh.data(), W.p, nm * sizeof(float), cudaMemcpyDeviceToHost, st));
+  SCL_CUDA(cudaStreamSynchronize(st));
+  const int j = first_positive(c.Lh);
+  if (j + nw <= iu) {
+    i0 = j;
+  } else {   // more than 64 non-positive eigenvalues: rebuild the Gram matrix and take the full solve below
+    gram_of(h, Xp, Sp, h->ws_op_hi, h->ws_op_lo, G.p, nm, c.bin_scale, split);
   }
   if (i0 < 0) {
     { ProfScope ps(&h->prof, st, PK_SYEVD); h->solver->syevd(G.p, nm, W.p, true, st); }
@@ -1007,8 +986,7 @@ void robust_tail(scl_handle* h, double th, int n_perturb, double p_, Timer& tm) 
       if (!solved) {
         {
           ProfScope ps(&h->prof, st, PK_SYEVD);
-          if (eig_api() & 4) h->solver->syevd_tri(G.p, nm, W.p, nm - min_pc, nm, st);
-          else h->solver->syevd(G.p, nm, W.p, true, st);
+          h->solver->syevd_tri(G.p, nm, W.p, nm - min_pc, nm, st);
         }
         unscale_eigenvalues(h, W.p, nm);
         SCL_CUDA(cudaMemcpyAsync(Lh.data(), W.p, nm * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1093,7 +1071,6 @@ void run_robustness(scl_handle* h, double th, double p_step, int n_perturb) {
   if (h->sinfo.n_signal == 0) throw Error(SCL_ERR_NOSIGNAL, "warning: There is no signal");
   SCL_REQUIRE(n_perturb >= 2, "n_perturb must be >= 2");
   cudaStream_t st = h->st;
-  const int nm = std::min(h->X.N, h->X.M);
   scl_robust_info& info = h->rinfo;
   Timer tm(st);
   robust_prepare(h);
@@ -1103,9 +1080,6 @@ void run_robustness(scl_handle* h, double th, double p_step, int n_perturb) {
   SearchCtx c;
   search_ctx_init(h, c);
   binref_solve(h, c);
-  SCL_CUDA(cudaMemcpyAsync(c.Lh.data(), h->ws_W.p, nm * sizeof(float), cudaMemcpyDeviceToHost, st));
-  SCL_CUDA(cudaStreamSynchronize(st));
-  c.lmax_ref = c.Lh.back();   // largest eigenvalue of the binarised matrix (scale of the "positive" threshold)
   binref_operand(h, c, true);
   info.t_search_syevd_ms += tm.stop();
 
@@ -1229,7 +1203,6 @@ void run_pass(scl_handle* h, double th, double p_step, int n_perturb) {
   sync_errors(h, err);
 
   Tmp<double> wave_dev(G_, st);
-  Tmp<float> lmax_dev(1, st);
   bool have_fit = false, have_basis = false;
   const int refine_task = (refine && !signal_only) ? pass_refine_task(G_) : -1;
   std::vector<float> Lr(nm);
@@ -1261,8 +1234,6 @@ void run_pass(scl_handle* h, double th, double p_step, int n_perturb) {
       if (task == 2 && !signal_only) {  // reference basis of the binarised matrix (:717-721)
         tm.stop();
         binref_solve(h, c);
-        // its largest eigenvalue (scale of the "positive" threshold) before the data spectrum arrives in the same buffer
-        SCL_CUDA(cudaMemcpyAsync(lmax_dev.p, W.p + (nm - 1), sizeof(float), cudaMemcpyDeviceToDevice, st));
         rinfo.t_search_syevd_ms += tm.stop();
       }
       if (!signal_only && my_step >= 0 && ss.reachable(my_step)) i0 = search_step_solve(h, c, ss, my_step, rinfo, tm, t_gram);
@@ -1310,8 +1281,6 @@ void run_pass(scl_handle* h, double th, double p_step, int n_perturb) {
         const size_t cnt = (size_t)nm * (size_t)c.Vr.ld;
         SCL_NCCL(nccl_api().Broadcast(h->ws_vr_hi.p, h->ws_vr_hi.p, cnt, ncclHalf, r_bin, (ncclComm_t)h->nccl, st));
         SCL_NCCL(nccl_api().Broadcast(h->ws_vr_lo.p, h->ws_vr_lo.p, cnt, ncclHalf, r_bin, (ncclComm_t)h->nccl, st));
-        SCL_NCCL(nccl_api().Broadcast(lmax_dev.p, lmax_dev.p, 1, ncclFloat, r_bin, (ncclComm_t)h->nccl, st));
-        SCL_CUDA(cudaMemcpyAsync(&c.lmax_ref, lmax_dev.p, sizeof(float), cudaMemcpyDeviceToHost, st));
         SCL_CUDA(cudaStreamSynchronize(st));
         h->prof.comm_bytes += 4.0 * (double)cnt;
         have_basis = true;

@@ -11,9 +11,11 @@
 //      kBand x kBand matrix (U R)^-1.
 //   3. T is recomputed from the V actually stored: inv(T) = striu(V'V) + diag(V'V)/2 (k_tfactor), so I - V T V' is
 //      orthogonal to working precision whatever rounding V suffered; the band receives R' = S R.
-//   4. Two-sided update of the trailing matrix, lower triangle only: Y = A22 V (k_symm: every lower tile is used
-//      for its rows and, transposed, for its columns), Z = Y T, S2 = T'(V'Z), W = Z - V S2 / 2, A22 -= V W' + W V' (k_syr2k).
-// All large products run on the register-tiled FP32 engine of sgemm_tile.cuh; every reduction has a fixed order.
+//   4. Two-sided update of the trailing matrix, lower triangle only: Y = A22 V (k_symm_tc: every lower tile is used
+//      for its rows and, transposed, for its columns), Z = Y T, S2 = T'(V'Z), W = Z - V S2 / 2, A22 -= V W' + W V' (k_syr2k_tc).
+// The two large products (k_symm_tc, k_syr2k_tc) run on the tensor-core tile engines of sgemm_tile.cuh: split binary16 for a
+// matrix that passes half_range_ok, three-term TF32 otherwise; the panel-sized products run on its FP32 engine.  Every
+// reduction has a fixed order.
 #include <algorithm>
 #include <cmath>
 #include <vector>
@@ -26,12 +28,9 @@ namespace scl {
 namespace {
 
 constexpr int B = kBand;
-// rows per CTA of the panel dot products (SCL_S1_SLAB; a multiple of 64): fewer rows = more CTAs on these short kernels, which
-// sit on the critical path of every panel, against more partial matrices for the single-CTA kernels that sum them
-static int slab_rows() {
-  static const int v = [] { const char* e = getenv("SCL_S1_SLAB"); const int s = e ? atoi(e) : 256; return std::max(64, s / 64 * 64); }();
-  return v;
-}
+// rows per CTA of the panel dot products (a multiple of 64): fewer rows = more CTAs on these short kernels, which sit on the
+// critical path of every panel, against more partial matrices for the single-CTA kernels that sum them
+constexpr int kSlab = 256;
 
 // part[p][c1][c2] = sum over the rows of slab p of X[c1][i] * Y[c2][i].  F64 = true: every product accumulated in Float64 (the
 // panel Gram matrix, whose Cholesky factor squares the panel's condition number).  F64 = false: Float32 accumulation over 64
@@ -326,44 +325,8 @@ __global__ void __launch_bounds__(256, 2) k_panel_mul(const float* In, long long
 }
 
 // Ypart[s][c][i] = sum over k in chunk s of A22sym(i, k) * V[c][k]: the trailing matrix is read from its lower triangle
-// (tiles left of the diagonal as stored, the diagonal tile mirrored element by element, tiles below the diagonal transposed)
-__global__ void __launch_bounds__(256, 2) k_symm(const float* __restrict__ A22, long long lda, int m, const float* __restrict__ V,
-                                                 long long ldv, float* __restrict__ Ypart, long long ldy, int chunk) {
-  __shared__ __align__(16) float smem[tile::Smem<64>::floats];
-  const int i0 = (int)blockIdx.x * tile::TM;
-  const int ka = (int)blockIdx.y * chunk, kb = min(m, ka + chunk);
-  tile::Acc<64> acc;
-  acc.clear();
-  const int mi = m - i0;
-  {  // tiles left of the diagonal tile
-    const int k1 = min(kb, i0);
-    if (k1 > ka)
-      tile::mac<64>(acc, tile::opnd(A22 + i0 + (long long)ka * lda, lda, 0, mi, k1 - ka), tile::opnd(V + ka, ldv, 1, B, k1 - ka),
-                    k1 - ka, smem);
-  }
-  if (ka <= i0 && i0 < kb) {  // the diagonal tile (chunk boundaries are multiples of the tile size)
-    const int kl = min(tile::TM, mi);
-    tile::mac<64>(acc, tile::opnd(A22 + i0 + (long long)i0 * lda, lda, 2, mi, kl), tile::opnd(V + i0, ldv, 1, B, kl), kl, smem);
-  }
-  {  // tiles below the diagonal tile, read transposed
-    const int k3 = max(ka, i0 + tile::TM);
-    if (kb > k3)
-      tile::mac<64>(acc, tile::opnd(A22 + k3 + (long long)i0 * lda, lda, 1, mi, kb - k3), tile::opnd(V + k3, ldv, 1, B, kb - k3),
-                    kb - k3, smem);
-  }
-  float* out = Ypart + (size_t)blockIdx.y * B * ldy;
-#pragma unroll
-  for (int b = 0; b < 4; ++b) {
-    const int c = tile::Acc<64>::col(b);
-#pragma unroll
-    for (int a = 0; a < 8; ++a) {
-      const int i = i0 + tile::Acc<64>::row(a);
-      if (i < m) out[(long long)c * ldy + i] = acc.v[a][b];
-    }
-  }
-}
-
-// k_symm on the tensor-core tile engines (ENG 1: three-term TF32, 2: split binary16)
+// (tiles left of the diagonal as stored, the diagonal tile mirrored element by element, tiles below the diagonal transposed),
+// on the tensor-core tile engine ENG (1: three-term TF32, 2: split binary16)
 template <int ENG>
 __global__ void __launch_bounds__(256, 2) k_symm_tc(const float* __restrict__ A22, long long lda, int m, const float* __restrict__ V,
                                                     long long ldv, float* __restrict__ Ypart, long long ldy, int chunk) {
@@ -373,17 +336,17 @@ __global__ void __launch_bounds__(256, 2) k_symm_tc(const float* __restrict__ A2
   tile::AccT<64> acc;
   acc.clear();
   const int mi = m - i0;
-  {
+  {  // tiles left of the diagonal tile
     const int k1 = min(kb, i0);
     if (k1 > ka)
       tile::mac_e<ENG, 64, 0, 1>(acc, tile::opnd(A22 + i0 + (long long)ka * lda, lda, 0, mi, k1 - ka), tile::opnd(V + ka, ldv, 1, B, k1 - ka),
                        k1 - ka, smem);
   }
-  if (ka <= i0 && i0 < kb) {
+  if (ka <= i0 && i0 < kb) {  // the diagonal tile (chunk boundaries are multiples of the tile size)
     const int kl = min(tile::TM, mi);
     tile::mac_e<ENG, 64, 0, 1>(acc, tile::opnd(A22 + i0 + (long long)i0 * lda, lda, 2, mi, kl), tile::opnd(V + i0, ldv, 1, B, kl), kl, smem);
   }
-  {
+  {  // tiles below the diagonal tile, read transposed
     const int k3 = max(ka, i0 + tile::TM);
     if (kb > k3)
       tile::mac_e<ENG, 64, 1, 1>(acc, tile::opnd(A22 + k3 + (long long)i0 * lda, lda, 1, mi, kb - k3), tile::opnd(V + k3, ldv, 1, B, kb - k3),
@@ -409,58 +372,14 @@ __global__ void k_sum_parts(const float* __restrict__ part, int nparts, size_t s
   out[i] = s;
 }
 
-// A22 -= V W' + W V', lower triangle, one 128 x 128 tile per CTA
-__global__ void __launch_bounds__(256, 2) k_syr2k(float* A22, long long lda, int m, const float* __restrict__ V, long long ldv,
-                                                  const float* __restrict__ W, long long ldw, int mode) {
-  __shared__ __align__(16) float smem[tile::Smem<128>::floats];
-  // mode 0: linear tile index -> (I, J), J <= I.  mode 1: the first tile column only (J = 0).  mode 2: everything else.
-  const int t = (int)blockIdx.x;
-  int I, J;
-  if (mode == 1) {
-    I = t;
-    J = 0;
-  } else {
-    I = (int)((sqrtf(8.f * (float)t + 1.f) - 1.f) * 0.5f);
-    while ((I + 1) * (I + 2) / 2 <= t) ++I;
-    while (I * (I + 1) / 2 > t) --I;
-    J = t - I * (I + 1) / 2;
-    if (mode == 2) {
-      ++I;
-      ++J;
-    }
-  }
-  const int i0 = I * tile::TM, j0 = J * tile::TM;
-  tile::Acc<128> acc;
-  acc.clear();
-  tile::mac<128>(acc, tile::opnd(V + i0, ldv, 0, m - i0, B), tile::opnd(W + j0, ldw, 0, m - j0, B), B, smem);
-  tile::mac<128>(acc, tile::opnd(W + i0, ldw, 0, m - i0, B), tile::opnd(V + j0, ldv, 0, m - j0, B), B, smem);
-#pragma unroll
-  for (int b = 0; b < 8; ++b) {
-    const int j = j0 + tile::Acc<128>::col(b);
-    if (j >= m) continue;
-    float* col = A22 + (long long)j * lda;
-#pragma unroll
-    for (int a4 = 0; a4 < 2; ++a4) {
-      const int i = i0 + tile::Acc<128>::row(a4 * 4);
-      if (i + 3 < m && i >= j) {
-        float4 c = *reinterpret_cast<float4*>(col + i);
-        c.x -= acc.v[a4 * 4 + 0][b]; c.y -= acc.v[a4 * 4 + 1][b]; c.z -= acc.v[a4 * 4 + 2][b]; c.w -= acc.v[a4 * 4 + 3][b];
-        *reinterpret_cast<float4*>(col + i) = c;
-      } else {
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          if (i + q < m && i + q >= j) col[i + q] -= acc.v[a4 * 4 + q][b];
-      }
-    }
-  }
-}
-
-// k_syr2k on the tensor-core tile engine: the tile is formed transposed (columns j of the trailing matrix on the rows of the
-// accumulator, rows i on its columns), so a thread's two adjacent outputs are adjacent in memory
+// A22 -= V W' + W V', lower triangle, one 128 x 128 tile per CTA, on the tensor-core tile engine ENG.  The tile is formed
+// transposed (columns j of the trailing matrix on the rows of the accumulator, rows i on its columns), so a thread's two
+// adjacent outputs are adjacent in memory.
 template <int ENG>
 __global__ void __launch_bounds__(256, 2) k_syr2k_tc(float* A22, long long lda, int m, const float* __restrict__ V, long long ldv,
                                                      const float* __restrict__ W, long long ldw, int mode) {
   __shared__ __align__(16) unsigned char smem[tile::SmemE<ENG, 128>::bytes];
+  // mode 0: linear tile index -> (I, J), J <= I.  mode 1: the first tile column only (J = 0).  mode 2: everything else.
   const int t = (int)blockIdx.x;
   int I, J;
   if (mode == 1) {
@@ -672,7 +591,6 @@ bool half_range_ok(const float* A, int n, long long lda, cudaStream_t st) {
 int sy2sb_lower(float* A, int n, long long lda, float* AB, float* T1, int* d_fail, cudaStream_t st, const Sy2sbAux* aux, bool half_ok) {
   SCL_REQUIRE((lda & 3) == 0 && ((uintptr_t)A & 15) == 0 && lda >= n, "sy2sb: leading dimension must be a multiple of 4");
   const long long ldy = ((long long)n + 3) & ~3LL;
-  const int kSlab = slab_rows();
   const int max_slabs = (n + kSlab - 1) / kSlab + 1;
   const int max_split = 16;
   Tmp<double> part((size_t)max_slabs * B * B, st), psum((size_t)B * B, st);
@@ -688,8 +606,7 @@ int sy2sb_lower(float* A, int n, long long lda, float* AB, float* T1, int* d_fai
     attr_done = true;
   }
   const int slots = 2 * sm_count();
-  const int eng = (tile_engine_s1() == 2 && !half_ok) ? 1 : tile_engine_s1();   // split binary16 only for a matrix within its range
-  const bool tc = eng != 0;
+  const int eng = half_ok ? 2 : 1;   // split binary16 only for a matrix within its range
   long launches = 0;
   // factorisation of panel k (full-size panels only) on stream s: V in place, T, V T into the upper triangle, R' into the band
   auto factor = [&](int k, cudaStream_t s) {
@@ -735,8 +652,7 @@ int sy2sb_lower(float* A, int n, long long lda, float* AB, float* T1, int* d_fai
     chunk = std::max(chunk, 2 * tile::TM);
     split = (m + chunk - 1) / chunk;
     if (eng == 2) k_symm_tc<2><<<dim3(ntile, split), 256, 0, st>>>(A22, lda, m, Pp, lda, Ypart.p, ldy, chunk);
-    else if (tc) k_symm_tc<1><<<dim3(ntile, split), 256, 0, st>>>(A22, lda, m, Pp, lda, Ypart.p, ldy, chunk);
-    else k_symm<<<dim3(ntile, split), 256, 0, st>>>(A22, lda, m, Pp, lda, Ypart.p, ldy, chunk);
+    else k_symm_tc<1><<<dim3(ntile, split), 256, 0, st>>>(A22, lda, m, Pp, lda, Ypart.p, ldy, chunk);
     const size_t ny = (size_t)B * ldy;
     k_sum_parts<<<(unsigned)((ny + 255) / 256), 256, 0, st>>>(Ypart.p, split, ny, ny, Y.p);
     k_panel_mul<<<ntile, 256, 0, st>>>(Y.p, ldy, Tk, Z.p, ldy, m, 1.f, nullptr, 0, 0);
@@ -750,22 +666,19 @@ int sy2sb_lower(float* A, int n, long long lda, float* AB, float* T1, int* d_fai
     const bool ahead = aux && aux->stream && ntile >= 4 && m - B >= B;
     if (ahead) {
       if (eng == 2) k_syr2k_tc<2><<<ntile, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 1);
-      else if (tc) k_syr2k_tc<1><<<ntile, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 1);
-      else k_syr2k<<<ntile, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 1);
+      else k_syr2k_tc<1><<<ntile, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 1);
       SCL_CUDA(cudaEventRecord(aux->ready, st));
       SCL_CUDA(cudaStreamWaitEvent(aux->stream, aux->ready, 0));
       factor(k + 1, aux->stream);
       SCL_CUDA(cudaEventRecord(aux->done, aux->stream));
       if (eng == 2) k_syr2k_tc<2><<<(ntile - 1) * ntile / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 2);
-      else if (tc) k_syr2k_tc<1><<<(ntile - 1) * ntile / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 2);
-      else k_syr2k<<<(ntile - 1) * ntile / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 2);
+      else k_syr2k_tc<1><<<(ntile - 1) * ntile / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 2);
       SCL_CUDA(cudaStreamWaitEvent(st, aux->done, 0));
       factored = true;
       ++launches;
     } else {
       if (eng == 2) k_syr2k_tc<2><<<ntile * (ntile + 1) / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 0);
-      else if (tc) k_syr2k_tc<1><<<ntile * (ntile + 1) / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 0);
-      else k_syr2k<<<ntile * (ntile + 1) / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 0);
+      else k_syr2k_tc<1><<<ntile * (ntile + 1) / 2, 256, 0, st>>>(A22, lda, m, Pp, lda, Z.p, ldy, 0);
     }
     ++launches;
   }

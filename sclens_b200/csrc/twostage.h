@@ -7,8 +7,6 @@
 // The algebra is restated on the CPU in oracle/two_stage_ref.py (tests/test_two_stage_cpu.py).
 #pragma once
 #include <cuda_runtime.h>
-#include <atomic>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace scl {
@@ -49,22 +47,13 @@ void apply_q2(const float* V2, long long ldv2, const float* tau2, long long ldt2
 void apply_q1(const float* A, int n, long long lda, const float* T1, int npanels, float* Z, long long ldz, int mvec,
               cudaStream_t st);
 
-// which engine runs the matrix-matrix products.  Tile engines of sgemm_tile.cuh: 0 = FP32 FMA, 1 = tensor cores in three-term
-// TF32 (mma.sync), 2 = tensor cores in split binary16 (mma.sync; operands must be O(1)).  3 (Q1 only): eight panels at a time on
-// the tcgen05 GEMM of gemm_umma.cu in split binary16 (backtrans.cu, apply_q1_umma).  SCL_TILE_ENGINE sets stage 1 (default 2, which
-// applies only to a matrix whose Frobenius norm passes half_range_ok - otherwise 1 runs; 304 vs 369 ms at n = 20 000), SCL_TILE_ENGINE_Q1 the Q1 back-transformation (default 3; measured at n = 20 000,
-// smallest half / all vectors: 83 / 130 ms against 192 / 366 ms for 2, 251 / 474 ms for 1, 252 / 487 ms for 0).
-// run-time overrides for the parity tests (scl_debug_set_two_stage): [0] Q2 variant, [1] stage-1 engine, [2] Q1 engine; < 0 = unset
-extern std::atomic<int> g_two_stage_override[3];
-inline int two_stage_choice(int which, const char* env, int dflt) {
-  const int o = g_two_stage_override[which].load(std::memory_order_relaxed);
-  if (o >= 0) return o;
-  const char* e = getenv(env);
-  return e ? atoi(e) : dflt;
-}
-inline int q2_variant() { return two_stage_choice(0, "SCL_Q2_VARIANT", 2); }
-inline int tile_engine_s1() { return two_stage_choice(1, "SCL_TILE_ENGINE", 2); }
-inline int tile_engine_q1() { return two_stage_choice(2, "SCL_TILE_ENGINE_Q1", 3); }
+// Engines of the matrix-matrix products, each chosen by the input (measured at n = 20 000; a / b = smallest half / all vectors):
+//   stage 1   split binary16 on the mma.sync tile engine of sgemm_tile.cuh when the matrix passes half_range_ok, three-term
+//             TF32 otherwise (304 vs 369 ms; FP32 FMA took 394 ms against 370 ms for TF32 in an earlier run)
+//   Q2        register-stationary split binary16 (254 / 440 ms; three-term TF32 380 / 558 ms, a shared-memory window 818 / 1627 ms)
+//   Q1        64 vectors or more: eight panels at a time on the tcgen05 GEMM of gemm_umma.cu in split binary16 (83 / 130 ms);
+//             fewer: panel by panel on the split-binary16 tile engine (192 / 366 ms at this size, where it is not used; TF32
+//             251 / 474 ms, FP32 FMA 252 / 487 ms)
 
 // every vector scaled to unit length (after the back-transformation: the tensor-core products of apply_q2 lose ~1e-7 n / 64)
 void unit_vectors(float* Z, long long ldz, int n, int mvec, cudaStream_t st);

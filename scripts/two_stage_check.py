@@ -83,16 +83,16 @@ with Handle() as h:
             h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double))
             return ms.value, [round(float(x), 2) for x in st]
 
-        for name, api, mode, il, iu in (("one_stage_values_only", 28, 8, 0, 0), ("two_stage_values_only", 60, 8, 0, 0),
-                                        ("two_stage_values_only_2", 60, 8, 0, 0),
-                                        ("two_stage_smallest_half", 60, 7, 1, n // 2 + 65), ("two_stage_all_vectors", 60, 6, 0, 0),
-                                        ("one_stage_smallest_half", 28, 7, 1, n // 2 + 65)):
-            h.lib.scl_debug_set_eig_api(api)
+        for name, one_stage, mode, il, iu in (("one_stage_values_only", 1, 8, 0, 0), ("two_stage_values_only", 0, 8, 0, 0),
+                                              ("two_stage_values_only_2", 0, 8, 0, 0),
+                                              ("two_stage_smallest_half", 0, 7, 1, n // 2 + 65), ("two_stage_all_vectors", 0, 6, 0, 0),
+                                              ("one_stage_smallest_half", 1, 7, 1, n // 2 + 65)):
+            h._ck(h.lib.scl_debug_force_one_stage(one_stage))
             try:
                 out[name] = bench(mode, il, iu)
             except Exception as ex:  # noqa: BLE001
                 out[name] = str(ex)
             print(name, out[name], flush=True)
-        h.lib.scl_debug_set_eig_api(-1)
+        h.lib.scl_debug_force_one_stage(0)
         report["timing_%d" % n] = out
 open("gpurun_out/r2_two_stage_check.json", "w").write(json.dumps(report, indent=1))

@@ -300,20 +300,24 @@ def test_syevd_tri_matches_float64(h, case):
 
 @pytest.mark.parametrize("n", [300, 1000, 2531])
 def test_own_tridiagonalisation_matches_float64(h, n):
-    """sytrd.cu (persistent cooperative Householder tridiagonalisation, lower triangle only) in place of cusolverDnSsytrd:
-    the full solve through it - eigenvalues, residuals, orthogonality - against numpy's Float64 eigh, same tolerances as the
-    library path; shapes that are not multiples of the 32-column panel or the 128 x 128 update tile."""
+    """The one-stage path, forced at every order (scl_debug_force_one_stage): sytrd.cu (persistent cooperative Householder
+    tridiagonalisation, lower triangle only), the own tridiagonal stage and Sormtr - eigenvalues, residuals, orthogonality -
+    against numpy's Float64 eigh, same tolerances as the library path; shapes that are not multiples of the 32-column panel or
+    the 128 x 128 update tile."""
     rng = np.random.default_rng(n)
     A = rng.standard_normal((n, n + 300))
     A -= A.mean(axis=0)
     G = (A @ A.T / A.shape[1]).astype(np.float32)
     Lref = np.linalg.eigvalsh(G.astype(np.float64))
+    st = np.zeros(8)
     try:
-        h.lib.scl_debug_set_eig_api(4 | 8 | 16)
+        h._ck(h.lib.scl_debug_force_one_stage(1))
         L, V, out = _tri_solve(h, G, 0, n)
+        h._ck(h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double)))
     finally:
-        h.lib.scl_debug_set_eig_api(-1)
+        h.lib.scl_debug_force_one_stage(0)
     assert out[5] == 0, "fell back to the library solver"
+    assert st[5] == 0, ("the two-stage path produced the result", st)
     np.testing.assert_allclose(L, Lref, rtol=2e-5, atol=3e-6 * float(Lref[-1]))
     G64 = G.astype(np.float64)
     assert np.max(np.abs(G64 @ V - V * L[None, :])) < 5e-5 * max(1.0, float(Lref[-1]))
@@ -518,15 +522,15 @@ def test_scores_match_oracle(h):
     np.testing.assert_array_equal(sid[:nrob.value], sig)
 
 
-TWO_STAGE = 4 | 8 | 16 | 32
-
-
-@pytest.mark.parametrize("n,case", [(300, "wishart"), (1000, "centred"), (2531, "wishart"), (1536, "wide_range_of_scales")])
+@pytest.mark.parametrize("n,case", [(300, "wishart"), (1000, "centred"), (1203, "centred"), (2531, "wishart"),
+                                    (1536, "wide_range_of_scales")])
 def test_two_stage_solver_matches_float64(h, n, case):
-    """Two-stage reduction (sy2sb.cu dense -> band, sb2st.cu band -> tridiagonal by bulge chasing, backtrans.cu) behind
-    SCL_EIG_API bit 5: eigenvalues, residuals and orthogonality against numpy's Float64 eigh of the same FP32 matrix, with the
+    """Two-stage reduction (sy2sb.cu dense -> band, sb2st.cu band -> tridiagonal by bulge chasing, backtrans.cu), the path of
+    every order >= 256: eigenvalues, residuals and orthogonality against numpy's Float64 eigh of the same FP32 matrix, with the
     tolerances of the one-stage path; orders that are not multiples of the 64-column panel, the 128 x 128 update tile or 4
-    (padded copy); all vectors / an index range / values only agree."""
+    (padded copy); all vectors / an index range / values only agree.  Stage 1 multiplies in split binary16 when
+    n / 8192 <= |G|_F <= 1024 and in three-term TF32 otherwise: the graded rows of "wide_range_of_scales" take TF32, the
+    other cases split binary16."""
     rng = np.random.default_rng(n)
     A = rng.standard_normal((n, n + 300))
     if case == "centred":
@@ -534,19 +538,17 @@ def test_two_stage_solver_matches_float64(h, n, case):
     if case == "wide_range_of_scales":
         A *= np.exp(rng.normal(0, 1.5, size=(n, 1)))
     G = (A @ A.T / A.shape[1]).astype(np.float32)
+    fro = np.linalg.norm(G.astype(np.float64))
+    assert (n / 8192 <= fro <= 1024) == (case != "wide_range_of_scales"), fro
     Lref = np.linalg.eigvalsh(G.astype(np.float64))
     scale = float(Lref[-1])
     st, st0 = np.zeros(8), np.zeros(8)
     h.lib.scl_debug_last_solve(h.h, ptr(st0, C.c_double))   # fallback counters are cumulative per handle
-    try:
-        h.lib.scl_debug_set_eig_api(TWO_STAGE)
-        L, V, out = _tri_solve(h, G, 0, n)
-        h._ck(h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double)))
-        v0, v1 = 3, n // 2 + 40
-        L2, V2, _ = _tri_solve(h, G, v0, v1)
-        L3, _, _ = _tri_solve(h, G, 0, 0)
-    finally:
-        h.lib.scl_debug_set_eig_api(-1)
+    L, V, out = _tri_solve(h, G, 0, n)
+    h._ck(h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double)))
+    v0, v1 = 3, n // 2 + 40
+    L2, V2, _ = _tri_solve(h, G, v0, v1)
+    L3, _, _ = _tri_solve(h, G, 0, 0)
     assert out[5] == 0 and st[5] == 1 and st[6] == st0[6], ("the two-stage path did not produce the result", out, st, st0)
     np.testing.assert_allclose(L, Lref, rtol=2e-5, atol=3e-6 * scale)
     G64 = G.astype(np.float64)
@@ -557,34 +559,6 @@ def test_two_stage_solver_matches_float64(h, n, case):
     np.testing.assert_array_equal(L3, L)
 
 
-@pytest.mark.parametrize("q2,s1,q1", [(0, 0, 0), (1, 1, 1), (2, 1, 2), (2, 0, 3), (2, 2, 3)])
-def test_two_stage_kernel_variants_agree(h, q2, s1, q1):
-    """Every selectable kernel variant of the two-stage solver (scl_debug_set_two_stage: stage-2 back-transformation in FP32 from a
-    shared-memory window / register-stationary three-term TF32 / split binary16; tile engines FP32 FMA / TF32 / split binary16 /
-    tcgen05 block reflectors) meets the tolerances of the default path on one matrix whose order is not a multiple of anything."""
-    n = 1203
-    rng = np.random.default_rng(77)
-    A = rng.standard_normal((n, n + 500))
-    A -= A.mean(axis=0)
-    G = (A @ A.T / A.shape[1]).astype(np.float32)
-    Lref = np.linalg.eigvalsh(G.astype(np.float64))
-    scale = float(Lref[-1])
-    st = np.zeros(8)
-    try:
-        h.lib.scl_debug_set_eig_api(TWO_STAGE)
-        h.lib.scl_debug_set_two_stage(q2, s1, q1)
-        L, V, out = _tri_solve(h, G, 0, n)
-        h._ck(h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double)))
-    finally:
-        h.lib.scl_debug_set_two_stage(-1, -1, -1)
-        h.lib.scl_debug_set_eig_api(-1)
-    assert out[5] == 0 and st[5] == 1, ("the two-stage path did not produce the result", out, st)
-    np.testing.assert_allclose(L, Lref, rtol=2e-5, atol=3e-6 * scale)
-    G64 = G.astype(np.float64)
-    assert np.max(np.abs(G64 @ V - V * L[None, :])) < 5e-5 * max(1.0, scale)
-    assert np.max(np.abs(V.T.astype(np.float64) @ V - np.eye(n))) < 5e-5
-
-
 @pytest.mark.parametrize("v0,v1", [(100, 110), (0, 1), (650, 700)])
 def test_two_stage_few_vectors(h, v0, v1):
     """An index range of a few eigenvectors (one 16-vector tile of the stage-2 kernel, the panel-by-panel stage-1
@@ -593,12 +567,8 @@ def test_two_stage_few_vectors(h, v0, v1):
     rng = np.random.default_rng(3)
     A = rng.standard_normal((n, n + 200))
     G = (A @ A.T / A.shape[1]).astype(np.float32)
-    try:
-        h.lib.scl_debug_set_eig_api(TWO_STAGE)
-        L, V, out = _tri_solve(h, G, 0, n)
-        L2, V2, out2 = _tri_solve(h, G, v0, v1)
-    finally:
-        h.lib.scl_debug_set_eig_api(-1)
+    L, V, out = _tri_solve(h, G, 0, n)
+    L2, V2, out2 = _tri_solve(h, G, v0, v1)
     assert out[5] == 0 and out2[5] == 0
     np.testing.assert_array_equal(L2, L)
     assert np.max(np.abs(np.abs(np.sum(V2 * V[:, v0:v1], axis=0)) - 1.0)) < 1e-5
@@ -616,12 +586,8 @@ def test_two_stage_solver_rank_deficient_panels_fall_back(h):
     G[:nb, :nb] = Bm
     G[nb:2 * nb, nb:2 * nb] = Bm
     st = np.zeros(8)
-    try:
-        h.lib.scl_debug_set_eig_api(TWO_STAGE)
-        L, V, out = _tri_solve(h, G, 0, n)
-        h._ck(h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double)))
-    finally:
-        h.lib.scl_debug_set_eig_api(-1)
+    L, V, out = _tri_solve(h, G, 0, n)
+    h._ck(h.lib.scl_debug_last_solve(h.h, ptr(st, C.c_double)))
     Lref = np.linalg.eigvalsh(G.astype(np.float64))
     np.testing.assert_allclose(L, Lref, rtol=2e-5, atol=5e-6)
     assert np.max(np.abs(G.astype(np.float64) @ V - V * L[None, :])) < 5e-5
