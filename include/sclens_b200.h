@@ -42,7 +42,8 @@ enum {
   SCL_ERR_CUSOLVER = -3,  /* cuSOLVER error or non-convergence (reference NaN fallback :379-381 is an error here) */
   SCL_ERR_NOGPU = -4,     /* no sm_100 device: there is no CPU fallback */
   SCL_ERR_NCCL = -5,
-  SCL_ERR_NOSIGNAL = -6   /* scl_run_robustness called with zero signals (:780-784) */
+  SCL_ERR_NOSIGNAL = -6,  /* scl_run_robustness called with zero signals (:780-784) */
+  SCL_ERR_GRAPH = -7      /* a clustering input graph is not a symmetric CSR with sorted columns and finite positive weights */
 };
 
 /* Gram operand precision. FP16: one tcgen05 kind::f16 pass. FP16X3: hi/lo split, three
@@ -317,6 +318,77 @@ SCL_API int32_t scl_get_umap_graph(scl_handle* h, int64_t* nnz, uint32_t* rowptr
 SCL_API int32_t scl_get_umap_knn(scl_handle* h, int32_t* idx, float* dist);
 /* The a / b fit of UMAP_ (Levenberg-Marquardt on the host, Float64).  Pure host code. */
 SCL_API int32_t scl_umap_fit_ab(double min_dist, double spread, double* a, double* b);
+
+/* ---- clustering (scICE clustering!: Leiden trials over resolutions, IC of each cluster count) on the device ---------- */
+/* Leiden with the modularity objective and resolution gamma (RB configuration model).  Weights are fixed point
+ * round(w 2^shift) (at least 1), shift <= 32 from the largest weight and nnz; every trial's draws hash (seed, trial).
+ * Defaults in the host mirrors: n_trials 50, max_iterations 10, max_sweeps 64, theta 0.01, seed 0. */
+typedef struct {
+  int32_t n_trials;          /* T >= 1 trials per resolution */
+  int32_t max_iterations;    /* >= 1: restarts from the last labels until one changes no label */
+  int32_t max_sweeps;        /* >= 1: local-moving sweeps per level (a level that reaches it is counted in capped_levels) */
+  int32_t reserved0;
+  double theta;              /* > 0: randomness of the refinement (probability ~ exp(gain / theta), leidenalg's 0.01) */
+  uint64_t seed;
+  int32_t reserved[4];
+} scl_leiden_params;
+
+typedef struct {
+  int32_t max_levels;        /* most levels of one iteration of one trial */
+  int32_t max_iterations;    /* most iterations of one trial */
+  int32_t capped_levels;     /* levels whose local moving stopped at max_sweeps */
+  int32_t weight_shift;      /* the fixed-point exponent */
+  int64_t copy_levels;       /* sum over trials and iterations of the levels run */
+  double t_validate_ms, t_move_ms, t_refine_ms, t_aggregate_ms, t_labels_ms;   /* CUDA events / host clock around synchronised work */
+  int32_t reserved[4];
+} scl_leiden_info;
+
+/* Resolution search of the clustering: for every k in [k_min, k_max] the resolution whose trials most often give exactly k
+ * clusters, and the IC of those trials.  Defaults: k_min 2, k_max 20, n_trials 50, max_rounds 12, n_grid 16, max_widen 4,
+ * gamma_lo 0.01, gamma_hi 10, and the Leiden defaults above. */
+typedef struct {
+  int32_t k_min, k_max;      /* 1 <= k_min <= k_max <= N */
+  int32_t n_trials;          /* >= 2 */
+  int32_t max_rounds;        /* >= 0 bisection / widening rounds after the start grid */
+  int32_t n_grid;            /* >= 2 log-spaced resolutions of the start grid on [gamma_lo, gamma_hi] */
+  int32_t max_widen;         /* decades the search may add below gamma_lo and above gamma_hi */
+  int32_t max_iterations, max_sweeps;
+  double gamma_lo, gamma_hi, theta;
+  uint64_t seed;
+  int32_t reserved[4];
+} scl_cluster_params;
+
+typedef struct {
+  int32_t n_rounds;          /* batches run, the start grid included */
+  int32_t n_evaluated;       /* resolutions evaluated */
+  int32_t n_found;           /* cluster counts in [k_min, k_max] found */
+  int32_t weight_shift;
+  int64_t copy_levels;
+  double t_validate_ms, t_leiden_ms, t_ecs_ms, t_total_ms;
+  int32_t reserved[4];
+} scl_cluster_info;
+
+/* R x T Leiden trials on an N-vertex graph.  rowptr (N+1) / colidx / val (nnz): symmetric CSR, sorted columns, 0-based,
+ * finite positive weights (validated on the device: SCL_ERR_GRAPH otherwise); rowptr == NULL takes the fuzzy graph of
+ * the handle's last scl_op_umap.  labels: [R][T][N] (ids 0..k-1 by cluster size, descending, ties by smallest member),
+ * n_clusters / modularity: [R][T].  A trial's labels do not depend on the other trials of the batch. */
+SCL_API int32_t scl_op_leiden(scl_handle* h, int32_t N, int64_t nnz, const uint32_t* rowptr, const uint32_t* colidx,
+                              const double* val, int32_t R, const double* resolutions, const scl_leiden_params* p,
+                              int32_t* labels, int32_t* n_clusters, double* modularity, scl_leiden_info* info);
+/* T x T element-centric similarity (row-major) of T labelings [T][N] with ids in [0, N). */
+SCL_API int32_t scl_op_label_ecs(scl_handle* h, int32_t T, int32_t N, const int32_t* labels, double* ecs);
+/* The whole search (graph as scl_op_leiden).  Per k = k_min + i: found[i] (0 / 1), gamma[i], share[i] (fraction of the
+ * trials at gamma[i] with exactly k clusters), ic[i] (1 / p^T S p over all trials at gamma[i]) and labels[i][N] (of the
+ * trials with exactly k clusters, the one with the largest ECS row sum, ties to the lowest); entries of a k not found are 0 / NaN / -1.  eval_gamma / eval_mode
+ * (capacity eval_cap, may be NULL) receive the evaluated resolutions and their modal cluster counts in evaluation order. */
+SCL_API int32_t scl_op_cluster(scl_handle* h, int32_t N, int64_t nnz, const uint32_t* rowptr, const uint32_t* colidx,
+                               const double* val, const scl_cluster_params* p, int32_t* found, double* gamma, double* share,
+                               double* ic, int32_t* labels, int32_t eval_cap, double* eval_gamma, int32_t* eval_mode,
+                               scl_cluster_info* info);
+/* One planning step of the search (host only): from n evaluated (gamma, modal count) pairs, the next resolutions (at most
+ * k_max - k_min + 3, ascending; *n_out = 0 when the search is done). */
+SCL_API int32_t scl_cluster_plan(int32_t n, const double* gammas, const int32_t* modes, const scl_cluster_params* p,
+                                 double* out, int32_t* n_out);
 
 /* ---- kernel-level timing harness (device-resident synthetic operands; used by bench.py and the ncu captures) ---- */
 /* Gram / GEMM kernel alone: rows x K binary16 operand generated on the device; mode bit0 = split (hi+lo) operands,

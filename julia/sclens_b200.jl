@@ -53,6 +53,33 @@ mutable struct SclUmapInfo
     reserved::NTuple{4,Int32}
     SclUmapInfo() = new()
 end
+struct SclLeidenParams
+    n_trials::Int32; max_iterations::Int32; max_sweeps::Int32; reserved0::Int32
+    theta::Float64
+    seed::UInt64
+    reserved::NTuple{4,Int32}
+end
+mutable struct SclLeidenInfo
+    max_levels::Int32; max_iterations::Int32; capped_levels::Int32; weight_shift::Int32
+    copy_levels::Int64
+    t_validate_ms::Float64; t_move_ms::Float64; t_refine_ms::Float64; t_aggregate_ms::Float64; t_labels_ms::Float64
+    reserved::NTuple{4,Int32}
+    SclLeidenInfo() = new()
+end
+struct SclClusterParams
+    k_min::Int32; k_max::Int32; n_trials::Int32; max_rounds::Int32
+    n_grid::Int32; max_widen::Int32; max_iterations::Int32; max_sweeps::Int32
+    gamma_lo::Float64; gamma_hi::Float64; theta::Float64
+    seed::UInt64
+    reserved::NTuple{4,Int32}
+end
+mutable struct SclClusterInfo
+    n_rounds::Int32; n_evaluated::Int32; n_found::Int32; weight_shift::Int32
+    copy_levels::Int64
+    t_validate_ms::Float64; t_leiden_ms::Float64; t_ecs_ms::Float64; t_total_ms::Float64
+    reserved::NTuple{4,Int32}
+    SclClusterInfo() = new()
+end
 
 function check(h, rc)
     rc == 0 && return
@@ -208,6 +235,102 @@ function apply_umap!(l_inp; k=15, nc=2, md=0.1, metric=:cosine, n_epochs=300, se
         ccall((:scl_destroy, LIB), Int32, (Ptr{Cvoid},), h)
     end
     l_inp
+end
+
+"""
+    clustering!(l_inp; k_min=2, k_max=20, n_trials=50, seed=0)
+
+scICE-style clustering on the device from `l_inp[:umap_obj].graph` (run `apply_umap!` first): `n_trials` Leiden trials
+per resolution, a resolution search for every cluster count in k_min:k_max and the inconsistency coefficient of each.
+Stores `:graph`, `:n_cluster` (the counts found), `:ic` (aligned with `:n_cluster`), `:l_df` (DataFrame: `:cell` plus
+one column `:k_<k>` per found count, labels 1..k by cluster size) and `:cluster_obj` (gamma, share, info).
+"""
+function clustering!(l_inp; k_min=2, k_max=20, n_trials=50, seed=0, max_rounds=12)
+    graph = l_inp[:umap_obj].graph                      # symmetric: its CSC arrays are the CSR arrays
+    N = size(graph, 1)
+    rowptr = UInt32.(graph.colptr .- 1); colidx = UInt32.(graph.rowval .- 1); val = Float64.(graph.nzval)
+    p = Ref(SclClusterParams(k_min, k_max, n_trials, max_rounds, 16, 4, 10, 64, 0.01, 10.0, 0.01, UInt64(seed),
+                             ntuple(_ -> Int32(0), 4)))
+    nk = k_max - k_min + 1
+    found = Vector{Int32}(undef, nk); gam = Vector{Float64}(undef, nk); share = Vector{Float64}(undef, nk)
+    ic = Vector{Float64}(undef, nk); labels = Matrix{Int32}(undef, N, nk)     # row-major nk x N == column-major N x nk
+    info = Ref(SclClusterInfo())
+    hr = Ref{Ptr{Cvoid}}(C_NULL)
+    cfg = Ref(default_config())
+    rc = ccall((:scl_create, LIB), Int32, (Ptr{Ptr{Cvoid}}, Ptr{SclConfig}), hr, cfg)
+    rc == 0 || check(C_NULL, rc)
+    h = hr[]
+    try
+        check(h, ccall((:scl_op_cluster, LIB), Int32,
+                       (Ptr{Cvoid}, Int32, Int64, Ptr{UInt32}, Ptr{UInt32}, Ptr{Float64}, Ptr{SclClusterParams}, Ptr{Int32},
+                        Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Int32, Ptr{Float64}, Ptr{Int32}, Ptr{SclClusterInfo}),
+                       h, N, length(val), rowptr, colidx, val, p, found, gam, share, ic, labels, 0, C_NULL, C_NULL, info))
+    finally
+        ccall((:scl_destroy, LIB), Int32, (Ptr{Cvoid},), h)
+    end
+    ks = [k_min + i - 1 for i in 1:nk if found[i] != 0]
+    sel = [i for i in 1:nk if found[i] != 0]
+    l_df = DataFrame(:cell => l_inp[:cell_id])
+    for (k, i) in zip(ks, sel)
+        l_df[!, Symbol("k_$(k)")] = labels[:, i] .+ 1
+    end
+    l_inp[:graph] = graph
+    l_inp[:n_cluster] = ks
+    l_inp[:ic] = ic[sel]
+    l_inp[:l_df] = l_df
+    l_inp[:cluster_obj] = (gamma = gam[sel], share = share[sel], info = info[])
+    l_inp
+end
+
+# a new handle for one call, destroyed afterwards
+function with_handle(f)
+    hr = Ref{Ptr{Cvoid}}(C_NULL)
+    cfg = Ref(default_config())
+    rc = ccall((:scl_create, LIB), Int32, (Ptr{Ptr{Cvoid}}, Ptr{SclConfig}), hr, cfg)
+    rc == 0 || check(C_NULL, rc)
+    h = hr[]
+    try
+        return f(h)
+    finally
+        ccall((:scl_destroy, LIB), Int32, (Ptr{Cvoid},), h)
+    end
+end
+
+"""
+    leiden(graph, resolutions; n_trials=50, seed=0, max_iterations=10, max_sweeps=64, theta=0.01)
+
+Leiden trials on a symmetric SparseMatrixCSC: labels (N x T x R, ids 1..k by cluster size), cluster counts and
+modularity (T x R each).
+"""
+function leiden(graph::SparseMatrixCSC, resolutions::Vector{Float64}; n_trials=50, seed=0, max_iterations=10, max_sweeps=64,
+                theta=0.01)
+    N = size(graph, 1); R = length(resolutions)
+    rowptr = UInt32.(graph.colptr .- 1); colidx = UInt32.(graph.rowval .- 1); val = Float64.(graph.nzval)
+    p = Ref(SclLeidenParams(n_trials, max_iterations, max_sweeps, 0, theta, UInt64(seed), ntuple(_ -> Int32(0), 4)))
+    labels = Array{Int32}(undef, N, n_trials, R); ncl = Matrix{Int32}(undef, n_trials, R); q = Matrix{Float64}(undef, n_trials, R)
+    info = Ref(SclLeidenInfo())
+    with_handle() do h
+        check(h, ccall((:scl_op_leiden, LIB), Int32,
+                       (Ptr{Cvoid}, Int32, Int64, Ptr{UInt32}, Ptr{UInt32}, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{SclLeidenParams},
+                        Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{SclLeidenInfo}),
+                       h, N, length(val), rowptr, colidx, val, R, resolutions, p, labels, ncl, q, info))
+    end
+    (labels = labels .+ Int32(1), n_clusters = ncl, modularity = q, info = info[])
+end
+
+"""
+    label_ecs(labels)
+
+T x T element-centric similarity of the columns of `labels` (N x T, ids 1..k per column).
+"""
+function label_ecs(labels::Matrix{<:Integer})
+    N, T = size(labels)
+    L = Int32.(labels .- 1)
+    S = Matrix{Float64}(undef, T, T)
+    with_handle() do h
+        check(h, ccall((:scl_op_label_ecs, LIB), Int32, (Ptr{Cvoid}, Int32, Int32, Ptr{Int32}, Ptr{Float64}), h, T, N, L, S))
+    end
+    S
 end
 
 end # module

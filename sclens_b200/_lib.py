@@ -75,6 +75,31 @@ class UmapInfo(C.Structure):
                 ("t_init_ms", C.c_double), ("t_layout_ms", C.c_double), ("reserved", C.c_int32 * 4)]
 
 
+class LeidenParams(C.Structure):
+    _fields_ = [("n_trials", C.c_int32), ("max_iterations", C.c_int32), ("max_sweeps", C.c_int32), ("reserved0", C.c_int32),
+                ("theta", C.c_double), ("seed", C.c_uint64), ("reserved", C.c_int32 * 4)]
+
+
+class LeidenInfo(C.Structure):
+    _fields_ = [("max_levels", C.c_int32), ("max_iterations", C.c_int32), ("capped_levels", C.c_int32),
+                ("weight_shift", C.c_int32), ("copy_levels", C.c_int64), ("t_validate_ms", C.c_double),
+                ("t_move_ms", C.c_double), ("t_refine_ms", C.c_double), ("t_aggregate_ms", C.c_double),
+                ("t_labels_ms", C.c_double), ("reserved", C.c_int32 * 4)]
+
+
+class ClusterParams(C.Structure):
+    _fields_ = [("k_min", C.c_int32), ("k_max", C.c_int32), ("n_trials", C.c_int32), ("max_rounds", C.c_int32),
+                ("n_grid", C.c_int32), ("max_widen", C.c_int32), ("max_iterations", C.c_int32), ("max_sweeps", C.c_int32),
+                ("gamma_lo", C.c_double), ("gamma_hi", C.c_double), ("theta", C.c_double), ("seed", C.c_uint64),
+                ("reserved", C.c_int32 * 4)]
+
+
+class ClusterInfo(C.Structure):
+    _fields_ = [("n_rounds", C.c_int32), ("n_evaluated", C.c_int32), ("n_found", C.c_int32), ("weight_shift", C.c_int32),
+                ("copy_levels", C.c_int64), ("t_validate_ms", C.c_double), ("t_leiden_ms", C.c_double),
+                ("t_ecs_ms", C.c_double), ("t_total_ms", C.c_double), ("reserved", C.c_int32 * 4)]
+
+
 _u32p = C.POINTER(C.c_uint32)
 _f32p = C.POINTER(C.c_float)
 _f64p = C.POINTER(C.c_double)
@@ -151,6 +176,12 @@ SIGNATURES = {
     "scl_get_umap_graph": [_hp, _i64p, _u32p, _u32p, _f32p],
     "scl_get_umap_knn": [_hp, _i32p, _f32p],
     "scl_umap_fit_ab": [C.c_double, C.c_double, _f64p, _f64p],
+    "scl_op_leiden": [_hp, C.c_int32, C.c_int64, _u32p, _u32p, _f64p, C.c_int32, _f64p, C.POINTER(LeidenParams), _i32p,
+                      _i32p, _f64p, C.POINTER(LeidenInfo)],
+    "scl_op_label_ecs": [_hp, C.c_int32, C.c_int32, _i32p, _f64p],
+    "scl_op_cluster": [_hp, C.c_int32, C.c_int64, _u32p, _u32p, _f64p, C.POINTER(ClusterParams), _i32p, _f64p, _f64p, _f64p,
+                       _i32p, C.c_int32, _f64p, _i32p, C.POINTER(ClusterInfo)],
+    "scl_cluster_plan": [C.c_int32, _f64p, _i32p, C.POINTER(ClusterParams), _f64p, _i32p],
     "scl_bench_gram": [_hp, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _f64p, _f64p],
     "scl_bench_syevd": [_hp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _f64p],
     "scl_bench_syevd_concurrent": [_hp, C.c_int32, C.c_int32, C.c_int32, _f64p],

@@ -23,7 +23,8 @@ except ImportError:  # pragma: no cover
     pd = None
 
 from . import _lib
-from ._lib import Config, Profile, RobustInfo, SclError, SignalInfo, UmapInfo, UmapParams, as_f32, as_u32, ptr
+from ._lib import (ClusterInfo, ClusterParams, Config, LeidenInfo, LeidenParams, Profile, RobustInfo, SclError, SignalInfo,
+                   UmapInfo, UmapParams, as_f32, as_u32, ptr)
 
 
 def df2sparr(inp_df):
@@ -305,6 +306,115 @@ class Handle:
         self._ck(self.lib.scl_get_umap_knn(self.h, ptr(idx, C.c_int32), ptr(dist, C.c_float)))
         return idx, dist
 
+    # ---- clustering (scl_op_leiden / scl_op_label_ecs / scl_op_cluster)
+    def leiden(self, graph=None, resolutions=(1.0,), n_trials=50, *, seed=0, max_iterations=10, max_sweeps=64, theta=0.01):
+        """Leiden (modularity with resolution) on a symmetric graph (scipy sparse, N x N; None: the fuzzy graph of the
+        last ``umap``): R x T trials in one batch.  Returns (labels R x T x N int32 with ids by cluster size, descending,
+        n_clusters R x T, modularity R x T, LeidenInfo)."""
+        res = _resolutions(resolutions)
+        p = _leiden_params(n_trials, seed, max_iterations, max_sweeps, theta)
+        N, nnz, rp, ci, v = self._cluster_graph(graph)
+        R, T = len(res), p.n_trials
+        lab = np.empty((R, T, N), np.int32)
+        ncl = np.empty((R, T), np.int32)
+        mod = np.empty((R, T), np.float64)
+        info = LeidenInfo()
+        self._ck(self.lib.scl_op_leiden(self.h, N, nnz, ptr(rp, C.c_uint32), ptr(ci, C.c_uint32), ptr(v, C.c_double), R,
+                                        ptr(res, C.c_double), C.byref(p), ptr(lab, C.c_int32), ptr(ncl, C.c_int32),
+                                        ptr(mod, C.c_double), C.byref(info)))
+        return lab, ncl, mod, info
+
+    def label_ecs(self, labels):
+        """T x T element-centric similarity of T labelings (T x N, any integer ids)."""
+        L = _canonical_ids(labels)
+        T, N = L.shape
+        S = np.empty((T, T), np.float64)
+        self._ck(self.lib.scl_op_label_ecs(self.h, T, N, ptr(L, C.c_int32), ptr(S, C.c_double)))
+        return S
+
+    def cluster(self, graph=None, k_min=2, k_max=20, n_trials=50, *, seed=0, max_rounds=12, n_grid=16, max_widen=4,
+                gamma_lo=0.01, gamma_hi=10.0, max_iterations=10, max_sweeps=64, theta=0.01):
+        """The resolution search: dict k -> {"gamma", "share", "ic", "labels" (N, ids 0..k-1)} for every k found in
+        [k_min, k_max], plus the evaluated (gamma, modal count) pairs and the ClusterInfo."""
+        N, nnz, rp, ci, v = self._cluster_graph(graph)
+        p = _cluster_params(N, k_min, k_max, n_trials, seed, max_rounds, n_grid, max_widen, gamma_lo, gamma_hi,
+                            max_iterations, max_sweeps, theta)
+        nk = p.k_max - p.k_min + 1
+        found = np.empty(nk, np.int32)
+        gam, share, ic = np.empty(nk), np.empty(nk), np.empty(nk)
+        lab = np.empty((nk, N), np.int32)
+        cap = p.n_grid + (p.max_rounds + 1) * (nk + 2)
+        eg, em = np.empty(cap), np.empty(cap, np.int32)
+        info = ClusterInfo()
+        self._ck(self.lib.scl_op_cluster(self.h, N, nnz, ptr(rp, C.c_uint32), ptr(ci, C.c_uint32), ptr(v, C.c_double),
+                                         C.byref(p), ptr(found, C.c_int32), ptr(gam, C.c_double), ptr(share, C.c_double),
+                                         ptr(ic, C.c_double), ptr(lab, C.c_int32), cap, ptr(eg, C.c_double),
+                                         ptr(em, C.c_int32), C.byref(info)))
+        out = {p.k_min + i: {"gamma": gam[i], "share": share[i], "ic": ic[i], "labels": lab[i]}
+               for i in range(nk) if found[i]}
+        ne = min(cap, info.n_evaluated)
+        return out, (eg[:ne].copy(), em[:ne].copy()), info
+
+    def _cluster_graph(self, graph):
+        if graph is None:
+            if not getattr(self, "umap_N", 0):
+                raise ValueError("no graph given and umap has not run on this handle")
+            return self.umap_N, 0, None, None, None
+        return _sym_csr(graph)
+
+
+def _sym_csr(graph):
+    """scipy sparse / dense N x N -> (N, nnz, rowptr u32, col u32, val f64) with sorted columns (checked on the device)."""
+    g = sp.csr_matrix(graph)
+    if g.ndim != 2 or g.shape[0] != g.shape[1] or g.shape[0] < 1:
+        raise ValueError("the graph must be a square N x N matrix")
+    if g.nnz >= 2 ** 32:
+        raise ValueError("the graph has too many entries")
+    if not g.has_sorted_indices:
+        g = g.sorted_indices()
+    return (g.shape[0], g.nnz, as_u32(g.indptr), np.ascontiguousarray(g.indices, dtype=np.uint32),
+            np.ascontiguousarray(g.data, dtype=np.float64))
+
+
+def _resolutions(resolutions):
+    r = np.ascontiguousarray(np.atleast_1d(np.asarray(resolutions, dtype=np.float64)))
+    if r.ndim != 1 or len(r) < 1 or not np.isfinite(r).all() or (r <= 0).any():
+        raise ValueError("resolutions must be a non-empty list of positive numbers")
+    return r
+
+
+def _leiden_params(n_trials, seed, max_iterations, max_sweeps, theta):
+    if int(n_trials) < 1 or int(max_iterations) < 1 or int(max_sweeps) < 1:
+        raise ValueError("n_trials, max_iterations and max_sweeps must be >= 1")
+    if not (math.isfinite(float(theta)) and float(theta) > 0):
+        raise ValueError("theta must be positive")
+    return LeidenParams(n_trials=int(n_trials), max_iterations=int(max_iterations), max_sweeps=int(max_sweeps),
+                        theta=float(theta), seed=int(seed) & (2 ** 64 - 1))
+
+
+def _cluster_params(N, k_min, k_max, n_trials, seed, max_rounds, n_grid, max_widen, gamma_lo, gamma_hi, max_iterations,
+                    max_sweeps, theta):
+    k_min, k_max = int(k_min), int(k_max)
+    if not (1 <= k_min <= k_max <= N):
+        raise ValueError(f"need 1 <= k_min <= k_max <= N (k_min = {k_min}, k_max = {k_max}, N = {N})")
+    if int(n_trials) < 2 or int(max_rounds) < 0 or int(n_grid) < 2 or not (0 <= int(max_widen) <= 30):
+        raise ValueError("need n_trials >= 2, max_rounds >= 0, n_grid >= 2 and 0 <= max_widen <= 30")
+    lo, hi = float(gamma_lo), float(gamma_hi)
+    if not (math.isfinite(lo) and math.isfinite(hi) and 0 < lo < hi):
+        raise ValueError("need 0 < gamma_lo < gamma_hi")
+    lp = _leiden_params(n_trials, seed, max_iterations, max_sweeps, theta)
+    return ClusterParams(k_min=k_min, k_max=k_max, n_trials=lp.n_trials, max_rounds=int(max_rounds), n_grid=int(n_grid),
+                         max_widen=int(max_widen), max_iterations=lp.max_iterations, max_sweeps=lp.max_sweeps,
+                         gamma_lo=lo, gamma_hi=hi, theta=lp.theta, seed=lp.seed)
+
+
+def _canonical_ids(labels):
+    """T x N labelings with any integer ids -> ids 0..k-1 per row (int32), as scl_op_label_ecs takes them."""
+    L = np.asarray(labels)
+    if L.ndim != 2 or L.shape[0] < 1 or L.shape[1] < 1 or not np.issubdtype(L.dtype, np.integer):
+        raise ValueError("labels must be a T x N integer array")
+    return np.ascontiguousarray(np.stack([np.unique(row, return_inverse=True)[1].ravel() for row in L]).astype(np.int32))
+
 
 _UMAP_METRICS = {"euclidean": 0, "cosine": 1}
 _UMAP_INITS = {"spectral": 0, "random": 1}
@@ -581,14 +691,8 @@ def get_denoised_df(inp_obj, device_="gpu", *, device=0, handle=None, dtype=np.f
     return odf
 
 
-def apply_umap(res, k=15, nc=2, md=0.1, metric="cosine", *, n_epochs=300, seed=0, init="spectral", device=0, handle=None,
-               spread=1.0, learning_rate=1.0, repulsion_strength=1.0, neg_sample_rate=5, local_connectivity=1.0,
-               spectral_maxiter=100):
-    """Drop-in for scLENS.apply_umap! (:863-873): UMAP of the robust signals on the device.  Reads ``res["pca_n1"]``
-    when it exists and has at least one column, otherwise ``res["pca"]`` (N x r, DataFrame with a leading "cell" column
-    or array).  Stores ``res["umap"]`` (N x nc, rows in ``cell_id`` order) and ``res["umap_obj"]`` = {"graph": the
-    symmetric fuzzy graph as scipy CSR, "knns", "dists": N x k (0-based), "a", "b", "info"} and returns ``res``.
-    Exact kNN (no NN-descent) and a synchronous, deterministic epoch: the same seed gives the same embedding."""
+def _signals(res):
+    """The matrix apply_umap embeds: res["pca_n1"] when it has a column besides "cell", else res["pca"]."""
     def signals(key):
         m = res.get(key)
         if pd is not None and isinstance(m, pd.DataFrame) and "cell" in m.columns:
@@ -600,7 +704,18 @@ def apply_umap(res, k=15, nc=2, md=0.1, metric="cosine", *, n_epochs=300, seed=0
         src = signals("pca")
     if src is None:
         raise ValueError("the result has neither a non-empty 'pca_n1' nor a 'pca' entry")
-    X = _umap_matrix(src)
+    return src
+
+
+def apply_umap(res, k=15, nc=2, md=0.1, metric="cosine", *, n_epochs=300, seed=0, init="spectral", device=0, handle=None,
+               spread=1.0, learning_rate=1.0, repulsion_strength=1.0, neg_sample_rate=5, local_connectivity=1.0,
+               spectral_maxiter=100):
+    """Drop-in for scLENS.apply_umap! (:863-873): UMAP of the robust signals on the device.  Reads ``res["pca_n1"]``
+    when it exists and has at least one column, otherwise ``res["pca"]`` (N x r, DataFrame with a leading "cell" column
+    or array).  Stores ``res["umap"]`` (N x nc, rows in ``cell_id`` order) and ``res["umap_obj"]`` = {"graph": the
+    symmetric fuzzy graph as scipy CSR, "knns", "dists": N x k (0-based), "a", "b", "info"} and returns ``res``.
+    Exact kNN (no NN-descent) and a synchronous, deterministic epoch: the same seed gives the same embedding."""
+    X = _umap_matrix(_signals(res))
     N = X.shape[1]
     _umap_params(N, k, nc, md, metric, n_epochs, seed, init, spread, learning_rate, repulsion_strength, neg_sample_rate,
                  local_connectivity, spectral_maxiter)    # every argument checked before a device is touched
@@ -622,4 +737,56 @@ def apply_umap(res, k=15, nc=2, md=0.1, metric="cosine", *, n_epochs=300, seed=0
                                 "init_fallback": info.init_fallback,
                                 "timings_ms": {"knn": info.t_knn_ms, "graph": info.t_graph_ms, "init": info.t_init_ms,
                                                "layout": info.t_layout_ms}}}
+    return res
+
+
+def clustering(res, k_min=2, k_max=20, n_trials=50, seed=0, *, max_rounds=12, n_grid=16, max_widen=4, gamma_lo=0.01,
+               gamma_hi=10.0, max_iterations=10, max_sweeps=64, theta=0.01, device=0, handle=None, k=15, metric="cosine"):
+    """scICE-style clustering of an ``apply_umap``/``sclens`` result on the device.  Takes the cell graph from
+    ``res["umap_obj"]["graph"]``; without it, builds the same fuzzy graph from the signals ``apply_umap`` reads (``k``,
+    ``metric``).  Runs ``n_trials`` Leiden trials per resolution, searches the resolutions for every cluster count in
+    [k_min, k_max] and stores ``res["graph"]``, ``res["n_cluster"]`` (the counts found), ``res["ic"]`` (their
+    inconsistency coefficients, aligned with ``n_cluster``), ``res["l_df"]`` (DataFrame: "cell" plus one column "k_<k>"
+    per found count, labels 1..k by cluster size) and ``res["cluster_obj"]`` (gamma, share, evaluated resolutions, info,
+    timings).  Returns ``res``.  The same seed gives the same labels."""
+    graph = (res.get("umap_obj") or {}).get("graph")
+    if graph is not None:
+        graph = sp.csr_matrix(graph)
+        N = graph.shape[0]
+    else:
+        X = _umap_matrix(_signals(res))
+        N = X.shape[1]
+        _umap_params(N, k, 2, 0.1, metric, 0, seed, "random", 1.0, 1.0, 1.0, 5, 1.0, 100)
+    p = _cluster_params(N, k_min, k_max, n_trials, seed, max_rounds, n_grid, max_widen, gamma_lo, gamma_hi,
+                        max_iterations, max_sweeps, theta)      # every argument checked before a device is touched
+    own = handle is None
+    h = Handle(device=device) if own else handle
+    try:
+        if graph is None:
+            h.umap(X.T, k, 2, metric=metric, n_epochs=0, init="random", seed=seed)
+            graph = h.umap_graph()
+        found, (eg, em), info = h.cluster(graph, p.k_min, p.k_max, p.n_trials, seed=p.seed, max_rounds=p.max_rounds,
+                                          n_grid=p.n_grid, max_widen=p.max_widen, gamma_lo=p.gamma_lo,
+                                          gamma_hi=p.gamma_hi, max_iterations=p.max_iterations,
+                                          max_sweeps=p.max_sweeps, theta=p.theta)
+    finally:
+        if own:
+            h.close()
+    ks = sorted(found)
+    cells = res.get("cell_id")
+    cells = np.asarray(cells) if cells is not None and len(cells) == N else np.array([f"c{i}" for i in range(N)], dtype=object)
+    cols = {"cell": cells}
+    for kk in ks:
+        cols[f"k_{kk}"] = found[kk]["labels"].astype(np.int64) + 1
+    res["graph"] = graph
+    res["n_cluster"] = np.asarray(ks, dtype=np.int64)
+    res["ic"] = np.asarray([found[kk]["ic"] for kk in ks], dtype=np.float64)
+    res["l_df"] = pd.DataFrame(cols) if pd is not None else cols
+    res["cluster_obj"] = {"gamma": np.asarray([found[kk]["gamma"] for kk in ks]),
+                          "share": np.asarray([found[kk]["share"] for kk in ks]),
+                          "evaluated_gamma": eg, "evaluated_mode": em,
+                          "info": {"n_rounds": info.n_rounds, "n_evaluated": info.n_evaluated, "n_found": info.n_found,
+                                   "weight_shift": info.weight_shift, "copy_levels": info.copy_levels,
+                                   "timings_ms": {"validate": info.t_validate_ms, "leiden": info.t_leiden_ms,
+                                                  "ecs": info.t_ecs_ms, "total": info.t_total_ms}}}
     return res

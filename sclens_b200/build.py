@@ -9,7 +9,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsclens_b200.so")
-SOURCES = ["sparse.cu", "normalize.cu", "gemm_umma.cu", "eigen.cu", "tridiag.cu", "sytrd.cu", "sy2sb.cu", "sb2st.cu", "backtrans.cu", "refine.cu", "subspace.cu", "pipeline.cu", "denoise.cu", "preprocess.cu", "umap.cu", "capi.cu"]
+SOURCES = ["sparse.cu", "normalize.cu", "gemm_umma.cu", "eigen.cu", "tridiag.cu", "sytrd.cu", "sy2sb.cu", "sb2st.cu", "backtrans.cu", "refine.cu", "subspace.cu", "pipeline.cu", "denoise.cu", "preprocess.cu", "umap.cu", "leiden.cu", "capi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-diag-suppress", "177"]

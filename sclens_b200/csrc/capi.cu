@@ -1,10 +1,13 @@
 // extern "C" surface of libsclens_b200.so (see include/sclens_b200.h).
 #include "nccl_dyn.h"
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstring>
+#include <map>
 #include <thread>
 #include "handle.h"
+#include "leiden.h"
 #include "tmp.cuh"
 #include "twostage.h"
 
@@ -1063,6 +1066,192 @@ int32_t scl_get_umap_knn(scl_handle* h, int32_t* idx, float* dist) {
 int32_t scl_umap_fit_ab(double min_dist, double spread, double* a, double* b) {
   if (!a || !b || !std::isfinite(min_dist) || !(min_dist >= 0) || !std::isfinite(spread) || !(spread > 0)) return SCL_ERR_INVALID;
   return guard(nullptr, [&] { umap_fit_ab(min_dist, spread, a, b); });
+}
+
+
+// ---- clustering (scICE clustering!) ----------------------------------------------------------------------------------
+namespace {
+// the caller's graph (rowptr != NULL) or the handle's fuzzy graph, validated and in fixed point
+void cluster_graph(scl_handle* h, int32_t N, int64_t nnz, const uint32_t* rowptr, const uint32_t* colidx, const double* val,
+                   FixGraph& g) {
+  if (!rowptr) {
+    SCL_REQUIRE(h->have_umap_graph, "no graph given and scl_op_umap has not completed");
+    SCL_REQUIRE(N == h->ug_N, "N differs from the handle's graph");
+    leiden_prepare(h->ug_rowptr.p, h->ug_col.p, nullptr, h->ug_val.p, N, h->ug_nnz, g, h->st);
+    return;
+  }
+  SCL_REQUIRE(N >= 1 && nnz >= 0 && nnz < (int64_t)1 << 32, "need N >= 1 and 0 <= nnz < 2^32");
+  SCL_REQUIRE(nnz == 0 || (colidx && val), "colidx / val are NULL");
+  Tmp<uint32_t> rp(N + 1, h->st), ci(std::max<int64_t>(nnz, 1), h->st);
+  Tmp<double> v(std::max<int64_t>(nnz, 1), h->st);
+  SCL_CUDA(cudaMemcpyAsync(rp.p, rowptr, (N + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, h->st));
+  if (nnz) {
+    SCL_CUDA(cudaMemcpyAsync(ci.p, colidx, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice, h->st));
+    SCL_CUDA(cudaMemcpyAsync(v.p, val, nnz * sizeof(double), cudaMemcpyHostToDevice, h->st));
+  }
+  leiden_prepare(rp.p, ci.p, v.p, nullptr, N, (size_t)nnz, g, h->st);
+}
+
+double ms_since(std::chrono::steady_clock::time_point t) {
+  return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count();
+}
+
+bool cluster_params_ok(const scl_cluster_params& q) {
+  return q.k_min >= 1 && q.k_max >= q.k_min && q.n_trials >= 2 && q.max_rounds >= 0 && q.n_grid >= 2 && q.max_widen >= 0 &&
+         q.max_widen <= 30 && q.max_iterations >= 1 && q.max_sweeps >= 1 && std::isfinite(q.gamma_lo) && q.gamma_lo > 0 &&
+         std::isfinite(q.gamma_hi) && q.gamma_hi > q.gamma_lo && std::isfinite(q.theta) && q.theta > 0;
+}
+}  // namespace
+
+int32_t scl_op_leiden(scl_handle* h, int32_t N, int64_t nnz, const uint32_t* rowptr, const uint32_t* colidx, const double* val,
+                      int32_t R, const double* resolutions, const scl_leiden_params* p, int32_t* labels, int32_t* n_clusters,
+                      double* modularity, scl_leiden_info* info) {
+  if (!h || !p || !resolutions || !labels || !n_clusters || !modularity || !info) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    const scl_leiden_params& q = *p;
+    SCL_REQUIRE(R >= 1 && q.n_trials >= 1 && q.max_iterations >= 1 && q.max_sweeps >= 1, "bad R / n_trials / max_iterations / max_sweeps");
+    SCL_REQUIRE(std::isfinite(q.theta) && q.theta > 0, "theta must be positive");
+    for (int r = 0; r < R; ++r) SCL_REQUIRE(std::isfinite(resolutions[r]) && resolutions[r] > 0, "resolutions must be positive");
+    SCL_REQUIRE(N >= 1, "N must be positive");
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    *info = scl_leiden_info{};
+    const auto t0 = std::chrono::steady_clock::now();
+    FixGraph g;
+    cluster_graph(h, N, nnz, rowptr, colidx, val, g);
+    info->t_validate_ms = ms_since(t0);
+    info->weight_shift = g.shift;
+    LeidenStats s;
+    leiden_batched(g, resolutions, R, q.n_trials, q.seed, q.max_iterations, q.max_sweeps, q.theta, labels, n_clusters, modularity,
+               &s, h->st);
+    info->max_levels = s.max_levels;
+    info->max_iterations = s.max_iterations;
+    info->capped_levels = s.capped_levels;
+    info->copy_levels = s.copy_levels;
+    info->t_move_ms = s.t_move_ms;
+    info->t_refine_ms = s.t_refine_ms;
+    info->t_aggregate_ms = s.t_aggregate_ms;
+    info->t_labels_ms = s.t_labels_ms;
+  });
+}
+
+int32_t scl_op_label_ecs(scl_handle* h, int32_t T, int32_t N, const int32_t* labels, double* ecs) {
+  if (!h || !labels || !ecs || T < 1 || N < 1) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    label_ecs(labels, T, N, ecs, h->st);
+  });
+}
+
+int32_t scl_cluster_plan(int32_t n, const double* gammas, const int32_t* modes, const scl_cluster_params* p, double* out,
+                         int32_t* n_out) {
+  if (!p || !out || !n_out || n < 0 || (n > 0 && (!gammas || !modes)) || !cluster_params_ok(*p)) return SCL_ERR_INVALID;
+  return guard(nullptr, [&] {
+    std::vector<double> g(gammas, gammas + n);
+    std::vector<int> m(modes, modes + n);
+    for (double x : g) SCL_REQUIRE(std::isfinite(x) && x > 0, "gammas must be positive");
+    const double lo = p->gamma_lo * std::pow(10.0, -p->max_widen), hi = p->gamma_hi * std::pow(10.0, p->max_widen);
+    const std::vector<double> nx = cluster_plan(g, m, p->k_min, p->k_max, lo, hi);
+    std::copy(nx.begin(), nx.end(), out);
+    *n_out = (int32_t)nx.size();
+  });
+}
+
+int32_t scl_op_cluster(scl_handle* h, int32_t N, int64_t nnz, const uint32_t* rowptr, const uint32_t* colidx, const double* val,
+                       const scl_cluster_params* p, int32_t* found, double* gamma, double* share, double* ic, int32_t* labels,
+                       int32_t eval_cap, double* eval_gamma, int32_t* eval_mode, scl_cluster_info* info) {
+  if (!h || !p || !found || !gamma || !share || !ic || !labels || !info || eval_cap < 0) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    const scl_cluster_params& q = *p;
+    SCL_REQUIRE(cluster_params_ok(q), "bad clustering parameters");
+    SCL_REQUIRE(N >= 1 && q.k_max <= N, "need k_max <= N");
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    *info = scl_cluster_info{};
+    const auto t0 = std::chrono::steady_clock::now();
+    FixGraph g;
+    cluster_graph(h, N, nnz, rowptr, colidx, val, g);
+    info->t_validate_ms = ms_since(t0);
+    info->weight_shift = g.shift;
+    const int nk = q.k_max - q.k_min + 1, T = q.n_trials;
+    std::vector<double> best_share(nk, 0.0), best_gamma(nk, 0.0);
+    std::vector<std::vector<int32_t>> best_lab(nk);
+    std::vector<double> eg;
+    std::vector<int> em;
+    std::vector<double> gs(q.n_grid);
+    const double l0 = std::log(q.gamma_lo), l1 = std::log(q.gamma_hi);
+    for (int i = 0; i < q.n_grid; ++i) gs[i] = std::exp(l0 + i * ((l1 - l0) / (q.n_grid - 1)));
+    const double lo_lim = q.gamma_lo * std::pow(10.0, -q.max_widen), hi_lim = q.gamma_hi * std::pow(10.0, q.max_widen);
+    std::vector<int32_t> lab, ncl;
+    std::vector<double> mod;
+    for (int round = 0;; ++round) {
+      const int R = (int)gs.size();
+      lab.resize((size_t)R * T * N);
+      ncl.resize((size_t)R * T);
+      mod.resize((size_t)R * T);
+      const auto tl = std::chrono::steady_clock::now();
+      LeidenStats s;
+      leiden_batched(g, gs.data(), R, T, q.seed, q.max_iterations, q.max_sweeps, q.theta, lab.data(), ncl.data(), mod.data(), &s,
+                 h->st);
+      info->t_leiden_ms += ms_since(tl);
+      info->copy_levels += s.copy_levels;
+      info->n_rounds = round + 1;
+      for (int r = 0; r < R; ++r) {
+        std::map<int, int> cnt;
+        for (int t = 0; t < T; ++t) ++cnt[ncl[(size_t)r * T + t]];
+        int mode = 0, mc = 0;
+        for (auto& kv : cnt) if (kv.second > mc) { mc = kv.second; mode = kv.first; }   // ties: the smaller count
+        eg.push_back(gs[r]);
+        em.push_back(mode);
+        for (int i = 0; i < nk; ++i) {
+          auto it = cnt.find(q.k_min + i);
+          if (it == cnt.end()) continue;
+          const double sh = (double)it->second / T;
+          if (sh > best_share[i] || (sh == best_share[i] && gs[r] < best_gamma[i])) {
+            best_share[i] = sh;
+            best_gamma[i] = gs[r];
+            best_lab[i].assign(lab.begin() + (size_t)r * T * N, lab.begin() + (size_t)(r + 1) * T * N);
+          }
+        }
+      }
+      if (round >= q.max_rounds) break;
+      gs = cluster_plan(eg, em, q.k_min, q.k_max, lo_lim, hi_lim);
+      if (gs.empty()) break;
+    }
+    info->n_evaluated = (int32_t)eg.size();
+    for (int i = 0; i < std::min<int>(eval_cap, (int)eg.size()); ++i) {
+      if (eval_gamma) eval_gamma[i] = eg[i];
+      if (eval_mode) eval_mode[i] = em[i];
+    }
+    const auto te = std::chrono::steady_clock::now();
+    std::vector<double> S((size_t)T * T);
+    for (int i = 0; i < nk; ++i) {
+      const bool f = std::find(em.begin(), em.end(), q.k_min + i) != em.end();
+      found[i] = f;
+      int32_t* out = labels + (size_t)i * N;
+      if (!f) {
+        gamma[i] = share[i] = ic[i] = NAN;
+        std::fill(out, out + N, -1);
+        continue;
+      }
+      ++info->n_found;
+      gamma[i] = best_gamma[i];
+      share[i] = best_share[i];
+      label_ecs(best_lab[i].data(), T, N, S.data(), h->st);
+      double tot = 0, best_row = -1;
+      int rep = 0;
+      for (int a = 0; a < T; ++a) {
+        double row = 0;
+        for (int b = 0; b < T; ++b) row += S[(size_t)a * T + b];
+        tot += row;
+        const int32_t* la = best_lab[i].data() + (size_t)a * N;
+        const bool has_k = *std::max_element(la, la + N) + 1 == q.k_min + i;   // ids 0..k-1
+        if (has_k && row > best_row) { best_row = row; rep = a; }
+      }
+      ic[i] = (double)T * T / tot;
+      std::copy(best_lab[i].begin() + (size_t)rep * N, best_lab[i].begin() + (size_t)(rep + 1) * N, out);
+    }
+    info->t_ecs_ms = ms_since(te);
+    info->t_total_ms = ms_since(t0);
+  });
 }
 
 }  // extern "C"
