@@ -426,6 +426,17 @@ SCL_API int32_t scl_debug_eig_stage_totals(scl_handle* h, double out[8]);
  * pointer may be NULL.  flags[0] = panel failure flag, flags[1] = number of panels. */
 SCL_API int32_t scl_debug_two_stage(scl_handle* h, int32_t n, const float* A, float* AB, float* d, float* e, float* Q2, float* Q,
                                     int32_t flags[2]);
+/* The Float64 Rayleigh-Ritz refinement of the eigenvalues on its own, as the pipeline runs it after an eigensolve: G (n x n,
+ * symmetric) and V (n x n, the eigenvectors as rows, any scaling, ascending order), n >= 2.  L (n) = the refined eigenvalues,
+ * ascending; stats (may be NULL): stats[0] = number of clusters solved as Rayleigh-Ritz blocks, stats[1] = size of the largest
+ * (1 when there is none). */
+SCL_API int32_t scl_debug_refine(scl_handle* h, int32_t n, const float* G, const float* V, float* L, int32_t stats[2]);
+/* The Gram matrix with the exact diagonal and the tensor-core bias calibration, as the pipeline forms it: the syrk of scl_op_gram
+ * (operand layout and scale as there; the handle's cta_group and gram_chunk_kb), the calibration samples, the diagonal set to
+ * scale * diag (diag: rows Float64 sums of squares), the fitted factor and the diagonal scaled by it.  Calibrates at every
+ * rows >= 2 (the pipeline from 64 on).  G (rows x rows) = the result; factor (may be NULL) = the common factor 1 - delta. */
+SCL_API int32_t scl_debug_gram_calibrated(scl_handle* h, int32_t rows, int64_t K, int64_t ld, const uint16_t* a_hi, const uint16_t* a_lo,
+                                          float scale, const double* diag, float* G, double* factor);
 /* Tuning studies only (process-wide).  stat_variant: launch shape of the statistics passes (0-7: line passes,
  * 8: strip passes; < 0 keeps the current one).  stat_heavy: line length above which a whole CTA takes a line
  * (<= 0 keeps).  writer: dense writer, -1 automatic, 0 register/overlay writer, 1 TMA bulk-store writer, 2 / 3

@@ -742,6 +742,52 @@ int32_t scl_debug_two_stage(scl_handle* h, int32_t n, const float* A, float* AB,
   });
 }
 
+int32_t scl_debug_refine(scl_handle* h, int32_t n, const float* G, const float* V, float* L, int32_t* stats) {
+  if (!h || !G || !V || !L || n < 2) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    const size_t nn = (size_t)n * n;
+    Tmp<float> dG(nn, h->st), dV(nn, h->st), dW(n, h->st);
+    SCL_CUDA(cudaMemcpyAsync(dG.p, G, nn * sizeof(float), cudaMemcpyHostToDevice, h->st));
+    SCL_CUDA(cudaMemcpyAsync(dV.p, V, nn * sizeof(float), cudaMemcpyHostToDevice, h->st));
+    int st[2] = {0, 0};
+    refine_eigenvalues(dG.p, dV.p, n, dW.p, h->st, st);
+    SCL_CUDA(cudaMemcpyAsync(L, dW.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaStreamSynchronize(h->st));
+    if (stats) { stats[0] = st[0]; stats[1] = st[1]; }
+  });
+}
+
+int32_t scl_debug_gram_calibrated(scl_handle* h, int32_t rows, int64_t K, int64_t ld, const uint16_t* a_hi, const uint16_t* a_lo,
+                                  float scale, const double* diag, float* G, double* factor) {
+  if (!h || !a_hi || !diag || !G || rows < 2 || K < 1 || ld < K || (ld & 7)) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    const size_t n = (size_t)rows * (size_t)ld;
+    Tmp<__half> hi(n, h->st), lo(a_lo ? n : 1, h->st);
+    Tmp<float> g((size_t)rows * rows, h->st);
+    Tmp<double> d(rows, h->st), ex(kCalibSamples, h->st), f(1, h->st);
+    SCL_CUDA(cudaMemcpyAsync(hi.p, a_hi, n * 2, cudaMemcpyHostToDevice, h->st));
+    if (a_lo) SCL_CUDA(cudaMemcpyAsync(lo.p, a_lo, n * 2, cudaMemcpyHostToDevice, h->st));
+    SCL_CUDA(cudaMemcpyAsync(d.p, diag, (size_t)rows * sizeof(double), cudaMemcpyHostToDevice, h->st));
+    GemmArgs a;
+    a.A.hi = hi.p; a.A.lo = a_lo ? lo.p : nullptr; a.A.rows = rows; a.A.K = K; a.A.ld = ld;
+    a.B = a.A;
+    a.syrk = true; a.alpha = scale; a.C = g.p; a.ldc = rows;
+    a.cta_group = h->cfg.cta_group == 1 ? 1 : 2;
+    a.chunk_kb = h->cfg.gram_chunk_kb;
+    gemm_umma(a, h->st);
+    // the order of gram_of(): samples, exact diagonal, fit, diagonal scale
+    calib_sample_dots(hi.p, a_lo ? lo.p : nullptr, (long long)ld, 0, (long long)K, rows, ex.p, h->st);
+    set_gram_diagonal(g.p, rows, d.p, (double)scale, h->st);
+    calib_fit(g.p, rows, scale, ex.p, f.p, h->st);
+    calib_scale_diagonal(g.p, rows, f.p, h->st);
+    SCL_CUDA(cudaMemcpyAsync(G, g.p, (size_t)rows * rows * sizeof(float), cudaMemcpyDeviceToHost, h->st));
+    if (factor) SCL_CUDA(cudaMemcpyAsync(factor, f.p, sizeof(double), cudaMemcpyDeviceToHost, h->st));
+    SCL_CUDA(cudaStreamSynchronize(h->st));
+  });
+}
+
 int32_t scl_debug_set_tuning(int32_t stat_variant, int32_t stat_heavy, int32_t writer) {
   scl::set_norm_tuning(stat_variant, stat_heavy, writer);
   return SCL_OK;

@@ -73,8 +73,8 @@ struct scl_handle {
 };
 
 namespace scl {
-// refine.cu
-void refine_eigenvalues(const float* dG, const float* dV, int n, float* dW, cudaStream_t st);
+// refine.cu.  stats (optional): [0] clusters solved as Rayleigh-Ritz blocks, [1] size of the largest
+void refine_eigenvalues(const float* dG, const float* dV, int n, float* dW, cudaStream_t st, int* stats = nullptr);
 // pipeline.cu
 void run_signal(scl_handle* h);
 void run_robustness(scl_handle* h, double th, double p_step, int n_perturb);
@@ -100,6 +100,14 @@ bool preprocess_device(const SpMat& X, const uint8_t* d_gene_flags, const scl_qc
 // partial Gram matrices are summed with ncclAllReduce
 void gram_of(scl_handle* h, const SpMat& A, NormStats& S, DBuf<__half>& hi, DBuf<__half>& lo, float* dG, int nm,
              float scale, bool split, bool shard = false, int reduce_root = -1);
+// the tensor-core bias calibration of gram_of(), step by step (pipeline.cu): exact dot products of kCalibSamples
+// off-diagonal pairs of the operand rows, the fitted common factor (1 - delta) clamped to 1 outside (0.999, 1.001), and the
+// diagonal scaled by it
+constexpr int kCalibSamples = 2048;
+void calib_sample_dots(const __half* hi, const __half* lo, long long ld, long long k0, long long Ks, int rows, double* ex,
+                       cudaStream_t st);
+void calib_fit(const float* G, int n, float scale, const double* ex, double* factor, cudaStream_t st);
+void calib_scale_diagonal(float* G, int n, const double* factor, cudaStream_t st);
 void corr_colabsmax(scl_handle* h, const float* dV, int nv, const float* dW, int nw, int n, float* d_out);
 void topk_subspace(scl_handle* h, const float* dG, int n, int k, float* dL, float* dV, int* iters);
 void score_sets(scl_handle* h, int N, int k, int min_pc, int n_perturb, const float* d_nV, const float* d_sets,

@@ -161,7 +161,7 @@ void gemm_splitk(scl_handle* h, const GemmOperand& A, const GemmOperand& B, bool
 // times delta at the lower Marchenko-Pastur edge.  delta is measured per Gram matrix from kCalibSamples
 // off-diagonal entries evaluated exactly (Float64 dot products of the binary16 operand rows); the diagonal is
 // scaled by (1 - delta) so the whole matrix carries one common factor, which is divided out of the eigenvalues.
-constexpr int kCalibSamples = 2048;
+// (kCalibSamples: handle.h)
 
 __device__ __forceinline__ void calib_pair(int s, int rows, int& i, int& j) {
   uint64_t h = (uint64_t)(s + 1) * 0x9E3779B97F4A7C15ull;
@@ -289,6 +289,27 @@ double quantile7(const std::vector<double>& sorted, double p) {
 
 }  // namespace
 
+// The three calibration steps of gram_of(), shared with scl_debug_gram_calibrated.
+// ex[s] = exact dot product of sample pair s over the operand columns [k0, k0 + Ks) (hi, plus the cross terms with lo)
+void calib_sample_dots(const __half* hi, const __half* lo, long long ld, long long k0, long long Ks, int rows, double* ex,
+                       cudaStream_t st) {
+  count_launches(1);
+  k_sample_dots<<<kCalibSamples, 256, 0, st>>>(hi, lo, ld, k0, Ks, rows, ex);
+  SCL_CUDA(cudaGetLastError());
+}
+// factor[0] = 1 - delta from the samples of G (= scale * operand operand'), 1 when the fit falls outside (0.999, 1.001)
+void calib_fit(const float* G, int n, float scale, const double* ex, double* factor, cudaStream_t st) {
+  count_launches(1);
+  k_fit_shrink<<<1, 256, 0, st>>>(G, n, 1.0 / (double)scale, ex, kCalibSamples, factor);
+  SCL_CUDA(cudaGetLastError());
+}
+// G[i][i] *= factor[0]: the exact diagonal takes the common factor of the tensor-core off-diagonal
+void calib_scale_diagonal(float* G, int n, const double* factor, cudaStream_t st) {
+  count_launches(1);
+  k_scale_diagonal<<<(n + 255) / 256, 256, 0, st>>>(G, n, factor);
+  SCL_CUDA(cudaGetLastError());
+}
+
 // Contraction-axis block of rank `rank`: whole 64-element k-blocks, ceil(kblocks / world) per rank, the last rank also
 // takes the zero padding up to ld.  Blocks are disjoint and cover [0, ld); a rank beyond the data gets an empty block.
 void plan_gram_shard(int64_t K, int64_t ld, int world, int rank, int64_t* k0, int64_t* k1) {
@@ -359,14 +380,11 @@ void gram_of(scl_handle* h, const SpMat& A, NormStats& S, DBuf<__half>& hi, DBuf
   h->gram_factor.ensure(4);
   if (calibrate) {
     ProfScope ps(&h->prof, h->st, PK_SMALL);
-    count_launches(1);
     if (have_work)
-      k_sample_dots<<<kCalibSamples, 256, 0, h->st>>>(hi.p, split ? lo.p : nullptr, (long long)lds,
-                                                      (long long)(sharded ? 0 : k0),
-                                                      (long long)(std::min<int64_t>(K, k1) - k0), rows, ex.p);
+      calib_sample_dots(hi.p, split ? lo.p : nullptr, (long long)lds, (long long)(sharded ? 0 : k0),
+                        (long long)(std::min<int64_t>(K, k1) - k0), rows, ex.p, h->st);
     else
       SCL_CUDA(cudaMemsetAsync(ex.p, 0, kCalibSamples * sizeof(double), h->st));
-    SCL_CUDA(cudaGetLastError());
   }
   if (sharded) {
     // packed lower triangle, summed in FP32 (rank order fixed by NCCL's algorithm choice for a given world size); to the
@@ -396,10 +414,8 @@ void gram_of(scl_handle* h, const SpMat& A, NormStats& S, DBuf<__half>& hi, DBuf
   }
   if (calibrate) {
     ProfScope ps(&h->prof, h->st, PK_SMALL);
-    count_launches(2);
-    k_fit_shrink<<<1, 256, 0, h->st>>>(dG, nm, 1.0 / (double)scale, ex.p, kCalibSamples, h->gram_factor.p);
-    k_scale_diagonal<<<(nm + 255) / 256, 256, 0, h->st>>>(dG, nm, h->gram_factor.p);
-    SCL_CUDA(cudaGetLastError());
+    calib_fit(dG, nm, scale, ex.p, h->gram_factor.p, h->st);
+    calib_scale_diagonal(dG, nm, h->gram_factor.p, h->st);
   } else {
     const double one = 1.0;
     SCL_CUDA(cudaMemcpyAsync(h->gram_factor.p, &one, sizeof(double), cudaMemcpyHostToDevice, h->st));

@@ -189,8 +189,9 @@ void jacobi_eigenvalues(std::vector<double>& a, int m, std::vector<double>& ev) 
 }  // namespace
 
 // dV: eigenvectors as rows of memory (cuSOLVER's column-major result), dG: the matrix they belong to (symmetric).
-// dW (ascending FP32 eigenvalues) is overwritten by the refined eigenvalues, ascending.
-void refine_eigenvalues(const float* dG, const float* dV, int n, float* dW, cudaStream_t st) {
+// dW (ascending FP32 eigenvalues) is overwritten by the refined eigenvalues, ascending.  stats (optional): [0] number of
+// clusters solved as Rayleigh-Ritz blocks, [1] size of the largest (1 when there is none).
+void refine_eigenvalues(const float* dG, const float* dV, int n, float* dW, cudaStream_t st, int* stats) {
   const int n_tiles = (n + kTile - 1) / kTile;
   const int nb = kBand + 1;
   Tmp<double> part((size_t)n * n_tiles * nb, st), vv(n, st), dHb((size_t)n * nb, st);
@@ -242,6 +243,7 @@ void refine_eigenvalues(const float* dG, const float* dV, int n, float* dW, cuda
     fprintf(stderr, "[scl] refine: n=%d, %d clusters (largest %d); H_00 %.6g H_11 %.6g H_22 %.6g H_01 %.3g H_12 %.3g; vv0 %.9g\n", n,
             n_clusters, max_cluster, H(0, 0), H(1, 1), H(2, 2), H(0, 1), H(1, 2), 0.0);
   }
+  if (stats) { stats[0] = n_clusters; stats[1] = max_cluster; }
   std::sort(out.begin(), out.end());
   std::vector<float> outf(n);
   for (int q = 0; q < n; ++q) outf[q] = (float)out[q];
