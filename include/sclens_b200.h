@@ -437,11 +437,26 @@ SCL_API int32_t scl_debug_refine(scl_handle* h, int32_t n, const float* G, const
  * rows >= 2 (the pipeline from 64 on).  G (rows x rows) = the result; factor (may be NULL) = the common factor 1 - delta. */
 SCL_API int32_t scl_debug_gram_calibrated(scl_handle* h, int32_t rows, int64_t K, int64_t ld, const uint16_t* a_hi, const uint16_t* a_lo,
                                           float scale, const double* diag, float* G, double* factor);
+/* The tcgen05 GEMM on its own with every launch field given: C = alpha * A B' (A: m x K, B: n x K, binary16 rows of lda / ldb
+ * elements; a_lo / b_lo: the low-order parts of split mode, both or neither).  All operand and result pointers are DEVICE
+ * pointers (16-byte aligned); the call synchronises its stream before it returns.  epi: 0 Store C[i*ldc + j], 1
+ * StoreTransposed C[j*ldc + i], 2 ColAbsMax C[j] = max(C[j], max_i |alpha (A B')_ij|) (C pre-filled by the caller).  syrk: A
+ * and B the same operand (m == n), lower tile triangle mirrored (Store only).  splits > 1: split-K partial s at C +
+ * s*split_stride; reduce_out (may be NULL): then also reduce_out[e] = reduce_scale * sum_s partial_s[e] for e <
+ * split_stride, as the pipeline reduces its partials.  chunk_kb: k-blocks of 64 per tensor-core accumulation chain (0: the
+ * default).  launch (may be NULL) = the launch as resolved: block_n, tile-splits, units (CTAs, or CTA pairs with
+ * cta_group 2), effective splits, chunk_kb, chunked, the most tile-splits one unit takes.  Returns SCL_ERR_INVALID, and
+ * launches nothing, for inconsistent arguments. */
+SCL_API int32_t scl_debug_gemm(scl_handle* h, int32_t m, int32_t n, int64_t K, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda,
+                               const uint16_t* b_hi, const uint16_t* b_lo, int64_t ldb, float alpha, int32_t epi, int32_t syrk,
+                               int32_t splits, int64_t split_stride, int32_t chunk_kb, int32_t cta_group, float* C, int64_t ldc,
+                               float* reduce_out, float reduce_scale, int32_t launch[7]);
 /* Tuning studies only (process-wide).  stat_variant: launch shape of the statistics passes (0-7: line passes,
  * 8: strip passes; < 0 keeps the current one).  stat_heavy: line length above which a whole CTA takes a line
  * (<= 0 keeps).  writer: dense writer, -1 automatic, 0 register/overlay writer, 1 TMA bulk-store writer, 2 / 3
- * TMA bulk-store writer with one / two cp.async-staged entries per thread and line (<= -2 keeps).  Results are
- * identical for every setting. */
+ * TMA bulk-store writer with one / two cp.async-staged entries per thread and line (<= -2 keeps).  Every writer and every
+ * line-pass variant (0-7) gives identical results; the strip passes (8) and another stat_heavy sum the Float64
+ * statistics in another order, which can change their last bits. */
 SCL_API int32_t scl_debug_set_tuning(int32_t stat_variant, int32_t stat_heavy, int32_t writer);
 SCL_API int32_t scl_bench_normalize(scl_handle* h, int32_t layout, int32_t with_lo, int32_t reps, double* ms_stats,
                             double* ms_densify, double* alg_bytes_densify);

@@ -191,6 +191,9 @@ SIGNATURES = {
     "scl_debug_two_stage": [_hp, C.c_int32, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.POINTER(C.c_int32)],
     "scl_debug_refine": [_hp, C.c_int32, _f32p, _f32p, _f32p, _i32p],
     "scl_debug_gram_calibrated": [_hp, C.c_int32, C.c_int64, C.c_int64, _u16p, _u16p, C.c_float, _f64p, _f32p, _f64p],
+    "scl_debug_gemm": [_hp, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                       C.c_int64, C.c_float, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
+                       C.c_int64, C.c_void_p, C.c_float, _i32p],
     "scl_debug_set_tuning": [C.c_int32, C.c_int32, C.c_int32],
     "scl_bench_normalize": [_hp, C.c_int32, C.c_int32, C.c_int32, _f64p, _f64p, _f64p],
 }

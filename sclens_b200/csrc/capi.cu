@@ -788,6 +788,49 @@ int32_t scl_debug_gram_calibrated(scl_handle* h, int32_t rows, int64_t K, int64_
   });
 }
 
+int32_t scl_debug_gemm(scl_handle* h, int32_t m, int32_t n, int64_t K, const uint16_t* a_hi, const uint16_t* a_lo, int64_t lda,
+                       const uint16_t* b_hi, const uint16_t* b_lo, int64_t ldb, float alpha, int32_t epi, int32_t syrk,
+                       int32_t splits, int64_t split_stride, int32_t chunk_kb, int32_t cta_group, float* C, int64_t ldc,
+                       float* reduce_out, float reduce_scale, int32_t* launch) {
+  auto aligned = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+  if (!h || !a_hi || !b_hi || !C || m < 1 || n < 1 || K < 1) return SCL_ERR_INVALID;
+  if ((a_lo == nullptr) != (b_lo == nullptr)) return SCL_ERR_INVALID;
+  if (lda < K || ldb < K || (lda & 7) || (ldb & 7)) return SCL_ERR_INVALID;
+  if (!aligned(a_hi) || !aligned(b_hi) || (a_lo && !aligned(a_lo)) || (b_lo && !aligned(b_lo)) || !aligned(C)) return SCL_ERR_INVALID;
+  if (epi < 0 || epi > 2 || splits < 1 || chunk_kb < 0 || (cta_group != 1 && cta_group != 2)) return SCL_ERR_INVALID;
+  if (syrk && (m != n || a_hi != b_hi || a_lo != b_lo || lda != ldb || epi != (int32_t)Epilogue::Store)) return SCL_ERR_INVALID;
+  // extent of one result: Store (and the syrk mirror) C[i*ldc + j], StoreTransposed C[j*ldc + i], ColAbsMax C[j]
+  int64_t extent = n;
+  if (epi == (int32_t)Epilogue::Store) {
+    if (ldc < n) return SCL_ERR_INVALID;
+    extent = (int64_t)(m - 1) * ldc + n;
+  } else if (epi == (int32_t)Epilogue::StoreTransposed) {
+    if (ldc < m) return SCL_ERR_INVALID;
+    extent = (int64_t)(n - 1) * ldc + m;
+  }
+  if (splits > 1 && split_stride < extent) return SCL_ERR_INVALID;
+  if (reduce_out && (splits < 2 || epi == (int32_t)Epilogue::ColAbsMax)) return SCL_ERR_INVALID;
+  return guard(h, [&] {
+    SCL_CUDA(cudaSetDevice(h->cfg.device));
+    GemmArgs a;
+    a.A.hi = reinterpret_cast<const __half*>(a_hi); a.A.lo = reinterpret_cast<const __half*>(a_lo);
+    a.A.rows = m; a.A.K = K; a.A.ld = lda;
+    a.B.hi = reinterpret_cast<const __half*>(b_hi); a.B.lo = reinterpret_cast<const __half*>(b_lo);
+    a.B.rows = n; a.B.K = K; a.B.ld = ldb;
+    a.syrk = syrk != 0; a.alpha = alpha; a.epi = (Epilogue)epi; a.C = C; a.ldc = ldc;
+    a.splits = splits; a.split_stride = split_stride; a.cta_group = cta_group; a.chunk_kb = chunk_kb;
+    GemmLaunch L;
+    gemm_umma(a, h->st, &L);
+    // as gemm_splitk and apply_G reduce their partials (the effective split count: the kernel never makes more than k-blocks)
+    if (reduce_out) reduce_splits(C, L.splits, split_stride, (size_t)split_stride, reduce_scale, reduce_out, h->st);
+    SCL_CUDA(cudaStreamSynchronize(h->st));
+    if (launch) {
+      const int v[7] = {L.block_n, L.n_tiles, L.units, L.splits, L.chunk_kb, L.chunked, L.max_per_unit};
+      for (int i = 0; i < 7; ++i) launch[i] = v[i];
+    }
+  });
+}
+
 int32_t scl_debug_set_tuning(int32_t stat_variant, int32_t stat_heavy, int32_t writer) {
   scl::set_norm_tuning(stat_variant, stat_heavy, writer);
   return SCL_OK;

@@ -176,7 +176,12 @@ struct GemmArgs {
   int cta_group = 2;        // 1 or 2
   int chunk_kb = 0;         // k-blocks (of 64) per tensor-core accumulation chunk; 0 = default (64, or 21 in split mode)
 };
-void gemm_umma(const GemmArgs& a, cudaStream_t st);
+// the launch gemm_umma resolved (scl_debug_gemm reports it): tile-splits = output tiles x effective splits, walked by
+// `units` persistent CTAs (pairs with cta_group 2); chunked: chunk_kb k-blocks per tensor-core chain, FP32 sum across chunks
+struct GemmLaunch {
+  int block_n = 0, n_tiles = 0, units = 0, splits = 0, chunk_kb = 0, chunked = 0, max_per_unit = 0;
+};
+void gemm_umma(const GemmArgs& a, cudaStream_t st, GemmLaunch* info = nullptr);
 void split_f32_to_f16(const float* in, size_t n, __half* hi, __half* lo, cudaStream_t st);
 // pre_scale (a power of two) is applied before rounding so the low-order part of small entries (unit vectors in
 // high dimension: ~1/sqrt(n)) stays in the normal binary16 range; the caller divides alpha by it

@@ -369,6 +369,9 @@ k_gemm_umma(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__
       const Tile t = p.tiles[it];
       const int kb0 = t.split * kb_per_split;
       const int kb1 = min(p.k_blocks_total, kb0 + kb_per_split);
+      // An empty split-K partition (the last ones when splits does not divide the k-blocks) takes no accumulator stage:
+      // no wait, no commit, no phase advance - the epilogue skips it alike and writes its zeros from registers.
+      if (kb1 <= kb0) continue;
       // The tensor core accumulates in FP32 with truncation towards zero: every partial sum shrinks by ~1e-7 of its
       // magnitude per MMA (more for coherent same-sign sums than for random-sign ones).  The truncation is symmetric in
       // sign - accumulating alternate chunks with the operand negated (instruction-descriptor bit 13) and subtracting
@@ -403,7 +406,7 @@ k_gemm_umma(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__
           umma_commit<CG>(&empty_bar[stage]);     // frees the smem slot in every CTA of the group
           if (++stage == C::kStages) { stage = 0; phase ^= 1; }
         }
-        if (kb1 > kb0) umma_commit<CG>(&tmem_full[accum]);
+        umma_commit<CG>(&tmem_full[accum]);
         if (++accum == n_acc) { accum = 0; accum_phase ^= 1; }
       } while (kb < kb1);
     }
@@ -431,18 +434,19 @@ k_gemm_umma(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__
       int n_cols = min(block_n, p.n_rows - col0);
       if (p.syrk) n_cols = min(n_cols, e.row0 + 32 - col0);
       if (e.row0 >= p.m_rows) n_cols = 0;
+      // an empty split-K partition: no accumulator stage (as in the issuer), zeros from registers
+      const bool have = kb1 > kb0;
       int kb = kb0;
       do {   // one pass per accumulation chunk
         const bool first_chunk = kb == kb0;
         kb = min(kb1, kb + p.chunk_kb);
         const bool last_chunk = kb >= kb1;
-        if (kb1 > kb0) {
+        if (have) {
           mbar_wait(&tmem_full[accum], accum_phase);
           tc_fence_after();
         }
         const uint32_t t_chunk = tmem_base + lane_sel + (uint32_t)(accum * kMaxBlockN);
         const uint32_t t_sum = tmem_base + lane_sel + (uint32_t)kMaxBlockN;     // chunked mode only
-        const bool have = kb1 > kb0;
         if (p.chunked && have) {
           // fold the chunk into the running sum, then hand the chunk accumulator back before any global store
           for (int c0 = 0; c0 < n_cols; c0 += 32) {
@@ -468,7 +472,7 @@ k_gemm_umma(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__
             if (CG == 2) mbar_arrive_cluster(&tmem_empty[accum], 0); else mbar_arrive_local(&tmem_empty[accum]);
           }
         };
-        if (p.chunked) release();
+        if (p.chunked && have) release();
         if (last_chunk) {
           const uint32_t t_src = p.chunked ? t_sum : t_chunk;
           for (int c0 = 0; c0 < n_cols; c0 += 32) {
@@ -502,8 +506,10 @@ k_gemm_umma(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__
             }
           }
         }
-        if (!p.chunked) release();
-        if (++accum == n_acc) { accum = 0; accum_phase ^= 1; }
+        if (have) {
+          if (!p.chunked) release();
+          if (++accum == n_acc) { accum = 0; accum_phase ^= 1; }
+        }
       } while (kb < kb1);
     }
   }
@@ -566,7 +572,7 @@ std::vector<Tile> build_tiles(int tiles_m, int tiles_n, int splits, bool syrk, i
 }
 
 template <int CG, bool SPLIT>
-void launch(const GemmArgs& a, cudaStream_t st) {
+void launch(const GemmArgs& a, cudaStream_t st, GemmLaunch* info) {
   using C = Cfg<CG, SPLIT>;
   const int tile_m = kTileRowsA * CG;
   int block_n = kMaxBlockN;
@@ -634,6 +640,15 @@ void launch(const GemmArgs& a, cudaStream_t st) {
   cfg.numAttrs = 1;
   SCL_CUDA(cudaLaunchKernelEx(&cfg, kern, mA_hi, mA_lo, mB_hi, mB_lo, p));
   count_launches(1);
+  if (info) {
+    info->block_n = block_n;
+    info->n_tiles = p.n_tiles;
+    info->units = units;
+    info->splits = splits;
+    info->chunk_kb = p.chunk_kb;
+    info->chunked = p.chunked;
+    info->max_per_unit = (p.n_tiles + units - 1) / units;
+  }
 }
 
 // ---- small elementwise helpers ----------------------------------------------------------
@@ -695,14 +710,14 @@ int sm_count() {
   return n;
 }
 
-void gemm_umma(const GemmArgs& a, cudaStream_t st) {
+void gemm_umma(const GemmArgs& a, cudaStream_t st, GemmLaunch* info) {
   SCL_REQUIRE(a.A.hi && a.B.hi && a.C, "null GEMM operand");
   SCL_REQUIRE(a.A.K == a.B.K, "contraction lengths differ");
   const bool split = a.A.lo != nullptr && a.B.lo != nullptr;
   if (a.cta_group == 1) {
-    if (split) launch<1, true>(a, st); else launch<1, false>(a, st);
+    if (split) launch<1, true>(a, st, info); else launch<1, false>(a, st, info);
   } else {
-    if (split) launch<2, true>(a, st); else launch<2, false>(a, st);
+    if (split) launch<2, true>(a, st, info); else launch<2, false>(a, st, info);
   }
 }
 

@@ -105,37 +105,88 @@ def test_gram_syrk(h, h1, rows, K, cg, split):
     assert np.array_equal(G, G.T)       # mirrored store: exactly symmetric
 
 
+def normalize_dev(h, X, layout, with_lo=True):
+    """scl_op_normalize: (hi, lo or None) as [lines][ld] uint16, and the statistics."""
+    N, M = X.shape
+    lines, length = (M, N) if layout == 0 else (N, M)
+    ld = (length + 7) // 8 * 8
+    hi = np.empty((lines, ld), dtype=np.uint16)
+    lo = np.empty((lines, ld), dtype=np.uint16) if with_lo else None
+    st = dict(tgc=np.empty(N), l2=np.empty(N), mean=np.empty(M), sd=np.empty(M), cent=np.empty(M))
+    colptr, rowval, val = _lib.as_u32(X.indptr), _lib.as_u32(X.indices), _lib.as_f32(X.data)
+    h._ck(h.lib.scl_op_normalize(h.h, N, M, X.nnz, ptr(colptr, C.c_uint32), ptr(rowval, C.c_uint32),
+                                 ptr(val, C.c_float), layout, ld, ptr(hi, C.c_uint16), ptr(lo, C.c_uint16),
+                                 ptr(st["tgc"], C.c_double), ptr(st["mean"], C.c_double), ptr(st["sd"], C.c_double),
+                                 ptr(st["l2"], C.c_double), ptr(st["cent"], C.c_double)))
+    return hi, lo, st, length
+
+
+def assert_normalize_oracle(ref, rec, layout, hi, lo, st, length):
+    np.testing.assert_array_equal(st["tgc"], rec["TGC"])
+    np.testing.assert_allclose(st["mean"], rec["mat2_mean"].ravel(), rtol=1e-12)
+    np.testing.assert_allclose(st["sd"], rec["mat2_std"].ravel(), rtol=1e-11)
+    np.testing.assert_allclose(st["l2"], rec["norm_tgc"], rtol=1e-11)
+    np.testing.assert_allclose(st["cent"], rec["cent_"].ravel(), rtol=1e-9, atol=1e-15)
+    want = ref.T if layout == 0 else ref
+    got_hi = hi.view(np.float16)[:, :length].astype(np.float64)
+    # hi alone is the correctly rounded binary16 value (up to float32 background arithmetic)
+    assert np.max(np.abs(got_hi - want) / (np.abs(want) + 1e-3)) < 6e-4
+    assert not hi.view(np.float16)[:, length:].any()
+    if lo is not None:
+        got = got_hi + lo.view(np.float16)[:, :length].astype(np.float64)
+        # hi + lo reproduces the Float32 rounding of the Float64 reference value
+        assert np.max(np.abs(got - want) / np.maximum(1.0, np.abs(want))) < 4e-7
+
+
 # (2301, 4700) spans several writer strips and has gene lines above the CTA-per-line threshold of the statistics
 # passes; (260, 20000) has cell lines above it
-@pytest.mark.parametrize("N,M", [(500, 800), (900, 400), (2301, 4700), (260, 20000)])
+NORM_SHAPES = [(500, 800), (900, 400), (2301, 4700), (260, 20000)]
+
+
+@pytest.mark.parametrize("N,M", NORM_SHAPES)
 @pytest.mark.parametrize("layout", [0, 1])
 def test_normalize_matches_oracle(h, N, M, layout):
     X = make_counts(N, M, seed=11, K=4, de_prob=0.3, lfc_sd=1.5)
     ref, rec = orc.normalize_main(X)
-    lines, length = (M, N) if layout == 0 else (N, M)
-    ld = (length + 7) // 8 * 8
-    hi = np.empty((lines, ld), dtype=np.uint16)
-    lo = np.empty((lines, ld), dtype=np.uint16)
-    tgc, l2 = np.empty(N), np.empty(N)
-    mean, sd, cent = np.empty(M), np.empty(M), np.empty(M)
-    colptr, rowval, val = _lib.as_u32(X.indptr), _lib.as_u32(X.indices), _lib.as_f32(X.data)
-    h._ck(h.lib.scl_op_normalize(h.h, N, M, X.nnz, ptr(colptr, C.c_uint32), ptr(rowval, C.c_uint32),
-                                 ptr(val, C.c_float), layout, ld, ptr(hi, C.c_uint16), ptr(lo, C.c_uint16),
-                                 ptr(tgc, C.c_double), ptr(mean, C.c_double), ptr(sd, C.c_double),
-                                 ptr(l2, C.c_double), ptr(cent, C.c_double)))
-    np.testing.assert_array_equal(tgc, rec["TGC"])
-    np.testing.assert_allclose(mean, rec["mat2_mean"].ravel(), rtol=1e-12)
-    np.testing.assert_allclose(sd, rec["mat2_std"].ravel(), rtol=1e-11)
-    np.testing.assert_allclose(l2, rec["norm_tgc"], rtol=1e-11)
-    np.testing.assert_allclose(cent, rec["cent_"].ravel(), rtol=1e-9, atol=1e-15)
-    want = ref.T if layout == 0 else ref
-    got_hi = hi.view(np.float16)[:, :length].astype(np.float64)
-    got = got_hi + lo.view(np.float16)[:, :length].astype(np.float64)
-    # hi alone is the correctly rounded binary16 value (up to float32 background arithmetic)
-    assert np.max(np.abs(got_hi - want) / (np.abs(want) + 1e-3)) < 6e-4
-    # hi + lo reproduces the Float32 rounding of the Float64 reference value
-    assert np.max(np.abs(got - want) / np.maximum(1.0, np.abs(want))) < 4e-7
-    assert not hi.view(np.float16)[:, length:].any()
+    hi, lo, st, length = normalize_dev(h, X, layout)
+    assert_normalize_oracle(ref, rec, layout, hi, lo, st, length)
+
+
+@pytest.fixture
+def norm_tuning(h):
+    """Restores the default launch choices of the normalisation kernels (statistics variant 4, whole-CTA lines above
+    4096 entries, automatic writer) after the test."""
+    yield lambda variant, heavy, writer: h._ck(h.lib.scl_debug_set_tuning(variant, heavy, writer))
+    h._ck(h.lib.scl_debug_set_tuning(4, 4096, -1))
+
+
+@pytest.mark.parametrize("N,M", NORM_SHAPES)
+@pytest.mark.parametrize("layout", [0, 1])
+def test_normalize_every_writer_and_statistics_variant(h, norm_tuning, N, M, layout):
+    """The hi-only output (the single-pass Gram operand: writer -1 picks the staged TMA-store writer 2 without lo) meets the
+    oracle; every dense writer gives the hi bytes of the hi+lo call, with or without lo, and a zero pad; every launch
+    variant of the statistics passes, and whole-CTA lines from 64 entries on, meet the oracle."""
+    X = make_counts(N, M, seed=11, K=4, de_prob=0.3, lfc_sd=1.5)
+    ref, rec = orc.normalize_main(X)
+    norm_tuning(4, 4096, -1)
+    hi0, lo0, st, length = normalize_dev(h, X, layout)
+    hi, _, st1, _ = normalize_dev(h, X, layout, with_lo=False)
+    assert_normalize_oracle(ref, rec, layout, hi, None, st1, length)
+    for writer in (-1, 0, 1, 2, 3):
+        norm_tuning(-1, 0, writer)
+        hi, _, _, _ = normalize_dev(h, X, layout, with_lo=False)
+        np.testing.assert_array_equal(hi, hi0, err_msg=f"writer {writer}, hi only")
+        hi, lo, _, _ = normalize_dev(h, X, layout)
+        np.testing.assert_array_equal(hi, hi0, err_msg=f"writer {writer}, hi + lo")
+        np.testing.assert_array_equal(lo, lo0, err_msg=f"writer {writer}, lo")
+    norm_tuning(-1, 0, -1)
+    for variant, heavy in [(v, 4096) for v in range(9)] + [(4, 64), (8, 64)]:
+        norm_tuning(variant, heavy, -2)
+        hi, lo, st1, _ = normalize_dev(h, X, layout)
+        assert_normalize_oracle(ref, rec, layout, hi, lo, st1, length)
+        if variant < 8 and heavy == 4096:   # the line passes differ in launch shape only: the same Float64 sums
+            for k in st:
+                np.testing.assert_array_equal(st1[k], st[k], err_msg=f"statistics variant {variant}: {k}")
 
 
 def csc_arrays(X):
